@@ -237,6 +237,25 @@ def per_call_latency(m, model, pt, pm, ev, th0_host, iters=40):
     return out
 
 
+DUMP_LIMIT_BYTES = 60 << 20     # with the .npy headers, under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes what the timed run returned for its last step, one row per chain, as <out_dir>/<name>.npy in float64, so that
+    two builds can be compared output for output. Above DUMP_LIMIT_BYTES a fixed seeded sample of the chains is written;
+    chain.npy holds the indices of the chains written."""
+    arrays = {k: v.cpu().numpy().reshape(v.shape[0], -1).astype(np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    per_chain = 8 * (1 + sum(a.shape[1] for a in arrays.values()))
+    chain = np.arange(n)
+    if n * per_chain > DUMP_LIMIT_BYTES:
+        chain = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // per_chain, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "chain.npy"), chain.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[chain].squeeze(1) if a.shape[1] == 1 else a[chain])
+
+
 # ---------------------------------------------------------------------------------------------------
 def run_gpu(args):
     import torch
@@ -305,6 +324,9 @@ def run_gpu(args):
     t_ms = max_over_ranks(dev_ms)
     value = world * C * steps / (t_ms * 1e-3)
     accept_rate = float(log_acc.float().mean().item())
+    if args.dump_outputs and rank == 0:     # rank 0 runs the same chains at any --gpus
+        dump_outputs(args.dump_outputs, {"component": log_comp[-1], "accepted": log_acc[-1], "values": log_val[-1],
+                                         "theta": log_th[-1], "theta_final": th_final, "n_accepted": n_acc})
 
     # ---- sustained arm: >= 2000 resumed steps of the same chains (seconds under load, clocks sampled) -------
     sustained = None
@@ -629,13 +651,20 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
-    ap.add_argument("--chains", type=int, default=4736, help="chains per GPU (32 x 148 SMs; 2368 gives 4 % less, profiles/r2_session3.md)")
+    ap.add_argument("--chains", type=int, default=4736, help="chains per GPU (32 x 148 SMs; 2368 gives 4 %% less, profiles/r2_session3.md)")
     ap.add_argument("--cpu-steps", type=int, default=120, help="MH steps of the cpu_baseline sample")
     ap.add_argument("--sustain-steps", type=int, default=2000, help="steps of the sustained-load arm (0 = skip)")
     ap.add_argument("--rank-update", default="int8", choices=["int8", "fp64"],
                     help="arithmetic of the posterior's rank update: INT8 tensor cores (tcgen05; default) or the FP64 tensor pipe")
     ap.add_argument("--ref-steps", type=int, default=12, help="MH steps per chain and bench step of --impl reference")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl b200 only: write what the timed run returned for its last step (one row per chain) to "
+                         "DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if args.warmup < 1:
         args.warmup = 1
     if args.impl == "reference":

@@ -1,6 +1,6 @@
 """CPU suite: the C oracle against its independent numpy restatement, against the committed golden
 values on the reference's femur fixtures, and against analytic known answers (SURVEY.md 8c i-vii)."""
-import os
+import struct
 
 import numpy as np
 import pytest
@@ -217,13 +217,123 @@ def test_femur_target_is_explained_by_the_model(femur):
     assert res.mean() < 0.5 and res.max() < 2.0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/data/femur"), reason="reference checkout not present")
-def test_fixture_readers_against_reference_files(femur):
-    m = fx.load_gpmm_h5("/root/reference/data/femur/femur_gp_model_100-components.h5")
+def _binary_stl(verts, tris):
+    """Binary STL of a triangle mesh: one float32 facet per triangle (corners in the triangle's vertex order, the facet
+    normal, a running attribute word)."""
+    rec = np.zeros(len(tris), dtype=[("n", "<f4", 3), ("v", "<f4", (3, 3)), ("a", "<u2")])
+    rec["v"] = verts[tris]
+    rec["n"] = np.cross(rec["v"][:, 1] - rec["v"][:, 0], rec["v"][:, 2] - rec["v"][:, 0])
+    rec["a"] = np.arange(len(tris)) & 0xFFFF
+    return b"binary STL".ljust(80) + struct.pack("<I", len(tris)) + rec.tobytes()
+
+
+def _hdf5_file(tree):
+    """An HDF5 file holding `tree`: name -> ndarray, bytes (a fixed-length string) or dict (a group, whose '@name' keys are
+    string attributes). It uses the constructs of the file format the statismo model files are written in: superblock v0,
+    v1 object headers (the layout message of every dataset in a continuation block), symbol-table groups with B-trees of
+    one and of two levels, scalar datasets, and both the v1 and the v3 contiguous-layout message."""
+    undef = 0xFFFFFFFFFFFFFFFF
+    buf = bytearray(96)                                   # superblock + root symbol-table entry, written last
+
+    def put(b):
+        addr = len(buf)
+        buf.extend(b + bytes(-len(b) % 8))
+        return addr
+
+    def messages(msgs):
+        return b"".join(struct.pack("<HHB3x", t, len(m) + -len(m) % 8, 0) + m + bytes(-len(m) % 8) for t, m in msgs)
+
+    def object_header(msgs, continued=()):
+        if continued:
+            more = messages(continued)
+            msgs = msgs + [(0x10, struct.pack("<QQ", put(more), len(more)))]
+        body = messages(msgs)
+        return put(struct.pack("<BBHII4x", 1, 0, len(msgs) + len(continued), 1, len(body)) + body)
+
+    def space(shape):
+        return struct.pack("<BBB5x", 1, len(shape), 0) + struct.pack(f"<{len(shape)}Q", *shape)
+
+    def string_type(n):
+        return struct.pack("<BBxxI", 0x13, 0, n)
+
+    def attribute(name, value):
+        parts = [name.encode() + b"\0", string_type(len(value)), space(())]
+        return struct.pack("<BxHHH", 1, *map(len, parts)) + b"".join(p + bytes(-len(p) % 8) for p in parts) + value
+
+    def dataset(a):
+        if isinstance(a, bytes):
+            layout = struct.pack("<BBQQ", 3, 1, put(a), len(a))
+            return object_header([(0x1, space(())), (0x3, string_type(len(a)))], [(0x8, layout)])
+        a = np.ascontiguousarray(a)
+        addr, bits = put(a.tobytes()), 8 * a.itemsize
+        if a.dtype.kind == "f":
+            exp, mant = {4: (8, 23), 8: (11, 52)}[a.itemsize]
+            dtype = struct.pack("<BBBxIHHBBBBI", 0x11, 0x20, bits - 1, a.itemsize, 0, bits, mant, exp, 0, mant, 2 ** (exp - 1) - 1)
+            layout = struct.pack("<BBQQ", 3, 1, addr, a.nbytes)
+        else:
+            dtype = struct.pack("<BBxxIHH", 0x10, 0x08 if a.dtype.kind == "i" else 0, a.itemsize, 0, bits)
+            layout = struct.pack("<BBB5xQ", 1, a.ndim + 1, 1, addr) + struct.pack(f"<{a.ndim + 1}I", *a.shape, a.itemsize)
+        return object_header([(0x1, space(a.shape)), (0x3, dtype)], [(0x8, layout)])
+
+    def group(children):
+        heap, entries = bytearray(8), []                  # heap offset 0: the empty name
+        for name in sorted(k for k in children if not k.startswith("@")):
+            child = children[name]
+            entries.append((len(heap), group(child) if isinstance(child, dict) else dataset(child)))
+            heap += name.encode() + bytes(8 - len(name) % 8)
+        local_heap = put(b"HEAP" + struct.pack("<B3xQQQ", 0, len(heap), undef, put(bytes(heap))))
+
+        def leaf(es):
+            snod = put(b"SNOD" + struct.pack("<BxH", 1, len(es)) + b"".join(struct.pack("<QQII16x", o, a, 0, 0) for o, a in es))
+            return put(b"TREE" + struct.pack("<BBHQQQQQ", 0, 0, 1, undef, undef, 0, snod, es[-1][0]))
+        btree = leaf(entries)
+        if len(entries) > 2:                              # a level-1 node over two leaves
+            h = len(entries) // 2
+            btree = put(b"TREE" + struct.pack("<BBHQQ5Q", 0, 1, 2, undef, undef, 0, leaf(entries[:h]), entries[h - 1][0],
+                                              leaf(entries[h:]), entries[-1][0]))
+        attrs = [(0xC, attribute(k[1:], v)) for k, v in children.items() if k.startswith("@")]
+        return object_header([(0x11, struct.pack("<QQ", btree, local_heap))] + attrs)
+
+    root = group(tree)
+    struct.pack_into("<8s8BHHIQQQQ", buf, 0, b"\x89HDF\r\n\x1a\n", 0, 0, 0, 0, 0, 8, 8, 0, 4, 16, 0, 0, undef, len(buf), undef)
+    struct.pack_into("<QQII16x", buf, 56, 0, root, 0, 0)
+    return bytes(buf)
+
+
+def test_fixture_readers_round_trip(femur, tmp_path):
+    """fixtures_io on files this test writes in the formats of the reference's data files (those files are not part of the
+    repository): a statismo model file holding the committed GPMM-100 fixture, and binary STLs of the femur mesh with the
+    facets in cell order and shuffled. The readers return the arrays written, pass over what they do not use (attributes,
+    string datasets) and merge STL corners into vertices in the order of first appearance."""
+    ref32, cells = femur["ref"].astype(np.float32), femur["cells"]
+    basis32, var32 = femur["gpmm_100"]["basis"].astype(np.float32), femur["gpmm_100"]["variance"].astype(np.float32)
+    path = str(tmp_path / "model.h5")
+    with open(path, "wb") as f:
+        f.write(_hdf5_file({
+            "@name": b"femur",
+            "version": {"majorVersion": np.array(0, np.int32), "minorVersion": np.array(9, np.int32)},
+            "modelinfo": {"build-time": b"2020-01-01 00:00:00"},
+            "representer": {"@datasetType": b"POLYGON_MESH", "points": np.ascontiguousarray(ref32.T), "cells": np.ascontiguousarray(cells.T)},
+            "model": {"mean": ref32.ravel(), "noiseVariance": np.array(0.0, np.float32), "pcaBasis": basis32, "pcaVariance": var32}}))
+    found = fx.read_hdf5_datasets(path)
+    assert sorted(found) == ["/model/mean", "/model/noiseVariance", "/model/pcaBasis", "/model/pcaVariance", "/representer/cells",
+                             "/representer/points", "/version/majorVersion", "/version/minorVersion"]
+    assert found["/version/minorVersion"] == 9 and found["/model/noiseVariance"] == 0.0
+    m = fx.load_gpmm_h5(path)
     assert m["basis"].shape == (4866, 101) and np.abs(m["mean_def"]).max() == 0.0
-    v, c = fx.read_binary_stl("/root/reference/data/femur/femur_reference.stl")
-    assert np.array_equal(c, m["cells"]) and np.array_equal(v, m["ref"])
-    assert np.array_equal(femur["ref"], m["ref"]) and np.array_equal(femur["gpmm_100"]["basis"], m["basis"])
+    assert np.array_equal(m["basis"], basis32) and np.array_equal(m["variance"], var32)
+    assert np.array_equal(m["ref"], ref32) and np.array_equal(m["cells"], cells)
+    with open(tmp_path / "mesh.stl", "wb") as f:
+        f.write(_binary_stl(ref32, cells))
+    v, c = fx.read_binary_stl(str(tmp_path / "mesh.stl"))
+    assert np.array_equal(v, m["ref"]) and np.array_equal(c, m["cells"])
+    shuffled = cells[np.random.default_rng(0).permutation(len(cells))][:, [1, 2, 0]]
+    with open(tmp_path / "shuffled.stl", "wb") as f:
+        f.write(_binary_stl(ref32, shuffled))
+    v, c = fx.read_binary_stl(str(tmp_path / "shuffled.stl"))
+    corners = shuffled.ravel()
+    assert np.array_equal(v, ref32[corners[np.sort(np.unique(corners, return_index=True)[1])]])
+    assert np.array_equal(v[c], ref32[shuffled])
 
 
 def test_chain_oracle_closed_form_tracks_reference_structure(twin31):
