@@ -66,6 +66,11 @@ class ChainIO(C.Structure):
                 ("metrics_interval", C.c_int32), ("reserved", C.c_int32), ("log_metrics", C.c_void_p)]
 
 
+class ChainStatsParams(C.Structure):
+    _fields_ = [("burn_in", C.c_int64), ("take_every_n", C.c_int64), ("end", C.c_int64), ("normals", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
 _SIGS = {
     "icp_ctx_create": [C.c_int32, C.POINTER(_h)],
     "icp_ctx_destroy": [_h],
@@ -124,6 +129,8 @@ _SIGS = {
     "icp_chain_last_run_stats": [_h, _dp, _lp],
     "icp_chain_set_lookahead": [_h, C.c_int32],
     "icp_chain_last_run_rounds": [_h, _lp],
+    "icp_chain_set_statistics": [_h, C.POINTER(ChainStatsParams)],
+    "icp_chain_statistics": [_h, C.c_int32, C.c_int32, _dp, _lp, _dp, _dp, _dp, _dp],
     "icp_debug_philox": [_h, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32)],
     "icp_debug_fp64_peak": [_h, _dp],
     "icp_debug_dmma_sweep": [_h, C.c_int32, C.c_int32, C.c_int32, _dp],

@@ -724,6 +724,7 @@ class SamplingRegistration:
     def __init__(self, model: StatisticalMeshModel, sample: TriangleMesh3D, seed=1024):
         self.model, self.sample, self.seed = model, sample, seed
         self.initialParametersZero = model.initial_parameters()
+        self.variability = None   # runfitting(variability=...)
 
     @staticmethod
     def _device_evaluator(model, target, evaluators):
@@ -737,13 +738,21 @@ class SamplingRegistration:
         return ev, ["product", "prior", dist_key]
 
     def runfitting(self, evaluators, generator: MixtureProposal, numOfSamples, initialModelParameters=None, jsonName=None,
-                   n_chains=1, initial_batch=None):
+                   n_chains=1, initial_batch=None, variability=None):
         """Returns the best sample (BestSampleLogger); writes the JSON chain log when jsonName is given.
-        n_chains > 1 runs independent chains batched on the GPU and returns the list of per-chain best samples."""
+        n_chains > 1 runs independent chains batched on the GPU and returns the list of per-chain best samples.
+        variability: dict(takeEveryN, total=0, burnIn=0, sumNormals=True, perChain=False) - the posterior variability maps
+        (PosteriorVariability.scala:30-73) of the samples LogHelper.samplesFromLog would take from the chain log, accumulated
+        inside the run (icp_chain_statistics; total <= 0: no limit). They are left in self.variability: one dict pooled over
+        the chains, or a list with one dict per chain (perChain), each as core.posterior_variability returns it plus n."""
         comps = generator.flatten()
         names = [c["name"] for c in comps]
         ev, keys = self._device_evaluator(self.model, self.sample, evaluators)
         chain = core.Chain(self.model, self.sample, comps, ev, max_chains=n_chains)
+        if variability is not None:
+            sum_normals = bool(variability.get("sumNormals", True))
+            chain.set_statistics(int(variability.get("burnIn", 0)), int(variability["takeEveryN"]), int(variability.get("total", 0)),
+                                 normals=sum_normals)
         if initial_batch is not None:
             th0 = np.asarray(initial_batch, float)
         else:
@@ -757,6 +766,11 @@ class SamplingRegistration:
             name = names[int(out["component"][same[0], c])] if len(same) else "Anonymous"
             best.append(ModelFittingParameters.from_vector(out["theta_best"][c], name))
         self.last_run = out
+        if variability is not None:
+            if variability.get("perChain", False):
+                self.variability = [chain.statistics(c, sum_normals) for c in range(n_chains)]
+            else:
+                self.variability = chain.statistics(-1, sum_normals)
         if jsonName is not None:
             # the device log goes to the reference's file format through the library's streaming writer (icp_jsonlog_*)
             native = core.JsonLog(jsonName, self.model.K, names, keys)

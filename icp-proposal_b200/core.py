@@ -568,6 +568,30 @@ class Chain:
         check(self.lib.icp_chain_last_run_rounds(self.h, C.byref(n)))
         return n.value
 
+    def set_statistics(self, burn_in, take_every_n=1, end=0, normals=True):
+        """icp_chain_set_statistics: accumulate the posterior variability maps of the records burn_in, burn_in + take_every_n, ...
+        below `end` (<= 0: no limit) inside the run, from the next run from theta0 on. burn_in=None switches them off."""
+        if burn_in is None:
+            check(self.lib.icp_chain_set_statistics(self.h, None), self.ctx.h)
+            return
+        p = _lib.ChainStatsParams(int(burn_in), int(take_every_n), int(end), 1 if normals else 0, 0)
+        check(self.lib.icp_chain_set_statistics(self.h, C.byref(p)), self.ctx.h)
+
+    def statistics(self, chain=-1, sum_normals=True, theta_ref=None):
+        """icp_chain_statistics: the maps of chain `chain` of the resident run, or pooled over its chains (-1): the dict of
+        posterior_variability plus n, the number of samples."""
+        n = self.model.N
+        mean, cov, tot, nrm = np.empty((n, 3)), np.empty((n, 3, 3)), np.empty(n), np.empty(n)
+        ref = None
+        if theta_ref is not None:
+            ref, one = self.model._theta(theta_ref)
+            if one != 1:
+                raise ValueError("theta_ref must be a single parameter vector")
+        s = C.c_int64(0)
+        check(self.lib.icp_chain_statistics(self.h, int(chain), 1 if sum_normals else 0, dptr(ref) if ref is not None else None,
+                                            C.byref(s), dptr(mean), dptr(cov), dptr(tot), dptr(nrm)), self.ctx.h)
+        return dict(mean=mean, cov=cov, total_variance=tot, normal_variance=nrm, n=int(s.value))
+
     def profile(self, theta0, n_steps, seed=1024):
         th, c = self.model._theta(theta0)
         ms = np.zeros(_lib.N_STAGES); n = np.zeros(_lib.N_STAGES, np.int64)

@@ -56,6 +56,22 @@ struct LogDev {
     int step_base;   // record index = step - step_base (resumed runs keep counting steps for the RNG)
 };
 
+// posterior variability accumulated inside the run (icp_chain_set_statistics, stats.cu); every pointer is null when off.
+// Per chain (look-ahead: per chain, not per lane): the selected records at which the current state was current and that
+// are not in the accumulators yet, and what the current step / round flushed into them.
+struct StatsDev {
+    long long *pending;      // [Cr]
+    long long *count;        // [Cr] samples in the accumulators
+    long long *flush_w;      // [Cr] weight flushed by this step / round (0: none)
+    long long *flush_n;      // [Cr] count before that flush
+    double *flush_theta;     // [Cr][L] the flushed state
+    long long burn_in, every, end;
+};
+
+__device__ __forceinline__ int stats_selected(const StatsDev &x, long long i) {
+    return i >= x.burn_in && (x.end <= 0 || i < x.end) && (i - x.burn_in) % x.every == 0;
+}
+
 struct StateDev {
     double *theta_cur, *theta_prop;     // [C][L]
     double *values_cur, *values_prop;   // [C][3]
@@ -74,6 +90,7 @@ struct StateDev {
     double *qf, *qb;
     // look-ahead only: the lanes' accept decisions and status words of this round, the first step the run must not take
     int *lane_ok, *lane_status, *step_end;
+    StatsDev sx;
 };
 
 // per-chain status bits of a run (icp_chain_io.status)
@@ -405,6 +422,24 @@ __global__ void __launch_bounds__(128) k_chain_accept(ChainParams P, StateDev st
     __syncthreads();
     if (P.W > 1) return;
     int ok = s_acc;
+    if (st.sx.pending) {
+        // statistics: an accepting chain flushes its old state with the selected records at which it was current; this
+        // step's record belongs to the state that is current after it
+        __shared__ int s_flush;
+        if (threadIdx.x == 0) {
+            const long long pend = st.sx.pending[c];
+            const int sel = stats_selected(st.sx, step);
+            const int flush = ok && pend > 0;
+            st.sx.flush_w[c] = flush ? pend : 0;
+            if (flush) { st.sx.flush_n[c] = st.sx.count[c]; st.sx.count[c] += pend; }
+            st.sx.pending[c] = ok ? sel : pend + sel;
+            s_flush = flush;
+        }
+        __syncthreads();
+        if (s_flush)
+            for (int j = threadIdx.x; j < Lt; j += blockDim.x) st.sx.flush_theta[(size_t)c * Lt + j] = cur[j];
+        __syncthreads();
+    }
     if (ok) {
         for (int j = threadIdx.x; j < Lt; j += blockDim.x) st.theta_cur[(size_t)c * Lt + j] = prp[j];
         if (threadIdx.x < 3) st.values_cur[3 * c + threadIdx.x] = st.values_prop[3 * c + threadIdx.x];
@@ -482,7 +517,10 @@ __global__ void __launch_bounds__(128) k_la_resolve(ChainParams P, StateDev st, 
     const int s0 = st.step[c];
     int limit = *st.step_end - s0;
     if (limit > P.Wa) limit = P.Wa;               // lanes that ran in this round
-    if (limit <= 0) return;                       // this chain has taken all its steps
+    if (limit <= 0) {                             // this chain has taken all its steps
+        if (st.sx.pending && threadIdx.x == 0) st.sx.flush_w[c] = 0;
+        return;
+    }
     int jstar = -1;
     for (int j = 0; j < limit; j++)
         if (st.lane_ok[v0 + j * Cr]) { jstar = j; break; }
@@ -506,6 +544,24 @@ __global__ void __launch_bounds__(128) k_la_resolve(ChainParams P, StateDev st, 
             }
             if (st.lane_status[v]) st.status[c] |= st.lane_status[v];
         }
+    }
+    if (st.sx.pending) {
+        // statistics, as k_chain_accept does them step by step: the rejected steps' records belong to the old state, which
+        // an accepting lane flushes; the accepting step's record belongs to the new state
+        __shared__ int s_flush;
+        if (threadIdx.x == 0) {
+            long long pend = st.sx.pending[c];
+            for (int j = 0; j < consumed; j++)
+                if (j != jstar) pend += stats_selected(st.sx, (long long)s0 + j);
+            const int flush = jstar >= 0 && pend > 0;
+            st.sx.flush_w[c] = flush ? pend : 0;
+            if (flush) { st.sx.flush_n[c] = st.sx.count[c]; st.sx.count[c] += pend; }
+            st.sx.pending[c] = jstar >= 0 ? stats_selected(st.sx, (long long)s0 + jstar) : pend;
+            s_flush = flush;
+        }
+        __syncthreads();
+        if (s_flush)
+            for (int k = threadIdx.x; k < Lt; k += blockDim.x) st.sx.flush_theta[(size_t)c * Lt + k] = cur[k];
     }
     __syncthreads();   // the log rows above read the old current state
     if (jstar >= 0) {
@@ -587,6 +643,12 @@ struct icp_chain_s {
     DevBuf<double> d_theta0, d_final;   // persistent staging of the host-buffer entry point
     DevBuf<long long> d_nacc;
     int steps_total = 0;     // value of the device step counter
+    // posterior variability inside the run: requested parameters (icp_chain_set_statistics) and those of the resident run
+    bool stats_req_on = false, stats_on = false;
+    icp_chain_stats_params stats_req{}, stats_run{};
+    DevBuf<long long> sx_pending, sx_count, sx_flush_w, sx_flush_n;   // StatsDev
+    DevBuf<double> sx_flush_theta, sx_mean, sx_m2, sx_nsum;          // StatsDev.flush_theta, StatsAcc
+    DevBuf<int> sx_idx, sx_nlist;                                    // launch_stats_flush's list of flushed chains
 };
 
 extern "C" int32_t icp_chain_create(icp_model m, icp_target t, const icp_component *components, int32_t n_components,
@@ -798,6 +860,14 @@ void enqueue_step(RunCtx &r) {
         else k_step_increment<<<1, 1, 0, r.s>>>(r.st.step);
         ICP_CUDA(cudaGetLastError());
     }
+    if (r.st.sx.pending) {
+        // statistics: the states the chains flushed in this step / round into their accumulators (stats.cu). ch->X, the
+        // meshes of this step's proposals, is free until the next step reconstructs into it.
+        ProfScope ps(ST_OTHER, r.s);
+        const StatsDev &x = r.st.sx;
+        launch_stats_flush(m->dev(), r.Cr, x.flush_theta, x.flush_w, x.flush_n, ch->sx_idx.p, ch->sx_nlist.p, ch->X.p,
+                           StatsAcc{ch->sx_mean.p, ch->sx_m2.p, ch->stats_run.normals ? ch->sx_nsum.p : nullptr}, r.s);
+    }
 }
 
 // Width of the rejection look-ahead a run of C chains will use (1 = the plain step-by-step runner). Off while profiling, with
@@ -861,6 +931,29 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
                     ch->slot_cur.p, ch->slot_prop.p, ch->comp_sel.p, ch->u_acc.p, ch->n_acc.p, ch->step.p, ch->L.p,
                     ch->mu.p, ch->any_svd ? ch->W.p : nullptr, ch->status.p, ch->theta_best.p, ch->value_best.p,
                     ch->qf.p, ch->qb.p, ch->lane_ok.p, ch->lane_status.p, ch->step_end.p};
+    if (!resume) { ch->stats_on = ch->stats_req_on; ch->stats_run = ch->stats_req; }
+    r.st.sx = StatsDev{};
+    if (ch->stats_on) {
+        const size_t nv = (size_t)Cr * m->N;
+        ch->sx_pending.ensure(Cr); ch->sx_count.ensure(Cr); ch->sx_flush_w.ensure(Cr); ch->sx_flush_n.ensure(Cr);
+        ch->sx_flush_theta.ensure((size_t)Cr * Lt); ch->sx_idx.ensure(Cr); ch->sx_nlist.ensure(1);
+        ch->sx_mean.ensure(nv * 3); ch->sx_m2.ensure(nv * 6);
+        if (ch->stats_run.normals) ch->sx_nsum.ensure(nv * 3);
+        if (!resume) {
+            ICP_CUDA(cudaMemsetAsync(ch->sx_pending.p, 0, sizeof(long long) * Cr, s));
+            ICP_CUDA(cudaMemsetAsync(ch->sx_count.p, 0, sizeof(long long) * Cr, s));
+            ICP_CUDA(cudaMemsetAsync(ch->sx_flush_w.p, 0, sizeof(long long) * Cr, s));
+            ICP_CUDA(cudaMemsetAsync(ch->sx_mean.p, 0, sizeof(double) * nv * 3, s));
+            ICP_CUDA(cudaMemsetAsync(ch->sx_m2.p, 0, sizeof(double) * nv * 6, s));
+            if (ch->stats_run.normals) ICP_CUDA(cudaMemsetAsync(ch->sx_nsum.p, 0, sizeof(double) * nv * 3, s));
+        }
+        r.st.sx = StatsDev{ch->sx_pending.p, ch->sx_count.p, ch->sx_flush_w.p, ch->sx_flush_n.p, ch->sx_flush_theta.p,
+                           ch->stats_run.burn_in, ch->stats_run.take_every_n, ch->stats_run.end};
+    } else if (!resume) {   // allocated only while statistics are on
+        ch->sx_pending.release(); ch->sx_count.release(); ch->sx_flush_w.release(); ch->sx_flush_n.release();
+        ch->sx_flush_theta.release(); ch->sx_idx.release(); ch->sx_nlist.release();
+        ch->sx_mean.release(); ch->sx_m2.release(); ch->sx_nsum.release();
+    }
     const int step_base = resume ? ch->steps_total : 0;
     r.rng = RngDev{io->seed, io->chain_id_offset, io->u_comp, io->z, io->u_acc, step_base};
     r.lg = LogDev{io->log_component, io->log_accepted, io->log_values, io->log_theta, step_base};
@@ -954,6 +1047,12 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
         key.append((const char *)&r.st, sizeof r.st);
         key.append((const char *)&r.rng, sizeof r.rng);
         key.append((const char *)&r.lg, sizeof r.lg);
+        key.push_back(ch->stats_on ? 1 : 0);   // the flush kernels are part of the step graph while statistics are on
+        if (ch->stats_on) {
+            const void *sx[] = {ch->sx_mean.p, ch->sx_m2.p, ch->stats_run.normals ? ch->sx_nsum.p : nullptr, ch->sx_idx.p,
+                                ch->sx_nlist.p, ch->X.p};
+            key.append((const char *)sx, sizeof sx);
+        }
         {   // buffers the captured kernels address that are not part of the descriptors above: the pipelines' status words
             // and the MODEL's BVH scratch, which other calls on the same model may reallocate (a replay would dangle)
             StatusSrc ss = status_sources(ch);
@@ -1268,6 +1367,104 @@ extern "C" int32_t icp_chain_last_run_rounds(icp_chain c, int64_t *rounds) {
     if (!c || !rounds) return ICP_ERR_INVALID_ARGUMENT;
     *rounds = c->last_rounds;
     return ICP_OK;
+}
+
+extern "C" int32_t icp_chain_set_statistics(icp_chain c, const icp_chain_stats_params *p) {
+    icp_ctx _ctx = c ? c->model->ctx : nullptr;
+    try {
+        ICP_REQUIRE(_ctx != nullptr, "null handle");
+        CtxLock lock(_ctx);
+        if (p) {
+            ICP_REQUIRE(p->take_every_n >= 1, "take_every_n must be >= 1");
+            ICP_REQUIRE(p->burn_in >= 0, "burn_in must be >= 0");
+            ICP_REQUIRE(p->normals == 0 || p->normals == 1, "normals must be 0 or 1");
+            c->stats_req = *p;
+        }
+        c->stats_req_on = p != nullptr;
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
+    }
+}
+
+// Reads the maps without changing the accumulators: copies of the chains' partials take their pending weight (the current
+// state) as one more flush, the partials are merged in chain order and finished with the direction chosen here.
+extern "C" int32_t icp_chain_statistics(icp_chain c, int32_t chain, int32_t sum_normals, const double *theta_ref,
+                                        int64_t *n_samples, double *mean, double *cov, double *total_variance,
+                                        double *normal_variance) {
+    icp_ctx _ctx = c ? c->model->ctx : nullptr;
+    try {
+        ICP_REQUIRE(_ctx != nullptr, "null handle");
+        CtxLock lock(_ctx);
+        ICP_REQUIRE(c->stats_on && c->resident_C > 0,
+                    "statistics were off for the resident run (icp_chain_set_statistics, then a run from theta0)");
+        const int Cr = c->resident_C;
+        ICP_REQUIRE(chain >= -1 && chain < Cr, "chain must be -1 (pooled) or in [0, C) of the resident run");
+        ICP_REQUIRE(!sum_normals || c->stats_run.normals, "sum_normals needs statistics accumulated with normals = 1");
+        icp_model m = c->model;
+        cudaStream_t s = _ctx->stream;
+        const int N = m->N, Lt = m->K + kTheta0;
+        const int c0 = chain < 0 ? 0 : chain, n = chain < 0 ? Cr : 1;
+        const size_t nv = (size_t)n * N;
+        const bool nrm = c->stats_run.normals != 0;
+        DevBuf<long long> cnt, w, n_old;
+        DevBuf<double> mu, q, ns, pmu, pq, pns, refX, refN, d_mean, tot7, d_cov, d_total, d_along;
+        DevBuf<int> idx, nlist;
+        cnt.alloc(n); w.alloc(n); n_old.alloc(n); idx.alloc(n); nlist.alloc(1);
+        mu.alloc(nv * 3); q.alloc(nv * 6);
+        ICP_CUDA(cudaMemcpyAsync(cnt.p, c->sx_count.p + c0, sizeof(long long) * n, cudaMemcpyDeviceToDevice, s));
+        ICP_CUDA(cudaMemcpyAsync(mu.p, c->sx_mean.p + (size_t)c0 * N * 3, sizeof(double) * nv * 3, cudaMemcpyDeviceToDevice, s));
+        ICP_CUDA(cudaMemcpyAsync(q.p, c->sx_m2.p + (size_t)c0 * N * 6, sizeof(double) * nv * 6, cudaMemcpyDeviceToDevice, s));
+        if (nrm) {
+            ns.alloc(nv * 3);
+            ICP_CUDA(cudaMemcpyAsync(ns.p, c->sx_nsum.p + (size_t)c0 * N * 3, sizeof(double) * nv * 3, cudaMemcpyDeviceToDevice, s));
+        }
+        const StatsAcc acc{mu.p, q.p, nrm ? ns.p : nullptr};
+        // the current state of every chain (look-ahead: lane 0 = the first Cr entries) with its pending weight
+        launch_stats_pending(n, c->sx_pending.p + c0, cnt.p, w.p, n_old.p, s);
+        c->X.ensure(nv * 3);
+        launch_stats_flush(m->dev(), n, c->theta_cur.p + (size_t)c0 * Lt, w.p, n_old.p, idx.p, nlist.p, c->X.p, acc, s);
+        std::vector<long long> h_cnt(n);
+        ICP_CUDA(cudaMemcpyAsync(h_cnt.data(), cnt.p, sizeof(long long) * n, cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaStreamSynchronize(s));
+        long long S = 0;
+        for (long long v : h_cnt) S += v;
+        if (n_samples) *n_samples = S;
+        ICP_REQUIRE(S >= 1, "no selected record: the run has not reached burn_in (or end <= burn_in)");
+        ICP_REQUIRE(S <= 0x7fffffffLL, "more than 2^31 - 1 samples");
+        pmu.alloc((size_t)N * 3); pq.alloc((size_t)N * 6);
+        if (nrm) pns.alloc((size_t)N * 3);
+        launch_stats_pool(n, N, cnt.p, acc, pmu.p, pq.p, nrm ? pns.p : nullptr, s);
+        const double *ref_normals = nullptr;
+        if (!sum_normals) {
+            // normals of transformedMesh(theta_ref), or of the model's reference mesh when theta_ref is NULL
+            refN.alloc((size_t)N * 3);
+            const double *rx = m->ref.p;
+            DevBuf<double> th;
+            if (theta_ref) {
+                th.upload(theta_ref, (size_t)Lt, s);
+                refX.alloc((size_t)N * 3);
+                launch_reconstruct(m->dev(), 1, th.p, refX.p, s);
+                rx = refX.p;
+                ICP_CUDA(cudaStreamSynchronize(s));   // th leaves scope
+            }
+            launch_vertex_normals(m->dev(), 1, rx, refN.p, s);
+            ref_normals = refN.p;
+        }
+        d_mean.alloc((size_t)N * 3); tot7.alloc((size_t)N * 7); d_cov.alloc((size_t)N * 9); d_total.alloc(N); d_along.alloc(N);
+        launch_stats_moments(N, S, pmu.p, pq.p, nrm ? pns.p : nullptr, ref_normals, d_mean.p, tot7.p, s);
+        launch_var_finish((int)S, N, tot7.p, d_cov.p, d_total.p, d_along.p, s);
+        auto dl = [&](double *h, const double *d, size_t cnt_) {
+            if (h) ICP_CUDA(cudaMemcpyAsync(h, d, cnt_ * sizeof(double), cudaMemcpyDeviceToHost, s));
+        };
+        dl(mean, d_mean.p, (size_t)N * 3); dl(cov, d_cov.p, (size_t)N * 9); dl(total_variance, d_total.p, N);
+        dl(normal_variance, d_along.p, N);
+        ICP_CUDA(cudaStreamSynchronize(s));
+        return ICP_OK;
+    } catch (...) {
+        if (_ctx) cudaStreamSynchronize(_ctx->stream);   // no copy may outlive the call's buffers
+        return translate_exception(_ctx);
+    }
 }
 
 // Philox block exactly as the chain runner draws it (integer-exact check against the oracle)

@@ -277,6 +277,12 @@ __global__ void k_var_finish(int S, int N, int P, const double *__restrict__ par
     along[v] = a[6];
 }
 
+// the finish of the maps the chain runner accumulates (icp_chain_statistics, stats.cu)
+void icp::launch_var_finish(int S, int N, const double *d_tot7, double *d_cov, double *d_total, double *d_along, cudaStream_t s) {
+    k_var_finish<<<(N + kVarThreads - 1) / kVarThreads, kVarThreads, 0, s>>>(S, N, 1, d_tot7, d_cov, d_total, d_along);
+    ICP_CUDA(cudaGetLastError());
+}
+
 
 // per-vertex totals over the partitions (deterministic partition order): tot[v][W] = sum_p part[p][v][W]
 template <int W>

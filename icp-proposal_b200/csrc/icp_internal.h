@@ -212,6 +212,26 @@ struct ModelDev {  // plain device view, passed by value to kernels
 void launch_reconstruct(const ModelDev &m, int C, const double *d_theta, double *d_X, cudaStream_t s);
 void launch_vertex_normals(const ModelDev &m, int C, const double *d_X, double *d_normals, cudaStream_t s);
 void launch_gram(const ModelDev &m, double *d_G /*Kp x Kp*/, cudaStream_t s);
+
+// ---- posterior variability accumulated inside the chain runner (stats.cu) ------------------------------------------
+struct StatsAcc {   // per-chain accumulators: mean [C][N][3], centred second moment [C][N][6] (xx yy zz xy xz yz), unit-normal sum
+    double *mean, *m2, *nsum;   // [C][N][3] (nullable)
+};
+// one weighted Welford / Chan update of every chain c with d_w[c] > 0: the mesh of d_theta[c] (and its unit vertex normals)
+// with weight d_w[c] into accumulators that held d_n_old[c] samples. d_idx [C] / d_count [1]: scratch for the list of those
+// chains; d_X: [C][N][3] scratch for their meshes.
+void launch_stats_flush(const ModelDev &m, int C, const double *d_theta, const long long *d_w, const long long *d_n_old,
+                        int *d_idx, int *d_count, double *d_X, const StatsAcc &acc, cudaStream_t s);
+// w = pending, n_old = count, count += pending (the read-out merges the chains' pending weight into copies)
+void launch_stats_pending(int C, const long long *d_pending, long long *d_count, long long *d_w, long long *d_n_old, cudaStream_t s);
+// Chan's merge of the C chains' partials in chain order into [N] arrays (d_nsum / acc.nsum nullable together)
+void launch_stats_pool(int C, int N, const long long *d_count, const StatsAcc &acc, double *d_mean, double *d_m2, double *d_nsum,
+                       cudaStream_t s);
+// mean out and the [N][7] moments k_var_finish reads, along the reference normals or (NULL) the mean unit normal d_nsum / S
+void launch_stats_moments(int N, long long S, const double *d_mean, const double *d_m2, const double *d_nsum, const double *d_ref_normals,
+                          double *d_mean_out, double *d_tot7, cudaStream_t s);
+// k_var_finish (comm.cu): [N][7] moments of S samples -> cov [N][9], total [N], along [N]
+void launch_var_finish(int S, int N, const double *d_tot7, double *d_cov, double *d_total, double *d_along, cudaStream_t s);
 void launch_scale_basis(int rows, int K, int Kp, const double *d_U, const double *d_var, double *d_Q, double *d_QT,
                         cudaStream_t s);
 

@@ -529,12 +529,22 @@ public:
         int64_t accepted = 0;
         int steps = 0;
         std::vector<jsonLogFormat> log;   // the chain log in the reference's record layout (also written to jsonName)
+        int64_t variabilitySamples = 0;   // with a variability request: S, and the maps (PosteriorVariability layout)
+        PosteriorVariability::Maps variability;
+    };
+    // PosteriorVariability over the samples LogHelper.samplesFromLog(log, takeEveryN, total, burnIn) selects, accumulated
+    // inside the run (icp_chain_set_statistics / icp_chain_statistics) instead of from the chain log
+    struct VariabilityRequest {
+        int64_t takeEveryN = 50, total = 0, burnIn = 0;   // total <= 0: no limit
+        bool sumNormals = true;
+        const ModelFittingParameters *ref = nullptr;      // sumNormals == false: normals of this state (nullptr: reference mesh)
     };
     // evaluator: the device evaluator behind evaluators("product") - build it with makeProductEvaluator so that it
     // carries prior x distance (ProductEvaluators.scala:44-47); distanceKey: the key of the distance term in the
     // evaluator map ("distance", "distance_haussdorff", "collective_distance")
     Result runfitting(DeviceDistanceEvaluator &evaluator, const std::string &distanceKey, ProposalGeneratorWithTransition &generator,
-                      int numOfSamples, const ModelFittingParameters &initial, const std::string &jsonName = "") {
+                      int numOfSamples, const ModelFittingParameters &initial, const std::string &jsonName = "",
+                      const VariabilityRequest *variability = nullptr) {
         std::vector<icp_component> comps;
         std::vector<std::string> names;
         generator.flatten(1.0, comps, names);
@@ -550,10 +560,23 @@ public:
         io.seed = seed_;
         io.log_component = comp.data(); io.log_accepted = acc.data(); io.log_values = vals.data(); io.log_theta = thl.data();
         io.theta_final = fin.data(); io.n_accepted = &nacc;
-        int32_t rc = icp_chain_run(chain, 1, numOfSamples, initial.allParameters.data(), &io);
+        Result r;
+        int32_t rc = ICP_OK;
+        if (variability) {
+            icp_chain_stats_params sp{variability->burnIn, variability->takeEveryN, variability->total, variability->sumNormals ? 1 : 0, 0};
+            rc = icp_chain_set_statistics(chain, &sp);
+        }
+        if (rc == ICP_OK) rc = icp_chain_run(chain, 1, numOfSamples, initial.allParameters.data(), &io);
+        if (rc == ICP_OK && variability) {
+            const int N = model_.numberOfPoints();
+            PosteriorVariability::Maps &v = r.variability;
+            v.mean.resize((size_t)3 * N); v.cov.resize((size_t)9 * N); v.total.resize(N); v.normal.resize(N);
+            const ModelFittingParameters *ref = variability->sumNormals ? nullptr : variability->ref;
+            rc = icp_chain_statistics(chain, -1, variability->sumNormals ? 1 : 0, ref ? ref->allParameters.data() : nullptr,
+                                      &r.variabilitySamples, v.mean.data(), v.cov.data(), v.total.data(), v.normal.data());
+        }
         icp_chain_destroy(chain);
         check(rc, model_.ctx());
-        Result r;
         r.best = initial; r.accepted = nacc; r.steps = numOfSamples;
         JSONAcceptRejectLogger logger(jsonName);
         for (int s = 0; s < numOfSamples; s++) {

@@ -326,6 +326,31 @@ int32_t icp_chain_last_run_stats(icp_chain c, double *device_ms, int64_t *kernel
 int32_t icp_chain_set_lookahead(icp_chain c, int32_t width);
 int32_t icp_chain_last_run_rounds(icp_chain c, int64_t *rounds);
 
+/* Posterior variability maps accumulated inside the run: icp_posterior_variability over the states LogHelper.samplesFromLog
+ * (apps/util/LogHelper.scala:25-42) would select from the chain log, without a chain log, per chain or pooled.
+ * Record i of a chain is its i-th step since theta0 (resumed runs keep counting); it is selected when
+ * burn_in <= i < end (end <= 0: no limit) and (i - burn_in) % take_every_n == 0, and its sample is the state current after
+ * that step (row i of log_theta). Unlike LogHelper, which fails there, a selected record before the chain's first acceptance
+ * counts theta0. Each chain keeps FP64 accumulators on the device: a count and per vertex the mean, the centred second
+ * moment and (normals = 1) the sum of unit vertex normals - 12 N doubles per chain. They are updated when a chain accepts,
+ * once per accepted state with the number of selected records at which that state was current, so the step-by-step
+ * runner, the rejection look-ahead at any width and runs split by resume produce bit-identical maps. */
+typedef struct {
+    int64_t burn_in;        /* LogHelper burnIn, >= 0 */
+    int64_t take_every_n;   /* LogHelper takeEveryN, >= 1 */
+    int64_t end;            /* LogHelper total: records below it; <= 0 = no limit */
+    int32_t normals;        /* 1: also accumulate unit vertex normals (needed to read with sum_normals != 0) */
+    int32_t reserved;
+} icp_chain_stats_params;
+/* NULL = off. Takes effect at the next run from theta0, which zeroes the accumulators; resumed runs keep accumulating. */
+int32_t icp_chain_set_statistics(icp_chain c, const icp_chain_stats_params *p);
+/* chain in [0, C) of the resident run, or -1 = pooled over all its chains (Chan's merge in chain order, on the device).
+ * Outputs (host memory) in the layout of icp_posterior_variability; any may be NULL; the direction of normal_variance is
+ * chosen here (sum_normals, theta_ref as there). n_samples: S. Reading leaves the accumulators unchanged. Error if
+ * statistics were off for the resident run, or if S == 0; S == 1 yields NaN variances. */
+int32_t icp_chain_statistics(icp_chain c, int32_t chain, int32_t sum_normals, const double *theta_ref,
+                             int64_t *n_samples, double *mean, double *cov, double *total_variance, double *normal_variance);
+
 /* ---- (7b) chain log in the reference's JSON wire format (host functions: no CUDA context needed) ---------------------- */
 /* JSONAcceptRejectLogger (api/sampling/loggers/JSONAcceptRejectLogger.scala:35,93-127) as a streaming writer and a loader.
  * The reference rewrites the whole file on every writeLog (:112-122), quadratic over a run; icp_jsonlog_append appends the
