@@ -16,7 +16,8 @@ ERR_INVALID_ARGUMENT, ERR_CUDA, ERR_OUT_OF_MEMORY, ERR_EMPTY_SET, ERR_NOT_POSITI
 CHAIN_EMPTY_SET, CHAIN_NOT_POSITIVE_DEFINITE, CHAIN_NAN_TRANSITION, CHAIN_NAN_VALUE = 1, 2, 4, 8
 FACTOR_CHOLESKY, FACTOR_SVD = 0, 1
 RANK_UPDATE_FP64, RANK_UPDATE_INT8 = 0, 1
-MODEL_SAMPLING, TARGET_SAMPLING = 0, 1
+MODEL_SAMPLING, TARGET_SAMPLING, MODEL_AND_TARGET_SAMPLING = 0, 1, 2
+STD_ICP_NON_FINITE, STD_ICP_NOT_POSITIVE_DEFINITE = 1, 2
 EVAL_ACCEPT_ALL, EVAL_INDEPENDENT, EVAL_HAUSDORFF, EVAL_COLLECTIVE = 0, 1, 2, 3
 MODEL_TO_TARGET, TARGET_TO_MODEL, SYMMETRIC = 0, 1, 2
 PROP_ICP, PROP_RANDOM_SHAPE, PROP_ROTATION, PROP_TRANSLATION = 0, 1, 2, 3
@@ -66,6 +67,11 @@ class ChainIO(C.Structure):
                 ("metrics_interval", C.c_int32), ("reserved", C.c_int32), ("log_metrics", C.c_void_p)]
 
 
+class StdIcpIO(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("fit_id_offset", C.c_uint64), ("directions", C.c_void_p), ("alpha_final", C.c_void_p),
+                ("log_alpha", C.c_void_p), ("log_direction", C.c_void_p), ("status", C.c_void_p), ("iterations_done", C.c_void_p)]
+
+
 class ChainStatsParams(C.Structure):
     _fields_ = [("burn_in", C.c_int64), ("take_every_n", C.c_int64), ("end", C.c_int64), ("normals", C.c_int32),
                 ("reserved", C.c_int32)]
@@ -98,6 +104,11 @@ _SIGS = {
     "icp_proposal_clear_cache": [_h],
     "icp_std_icp_iteration": [_h, _h, C.c_int32, _ip, C.c_int32, _dp, C.c_int32, C.c_double, C.c_double, C.c_int32, _dp, _dp],
     "icp_std_icp_iteration_theta": [_h, _h, C.c_int32, _ip, C.c_int32, _dp, C.c_int32, C.c_double, C.c_double, C.c_int32, _dp, _dp],
+    "icp_std_icp_create": [_h, _h, _ip, C.c_int32, _dp, C.c_int32, C.c_double, C.c_int32, C.c_int32, C.POINTER(_h)],
+    "icp_std_icp_destroy": [_h],
+    "icp_std_icp_run": [_h, C.c_int32, _dp, C.c_int32, _dp, C.c_int32, C.POINTER(StdIcpIO)],
+    "icp_std_icp_run_device": [_h, C.c_int32, C.c_void_p, C.c_int32, _dp, C.c_int32, C.POINTER(StdIcpIO), C.c_int32],
+    "icp_std_icp_last_run_stats": [_h, _dp, _lp],
     "icp_evaluator_create": [_h, _h, C.POINTER(EvaluatorParams), _ip, C.c_int32, _dp, C.c_int32, C.POINTER(_h)],
     "icp_evaluator_destroy": [_h],
     "icp_eval_log_value": [_h, C.c_int32, _dp, _dp, _ip],

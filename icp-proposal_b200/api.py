@@ -794,19 +794,34 @@ class IcpBasedSurfaceFitting:
         self.tp = _decimated_points(target, numOfSamplePoints) if target_points is None else np.asarray(target_points, float)
 
     def runfitting(self, numIterations, iterationSeq=(1.0, 0.1, 0.01), initialCoefficients=None, directions=None):
-        alpha = np.zeros((1, self.model.K)) if initialCoefficients is None else np.asarray(initialCoefficients, float).reshape(1, -1)
-        it = 0
-        for sigma in iterationSeq:
-            for _ in range(numIterations + 1):                 # recursion runs numIterations + 1 times per sigma (:55-109)
-                if self.projectionDirection == ModelAndTargetSampling:
-                    d = directions[it] if directions is not None else (ModelSampling if self.rand.random() < 0.5 else TargetSampling)
-                else:
-                    d = self.projectionDirection
-                alpha = core.std_icp_iteration(self.model, self.target, _lib.TARGET_SAMPLING if d == TargetSampling else _lib.MODEL_SAMPLING,
-                                               self.ids, self.tp, sigma, self.stepLength, alpha)
-                it += 1
-        self.coefficients = alpha[0]
-        return self.model.instance(alpha[0])
+        """The whole loop on the device (core.StdIcp). initialCoefficients of shape (C, K) runs C independent fits and returns
+        C instances (self.coefficients becomes C x K); directions is then (iterations, C) or (iterations,) for all fits. With
+        ModelAndTargetSampling and no directions the coin is self.rand, drawn iteration by iteration (fit by fit) as before."""
+        K = self.model.K
+        batched = initialCoefficients is not None and np.ndim(initialCoefficients) == 2
+        alpha = np.zeros((1, K)) if initialCoefficients is None else np.asarray(initialCoefficients, float).reshape(-1, K)
+        n_fits = len(alpha)
+        iters = len(iterationSeq) * (numIterations + 1)        # recursion runs numIterations + 1 times per sigma (:55-109)
+        if self.projectionDirection == ModelAndTargetSampling:
+            if directions is None:
+                target = self.rand.random((iters, n_fits)) >= 0.5
+            else:
+                target = np.asarray(directions, dtype=object) == TargetSampling
+                target = np.broadcast_to(target.reshape(iters, -1), (iters, n_fits))
+        else:
+            target = np.full((iters, n_fits), self.projectionDirection == TargetSampling)
+        theta0 = np.stack([self.model.theta(alpha=a, center=(0, 0, 0)) for a in alpha])
+        runner = core.StdIcp(self.model, self.target, self.ids, self.tp, self.stepLength, _lib.MODEL_SAMPLING, n_fits)
+        try:
+            out = runner.run(theta0, np.asarray(iterationSeq, float), numIterations,
+                             directions=np.where(target, _lib.TARGET_SAMPLING, _lib.MODEL_SAMPLING), log=False)
+        finally:
+            runner.close()
+        if batched:
+            self.coefficients = out["alpha_final"]
+            return [self.model.instance(a) for a in out["alpha_final"]]
+        self.coefficients = out["alpha_final"][0]
+        return self.model.instance(out["alpha_final"][0])
 
 
 class RegistrationComparison:

@@ -12,7 +12,7 @@ CSRC = os.path.join(HERE, "csrc")
 _TAG = os.environ.get("ICPCUDA_LIB_TAG", "")
 OBJ = os.path.join(HERE, "build" + ("_" + _TAG if _TAG else ""))
 LIB = os.path.join(HERE, "libicpcuda" + ("_" + _TAG if _TAG else "") + ".so")
-SOURCES = ["api.cu", "bvh.cu", "model.cu", "posterior.cu", "evaluate.cu", "chain.cu", "debug.cu", "gpmm.cu", "svdfactor.cu", "metrics.cu", "bvh_wide.cu", "comm.cu", "jsonlog.cu", "tc_i8.cu", "stats.cu"]
+SOURCES = ["api.cu", "bvh.cu", "model.cu", "posterior.cu", "evaluate.cu", "chain.cu", "debug.cu", "gpmm.cu", "svdfactor.cu", "metrics.cu", "bvh_wide.cu", "comm.cu", "jsonlog.cu", "tc_i8.cu", "stats.cu", "stdicp.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr"] + os.environ.get("ICPCUDA_NVCC_EXTRA", "").split()
 

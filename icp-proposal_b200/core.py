@@ -246,6 +246,62 @@ def std_icp_iteration_theta(model: Model, target: Target, direction, model_point
     return out
 
 
+class StdIcp:
+    """Device-resident IcpBasedSurfaceFitting.runfitting for batches of independent fits (icp_std_icp_*)."""
+
+    def __init__(self, model: Model, target: Target, model_point_ids, target_points, step_length=1.0,
+                 direction=_lib.MODEL_SAMPLING, max_fits=1):
+        self.model, self.target, self.lib, self.ctx = model, target, model.lib, model.ctx
+        self.ids = i32(np.asarray(model_point_ids).reshape(-1))
+        self.tp = f64(np.asarray(target_points, dtype=np.float64).reshape(-1, 3))
+        self.max_fits = int(max_fits)
+        self.h = C.c_void_p()
+        check(self.lib.icp_std_icp_create(model.h, target.h, iptr(self.ids), len(self.ids), dptr(self.tp), len(self.tp),
+                                          float(step_length), int(direction), self.max_fits, C.byref(self.h)), self.ctx.h)
+
+    def run(self, theta0, sigma2, num_iterations, directions=None, seed=1024, fit_id_offset=0, log=True):
+        """theta0 (C, K + 10); sigma2: iterationSeq; directions (iters, C) or None. Returns dict(alpha_final (C, K), status (C,),
+        iterations_done (C,), and with log=True log_alpha (iters, C, K) and log_direction (iters, C))."""
+        th, c = self.model._theta(theta0)
+        s2 = f64(np.atleast_1d(sigma2))
+        K, iters = self.model.K, len(s2) * (int(num_iterations) + 1)
+        io = _lib.StdIcpIO()
+        io.seed, io.fit_id_offset = int(seed), int(fit_id_offset)
+        d = None
+        if directions is not None:
+            d = i32(directions).reshape(iters, c)
+            io.directions = d.ctypes.data
+        out = dict(alpha_final=np.empty((c, K)), status=np.zeros(c, np.int32), iterations_done=np.zeros(c, np.int32))
+        io.alpha_final, io.status, io.iterations_done = (out[k].ctypes.data for k in ("alpha_final", "status", "iterations_done"))
+        if log:
+            out["log_alpha"], out["log_direction"] = np.empty((iters, c, K)), np.empty((iters, c), np.int32)
+            io.log_alpha, io.log_direction = out["log_alpha"].ctypes.data, out["log_direction"].ctypes.data
+        check(self.lib.icp_std_icp_run(self.h, c, dptr(th), len(s2), dptr(s2), int(num_iterations), C.byref(io)), self.ctx.h)
+        return out
+
+    def run_device(self, C_, theta0_ptr, sigma2, num_iterations, directions=0, seed=1024, fit_id_offset=0, alpha_final=0,
+                   log_alpha=0, log_direction=0, status=0, iterations_done=0, async_=False):
+        """All pointers are raw device addresses (e.g. torch.Tensor.data_ptr()); sigma2 is a host sequence."""
+        s2 = f64(np.atleast_1d(sigma2))
+        io = _lib.StdIcpIO()
+        io.seed, io.fit_id_offset, io.directions = int(seed), int(fit_id_offset), directions or None
+        io.alpha_final, io.log_alpha, io.log_direction = alpha_final or None, log_alpha or None, log_direction or None
+        io.status, io.iterations_done = status or None, iterations_done or None
+        check(self.lib.icp_std_icp_run_device(self.h, int(C_), theta0_ptr, len(s2), dptr(s2), int(num_iterations), C.byref(io),
+                                              int(async_)), self.ctx.h)
+
+    def last_run_stats(self):
+        """(device milliseconds, kernel launches) of the last run."""
+        ms = C.c_double(0); n = C.c_int64(0)
+        check(self.lib.icp_std_icp_last_run_stats(self.h, C.byref(ms), C.byref(n)))
+        return ms.value, n.value
+
+    def close(self):
+        if self.h:
+            self.lib.icp_std_icp_destroy(self.h)
+            self.h = None
+
+
 class Evaluator:
     """Device side of the DistributionEvaluators (api/sampling/evaluators/*.scala)."""
 

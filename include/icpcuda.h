@@ -180,6 +180,48 @@ int32_t icp_std_icp_iteration_theta(icp_model m, icp_target t, int32_t direction
                                     int32_t n_ids, const double *target_points, int32_t n_tp, double sigma2,
                                     double step_length, int32_t C, const double *theta, double *alpha_out);
 
+/* ---- (5b) IcpBasedSurfaceFitting.runfitting on the device (api/other/IcpBasedSurfaceFitting.scala:46-126) ----------- */
+/* The whole deterministic-ICP loop for C independent fits: every sigma2 of iterationSeq runs num_iterations + 1 iterations
+ * (:55-109), each one the icp_std_icp_iteration_theta of its fit, with the rigid transform of theta0 (currentTrans, :61) fixed
+ * and only the coefficients moving. Iterations are replayed CUDA graphs; a run synchronises once. */
+#define ICP_MODEL_AND_TARGET_SAMPLING 2   /* IcpProjectionDirection.scala: a coin per iteration (:67); icp_std_icp only */
+typedef struct icp_std_icp_s *icp_std_icp;
+/* model_point_ids / target_points as for icp_std_icp_iteration (uploaded once; n_ids, n_tp >= 1). direction: the direction
+ * of every iteration unless a run supplies its own: ICP_MODEL_SAMPLING, ICP_TARGET_SAMPLING or ICP_MODEL_AND_TARGET_SAMPLING
+ * (a Philox coin, see icp_std_icp_io). The handle holds references on the model and the target. */
+int32_t icp_std_icp_create(icp_model m, icp_target t, const int32_t *model_point_ids, int32_t n_ids, const double *target_points,
+                           int32_t n_tp, double step_length, int32_t direction, int32_t max_fits, icp_std_icp *out);
+int32_t icp_std_icp_destroy(icp_std_icp h);
+/* per-fit status words (icp_std_icp_io.status): where the reference catches an exception and returns the last coefficients
+ * (:94-104), that fit stops: it keeps its coefficients for the rest of the run, its later log rows repeat them and
+ * iterations_done stops counting. The other fits are unaffected and the run returns ICP_OK. */
+#define ICP_STD_ICP_NON_FINITE 1             /* theta0 or the new coefficients were not finite */
+#define ICP_STD_ICP_NOT_POSITIVE_DEFINITE 2  /* the posterior's factorisation failed */
+typedef struct {
+    /* directions == NULL with ICP_MODEL_AND_TARGET_SAMPLING: fit c flips a coin in iteration i with Philox4x32-10 keyed by seed,
+     * counter (fit_id_offset + c, i, block 0) as in icp_chain_io: u = 53-bit uniform of words x (high) and y (low), model
+     * sampling when u < 0.5. Results do not depend on how fits are batched or sharded over GPUs. */
+    uint64_t seed;
+    uint64_t fit_id_offset;
+    const int32_t *directions;  /* [iters][C] ICP_MODEL_SAMPLING | ICP_TARGET_SAMPLING, or NULL; iters = n_sigma (num_iterations + 1) */
+    /* outputs, any may be NULL */
+    double *alpha_final;        /* [C][K] */
+    double *log_alpha;          /* [iters][C][K] coefficients after every iteration */
+    int32_t *log_direction;     /* [iters][C] */
+    int32_t *status;            /* [C] OR of ICP_STD_ICP_* */
+    int32_t *iterations_done;   /* [C] iterations completed before the fit stopped (iters when it never did) */
+} icp_std_icp_io;
+/* theta0 C x (K+10), sigma2 n_sigma values > 0 (iterationSeq), 1 <= C <= max_fits. Host buffers. */
+int32_t icp_std_icp_run(icp_std_icp h, int32_t C, const double *theta0, int32_t n_sigma, const double *sigma2,
+                        int32_t num_iterations, const icp_std_icp_io *io);
+/* the same with theta0_dev and every io pointer in DEVICE memory (sigma2 stays a host array). Caller directions are read
+ * back to the host before the run is enqueued (the split of every iteration is planned there); the run is synchronised before
+ * returning unless async != 0. */
+int32_t icp_std_icp_run_device(icp_std_icp h, int32_t C, const double *theta0_dev, int32_t n_sigma, const double *sigma2,
+                               int32_t num_iterations, const icp_std_icp_io *io_dev, int32_t async);
+/* device time in milliseconds of the last run (CUDA events on the library stream) and the kernels + memsets it launched */
+int32_t icp_std_icp_last_run_stats(icp_std_icp h, double *device_ms, int64_t *launches);
+
 /* ---- (6) evaluators (api/sampling/evaluators/<Name>.scala, ProductEvaluators.scala) -------------- */
 #define ICP_EVAL_ACCEPT_ALL 0     /* AcceptAllEvaluator.scala:22-28 */
 #define ICP_EVAL_INDEPENDENT 1    /* IndependentPointDistanceEvaluator.scala:27-67, Gaussian(p0 = mean, p1 = sd) */
