@@ -149,6 +149,7 @@ _SIGS = {
     "icp_debug_time_closest_point": [_h, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, _dp],
     "icp_debug_l2_bandwidth": [_h, C.c_int64, _dp],
     "icp_debug_i8_gram": [_h, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, _dp],
+    "icp_debug_factor": [_h, C.c_int32, C.c_int32, _dp, _dp, _dp, _dp, C.c_double, C.c_int32, _dp, _dp, _dp, _ip],
 }
 EXPORTED_SYMBOLS = sorted(list(_SIGS) + ["icp_stage_name"])
 

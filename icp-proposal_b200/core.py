@@ -49,6 +49,20 @@ class Context:
         check(self.lib.icp_debug_l2_bandwidth(self.h, int(working_set_bytes), C.byref(out)), self.h)
         return out.value
 
+    def factor(self, M, b, theta_post=None, theta_other=None, step=1.0, ymean=False):
+        """Cholesky factorisation of C posterior matrices M (C x K x K) with right-hand sides b on the device path the
+        posterior pipeline takes at rank K (icp_debug_factor): L, the mean slot (mu, or y = L^-1 b when ymean), the
+        backward-form |L^T (w - mu)|^2 of theta_post -> theta_other (None without thetas) and the status words."""
+        M = f64(M); c, K = M.shape[0], M.shape[1]
+        b = f64(b).reshape(c, K)
+        L = np.zeros((c, K, K)); mean = np.empty((c, K)); st = np.empty(c, np.int32)
+        q = np.empty(c) if theta_post is not None else None
+        tp = None if q is None else f64(theta_post).reshape(c, K + THETA0)
+        to = None if q is None else f64(theta_other).reshape(c, K + THETA0)
+        check(self.lib.icp_debug_factor(self.h, c, K, dptr(M), dptr(b), None if tp is None else dptr(tp), None if to is None else dptr(to),
+                                        float(step), int(bool(ymean)), dptr(L), dptr(mean), None if q is None else dptr(q), iptr(st)), self.h)
+        return L, mean, q, st
+
     def philox(self, seed, chain, step, block):
         out = (C.c_uint32 * 4)()
         check(self.lib.icp_debug_philox(self.h, seed, chain, step, block, out), self.h)

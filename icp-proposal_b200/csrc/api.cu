@@ -763,7 +763,7 @@ void nearest_model_vertex(icp_model m, int C, const double *d_X, int64_t nq, con
 
 void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, double *d_L,
                         double *d_mu, const int *d_out_slot, cudaStream_t s, const SharedCp *shared, double *d_W,
-                        const QuadArgs *qa) {
+                        const QuadArgs *qa, bool ymean) {
     if (C <= 0) return;
     icp_model m = p->model;
     icp_target t = p->target;
@@ -845,15 +845,15 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
     }
     if (want_i8 && !grouped &&
         launch_rank_update_i8(md, C, od, gfp, I8Model{m->Qhat.p, m->col_norm.p, p->Qsub.p}, sc, w.Mp.p, w.b.p, m->ctx->sm_count, s)) {
-        launch_cholesky_packed(C, Kp, w.Mp.p, w.b.p, w.want_M ? w.M.p : nullptr, d_L, d_mu, d_out_slot, w.status.p, qa, s);
+        launch_cholesky_packed(C, Kp, w.Mp.p, w.b.p, w.want_M ? w.M.p : nullptr, d_L, d_mu, d_out_slot, w.status.p, qa, ymean, s);
         quad_done = qa != nullptr;
     } else
     if (!launch_posterior_fused(md, C, od, gfp, w.want_M ? w.M.p : nullptr, d_L, d_mu, d_out_slot, w.status.p, w.Mp.p, w.b.p, s, qa,
-                                &quad_done)) {
+                                &quad_done, ymean)) {
         launch_posterior_build(md, C, od, w.M.p, w.b.p, s, gfp);
-        launch_cholesky_solve(C, m->K, Kp, w.M.p, w.b.p, d_L, d_mu, d_out_slot, w.status.p, s, w.Mp.p, qa, &quad_done);
+        launch_cholesky_solve(C, m->K, Kp, w.M.p, w.b.p, d_L, d_mu, d_out_slot, w.status.p, s, w.Mp.p, qa, &quad_done, ymean);
     }
-    if (qa && !quad_done) launch_quad_form(C, Kp, d_L, d_mu, d_out_slot, *qa, s);
+    if (qa && !quad_done) launch_quad_form(C, Kp, d_L, d_mu, d_out_slot, *qa, ymean, s);
     if (d_W) launch_svd_factor(C, m->K, Kp, d_L, m->sqrt_var.p, d_out_slot, d_W, w.svd_scratch, s);
 }
 

@@ -81,7 +81,9 @@ struct StateDev {
     double *u_acc;                      // [C]
     long long *n_acc;                   // [C]
     int *step;                          // [1] device step counter
-    double *L, *mu;                     // [n_icp][2 C][Kp Kp], [n_icp][2 C][Kp]
+    // [n_icp][2 C][Kp Kp], [n_icp][2 C][Kp]: L and the whitened mean y = L^-1 b = L^T mu of each posterior (ICP_FACTOR_SVD
+    // components: mu itself, which their factor W needs)
+    double *L, *ymean;
     double *W;                          // [n_icp][2 C][Kp Kp] the reference's SVD factor (ICP_FACTOR_SVD components; else null)
     int *status;                        // [C] sticky per-chain status bits (kSt*)
     double *theta_best, *value_best;    // [C][L], [C]: BestSampleLogger - the state with the largest product value so far
@@ -195,9 +197,10 @@ __device__ __forceinline__ void stage_packed_L(const double *__restrict__ Lc, in
     }
 }
 
-// |L^T d|^2 with the packed lower triangle and d in shared memory: thread j owns column j (for a fixed row the threads read
-// consecutive words); result valid in every thread
-__device__ __forceinline__ double block_quad_packed(const double *sL, int Kp, const double *d_sm, double *red) {
+// |L^T d - y|^2 (y nullable: |L^T d|^2) with the packed lower triangle and d in shared memory: thread j owns column j (for a
+// fixed row the threads read consecutive words); result valid in every thread
+__device__ __forceinline__ double block_quad_packed(const double *sL, int Kp, const double *d_sm, double *red,
+                                                    const double *__restrict__ y) {
     double part = 0.0;
     for (int j = threadIdx.x; j < Kp; j += blockDim.x) {
         double v0 = 0.0, v1 = 0.0;
@@ -207,7 +210,7 @@ __device__ __forceinline__ double block_quad_packed(const double *sL, int Kp, co
             v1 = fma(sL[((i + 1) * (i + 2)) / 2 + j], d_sm[i + 1], v1);
         }
         if (i < Kp) v0 = fma(sL[(i * (i + 1)) / 2 + j], d_sm[i], v0);
-        const double v = v0 + v1;
+        const double v = y ? (v0 + v1) - y[j] : v0 + v1;
         part = fma(v, v, part);
     }
     return block_sum(part, red);
@@ -219,7 +222,8 @@ __device__ __forceinline__ double block_quad_packed(const double *sL, int Kp, co
 __global__ void __launch_bounds__(256) k_chain_propose(ChainParams P, ModelDev m, StateDev st, RngDev rng) {
     extern __shared__ double sm[];
     const int K = P.K, Kp = P.Kp, Lt = K + kTheta0, C = P.C;
-    // sz: z, then v = mu + W z | sw: W z | sdl: alpha' - alpha | sd: transition argument | sdg: diagonal of the staged factor |
+    // sz: z (+ y) | sw: v = L^-T (y + z) (SVD factor: mu + W z) | sdl: alpha' - alpha | sd: transition argument |
+    // sdg: diagonal of the staged factor |
     // part: 2 Kp partial sums of S v | red: block reduction | sL: packed lower triangle
     double *sz = sm, *sw = sm + Kp, *sdl = sm + 2 * Kp, *sd = sm + 3 * Kp, *sdg = sm + 4 * Kp, *part = sm + 5 * Kp, *red = sm + 7 * Kp,
            *sL = sm + 7 * Kp + 40;
@@ -265,11 +269,16 @@ __global__ void __launch_bounds__(256) k_chain_propose(ChainParams P, ModelDev m
     bool staged = false;   // sL holds the selected component's factor (diagonal inverted, true diagonal in sdg)
     if (cd.kind == ICP_PROP_ICP) {
         size_t pslot = (size_t)cd.icp_index * 2 * C + st.slot_cur[c];
-        const double *Lc = st.L + pslot * Kp * Kp, *muc = st.mu + pslot * Kp;
+        const double *Lc = st.L + pslot * Kp * Kp, *mean = st.ymean + pslot * Kp;
         if (cd.factor == ICP_FACTOR_SVD) {
-            // the reference's factor W = D^-1 Ubar diag(sqrt(lambda')) of the current state's posterior (svdfactor.cu)
+            // the reference's factor W = D^-1 Ubar diag(sqrt(lambda')) of the current state's posterior (svdfactor.cu); the
+            // mean slot of an SVD component holds mu: v = mu + W z
             block_matvec_rows(st.W + pslot * Kp * Kp, Kp, sz, sw);
+            __syncthreads();
+            for (int k = threadIdx.x; k < Kp; k += blockDim.x) sw[k] = mean[k] + sw[k];
         } else {
+            // v = mu + L^-T z = L^-T (y + z): one back substitution
+            for (int k = threadIdx.x; k < Kp; k += blockDim.x) sz[k] += mean[k];
             stage_packed_L(Lc, Kp, sL);
             __syncthreads();
             for (int i = threadIdx.x; i < Kp; i += blockDim.x) { double *d = sL + (i * (i + 1)) / 2 + i; sdg[i] = *d; *d = 1.0 / *d; }
@@ -278,15 +287,13 @@ __global__ void __launch_bounds__(256) k_chain_propose(ChainParams P, ModelDev m
             staged = true;
         }
         __syncthreads();
-        for (int k = threadIdx.x; k < Kp; k += blockDim.x) sz[k] = muc[k] + sw[k];
-        __syncthreads();
         // S v with S symmetric (read column-wise, coalesced); two halves of the k range per output
         for (int idx = threadIdx.x; idx < 2 * Kp; idx += blockDim.x) {
             int jj = idx % Kp, half = idx / Kp;
             int k0 = half * (Kp / 2), k1 = half ? Kp : Kp / 2;
             double acc = 0.0;
 #pragma unroll 8
-            for (int k = k0; k < k1; k++) acc = fma(__ldg(&m.S[(size_t)k * Kp + jj]), sz[k], acc);
+            for (int k = k0; k < k1; k++) acc = fma(__ldg(&m.S[(size_t)k * Kp + jj]), sw[k], acc);
             part[idx] = acc;
         }
         __syncthreads();
@@ -315,7 +322,8 @@ __global__ void __launch_bounds__(256) k_chain_propose(ChainParams P, ModelDev m
         }
     }
     __syncthreads();
-    // forward forms: d = (alpha + (alpha' - alpha) / step_i) - mu_cur,i   (NonRigidIcpProposal.scala:79, :82-83)
+    // forward forms |L_cur,i^T d|^2, d = (alpha + (alpha' - alpha) / step_i) - mu_cur,i   (NonRigidIcpProposal.scala:79, :82-83),
+    // formed as |L_cur,i^T s - y_cur,i|^2 with s = alpha + (alpha' - alpha) / step_i (SVD-factor components: d itself, from mu)
     // The selected component goes first when its factor is still staged: the other components stage theirs over it. (Taking
     // the components in index order formed the selected component's form from an overwritten factor whenever an ICP
     // component with a smaller index came before it - invisible next to a random-walk component, whose density dominates
@@ -332,11 +340,14 @@ __global__ void __launch_bounds__(256) k_chain_propose(ChainParams P, ModelDev m
         } else {
             stage_packed_L(st.L + pslot * Kp * Kp, Kp, sL);
         }
-        const double *mui = st.mu + pslot * Kp;
-        for (int k = threadIdx.x; k < Kp; k += blockDim.x)
-            sd[k] = k < K ? (th[kTheta0 + k] + (sdl[k] / ci.step)) - mui[k] : 0.0;
+        const double *mean = st.ymean + pslot * Kp;
+        const bool ym = ci.factor != ICP_FACTOR_SVD;
+        for (int k = threadIdx.x; k < Kp; k += blockDim.x) {
+            const double s = k < K ? th[kTheta0 + k] + (sdl[k] / ci.step) : 0.0;
+            sd[k] = ym ? s : k < K ? s - mean[k] : 0.0;
+        }
         __syncthreads();
-        const double qf = block_quad_packed(sL, Kp, sd, red);
+        const double qf = block_quad_packed(sL, Kp, sd, red, ym ? mean : nullptr);
         if (threadIdx.x == 0) st.qf[(size_t)ci.icp_index * C + c] = qf;
         __syncthreads();
     }
@@ -602,7 +613,7 @@ struct icp_chain_s {
     ChainParams P{};
     std::vector<icp_proposal> icp_props;
     // state
-    DevBuf<double> theta_cur, theta_prop, values_cur, values_prop, u_acc, L, mu, X, W, theta_best, value_best, qf, qb;
+    DevBuf<double> theta_cur, theta_prop, values_cur, values_prop, u_acc, L, ymean, X, W, theta_best, value_best, qf, qb;
     MetricsWork mwork;       // periodic RegistrationComparison of the best sample (icp_chain_io.metrics_interval)
     DevBuf<int> cur_sel, slot_cur, slot_prop, comp_sel, step, status;
     DevBuf<int> lane_ok, lane_status, step_end;   // rejection look-ahead (k_la_resolve)
@@ -810,10 +821,11 @@ void enqueue_state_eval(RunCtx &r, const double *d_theta, double *d_values, cons
         if (ch->cp_shared[i] || !fork || n_side >= icp_ctx_s::kAux) continue;
         cudaStream_t ss = ctx->aux[n_side];
         ICP_CUDA(cudaStreamWaitEvent(ss, ctx->ev_fork, 0));
-        double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *mub = r.st.mu + (size_t)i * 2 * C * Kp;
+        double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *yb = r.st.ymean + (size_t)i * 2 * C * Kp;
         double *Wb = ch->icp_props[i]->prm.factor == ICP_FACTOR_SVD ? r.st.W + (size_t)i * 2 * C * Kp * Kp : nullptr;
         QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
-        posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, mub, d_slots, ss, nullptr, Wb, proposal ? &qa : nullptr);
+        posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, yb, d_slots, ss, nullptr, Wb, proposal ? &qa : nullptr,
+                           Wb == nullptr);
         ICP_CUDA(cudaEventRecord(ctx->ev_join[n_side], ss));
         ch->on_side[i] = 1;
         n_side++;
@@ -821,12 +833,12 @@ void enqueue_state_eval(RunCtx &r, const double *d_theta, double *d_values, cons
     evaluator_pipeline(ch->evaluator, ch->ework, Cn, d_theta, ch->X.p, d_values, ch->estatus.p, r.s);
     for (int i = 0; i < ch->P.n_icp; i++) {
         if (ch->on_side[i]) { ch->on_side[i] = 0; continue; }
-        double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *mub = r.st.mu + (size_t)i * 2 * C * Kp;
+        double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *yb = r.st.ymean + (size_t)i * 2 * C * Kp;
         SharedCp sh{ch->ework.cp_m2t.p, ch->evaluator->n_ids, ch->cp_map[i].p};
         double *Wb = ch->icp_props[i]->prm.factor == ICP_FACTOR_SVD ? r.st.W + (size_t)i * 2 * C * Kp * Kp : nullptr;
         QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
-        posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, mub, d_slots, r.s, ch->cp_shared[i] ? &sh : nullptr, Wb,
-                           proposal ? &qa : nullptr);
+        posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, yb, d_slots, r.s, ch->cp_shared[i] ? &sh : nullptr, Wb,
+                           proposal ? &qa : nullptr, Wb == nullptr);
     }
     for (int k = 0; k < n_side; k++) ICP_CUDA(cudaStreamWaitEvent(r.s, ctx->ev_join[k], 0));   // join
 }
@@ -922,14 +934,14 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
     ch->qf.ensure((size_t)std::max(n_icp, 1) * C); ch->qb.ensure((size_t)std::max(n_icp, 1) * C);
     ICP_REQUIRE(io->metrics_interval >= 0, "metrics_interval must be >= 0");
     ICP_REQUIRE(io->metrics_interval == 0 || io->log_metrics != nullptr, "metrics_interval > 0 needs log_metrics");
-    ch->L.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp * Kp); ch->mu.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp);
+    ch->L.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp * Kp); ch->ymean.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp);
     ch->X.ensure((size_t)C * m->N * 3);
 
     RunCtx r;
     r.ch = ch; r.C = C; r.Cn = C; r.s = s; r.W = W; r.Cr = Cr; r.Wa = W;
     r.st = StateDev{ch->theta_cur.p, ch->theta_prop.p, ch->values_cur.p, ch->values_prop.p, ch->cur_sel.p,
                     ch->slot_cur.p, ch->slot_prop.p, ch->comp_sel.p, ch->u_acc.p, ch->n_acc.p, ch->step.p, ch->L.p,
-                    ch->mu.p, ch->any_svd ? ch->W.p : nullptr, ch->status.p, ch->theta_best.p, ch->value_best.p,
+                    ch->ymean.p, ch->any_svd ? ch->W.p : nullptr, ch->status.p, ch->theta_best.p, ch->value_best.p,
                     ch->qf.p, ch->qb.p, ch->lane_ok.p, ch->lane_status.p, ch->step_end.p};
     if (!resume) { ch->stats_on = ch->stats_req_on; ch->stats_run = ch->stats_req; }
     r.st.sx = StatsDev{};

@@ -287,9 +287,12 @@ struct QuadArgs {
 };
 // qa (nullable): also the quadratic form above; *quad_done tells whether the launched path formed it (the caller runs
 // launch_quad_form otherwise)
+// ymean (every factorisation entry below): d_mu receives y = L^-1 b instead of mu = L^-T y, and the quadratic form is
+// |L^T w - y|^2 with w = theta_post + (theta_other - theta_post) / step - the chain runner's mean slot (it needs neither mu
+// nor the back substitution that forms it)
 bool launch_posterior_fused(const ModelDev &m, int C, const ObsDev &o, const GramFast *gf, double *d_M_or_null, double *d_L,
                             double *d_mu, const int *d_out_slot, int *d_status, double *d_Mp, double *d_b, cudaStream_t s,
-                            const QuadArgs *qa = nullptr, bool *quad_done = nullptr);
+                            const QuadArgs *qa = nullptr, bool *quad_done = nullptr, bool ymean = false);
 // rank update on the INT8 tensor cores (tc_i8.cu): block-packed M and b like the DMMA rank update.
 // I8Model: the basis with every column divided by its bound (max over the vertices of |Q_v[:, j]|) and the bounds;
 // I8Scale: frame multiplier that brings the whitened rows into |x| <= 2^30 and the factors that undo it.
@@ -302,15 +305,16 @@ void launch_unit_basis(int rows, int Kp, const double *d_Q, const double *d_coln
 void launch_pack_obs_rows(int n, int Kp, const int *d_ids, const double *d_Qhat, double *d_Qsub /* [n][3 Kp + 2] */, cudaStream_t s);
 // k_cholesky_packed on a block-packed M (the second half of launch_posterior_fused's default path)
 void launch_cholesky_packed(int C, int Kp, const double *d_Mp, const double *d_b, double *d_M_or_null, double *d_L, double *d_mu,
-                            const int *d_out_slot, int *d_status, const QuadArgs *qa, cudaStream_t s);
-// the same quadratic form from L / mu in global memory (paths whose factorisation kernel does not form it)
-void launch_quad_form(int C, int Kp, const double *d_L, const double *d_mu, const int *d_slot, const QuadArgs &qa, cudaStream_t s);
+                            const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s);
+// the same quadratic form from L / mu (ymean: y) in global memory (paths whose factorisation kernel does not form it)
+void launch_quad_form(int C, int Kp, const double *d_L, const double *d_mu, const int *d_slot, const QuadArgs &qa, bool ymean,
+                      cudaStream_t s);
 // in: M (C x Kp x Kp), b (C x Kp). out: L (lower Cholesky factor, C x Kp x Kp), mu = M^-1 b, status (0 ok)
 // out_slot (nullable): chain c writes L / mu at index out_slot[c] instead of c
 // d_Mp: scratch for the block-packed lower triangle (C x NB (NB + 1) / 2 x 64 doubles), needed when Kp > 160
 void launch_cholesky_solve(int C, int K, int Kp, const double *d_M, const double *d_b, double *d_L, double *d_mu,
                            const int *d_out_slot, int *d_status, cudaStream_t s, double *d_Mp = nullptr,
-                           const QuadArgs *qa = nullptr, bool *quad_done = nullptr);
+                           const QuadArgs *qa = nullptr, bool *quad_done = nullptr, bool ymean = false);
 // alpha' = alpha + step (S (mu + L^-T z) - alpha); L/mu addressed through per-chain slot indices
 // d_W (nullable): explicit factor [slot][Kp][Kp] (ICP_FACTOR_SVD); alpha' then uses W z instead of L^-T z
 void launch_propose(const ModelDev &m, int C, double step, const double *d_theta, const double *d_z,
@@ -618,9 +622,10 @@ struct SharedCp {
     const int *map;     // [n_ids] index into the shared list
 };
 // d_W (nullable, [slot][Kp][Kp]): also the reference's SVD-based covariance factor (ICP_FACTOR_SVD)
+// ymean: d_mu receives y = L^-1 b instead of mu (see launch_posterior_fused); only the chain runner asks for it
 void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, double *d_L,
                         double *d_mu, const int *d_out_slot, cudaStream_t s, const SharedCp *shared = nullptr,
-                        double *d_W = nullptr, const QuadArgs *qa = nullptr);
+                        double *d_W = nullptr, const QuadArgs *qa = nullptr, bool ymean = false);
 // distance evaluator pipeline: values [C][3] = {product, prior, distance}
 void evaluator_pipeline(icp_evaluator e, EvalWork &w, int C, const double *d_theta, const double *d_X, double *d_values,
                         int *d_status, cudaStream_t s);

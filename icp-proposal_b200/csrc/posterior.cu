@@ -743,9 +743,10 @@ __device__ long long g_ft[kFtStride * 8192];
 // Factorises the matrix staged in shared memory (A: [Kp + 8][Kp + 4], lower triangle of M in rows 0..Kp-1, b in row Kp,
 // rows Kp+1..Kp+7 zero), solves M mu = b and stores L (lower triangle only) and mu. Every one of the NT threads of the CTA
 // must call it (it synchronises the CTA); *bad (shared) must have been cleared before the preceding barrier.
+// ymean: store y = L^-1 b (the chain runner's mean slot) instead of mu, and skip the back substitution.
 template <int NT>
 __device__ void chol_factor_solve_store(double *A, int Kp, int *bad, double *__restrict__ Lc, double *__restrict__ muc,
-                                        int *__restrict__ status) {
+                                        int *__restrict__ status, bool ymean) {
     const int ld = Kp + 4, NB = Kp >> 3, R = Kp + 8;
     double *dinv = A + (size_t)R * ld;      // [Kp] reciprocals of the diagonal of L
     double *xs = dinv + Kp;                 // [Kp] running right-hand side of the back substitution
@@ -831,7 +832,7 @@ __device__ void chol_factor_solve_store(double *A, int Kp, int *bad, double *__r
     ICP_FT(const long long ftc1 = clock64();)
     for (int k = tid; k < Kp; k += NT) xs[k] = A[Kp * ld + k];
     __syncthreads();
-    for (int bj = NB - 1; bj >= 0; bj--) {
+    for (int bj = ymean ? -1 : NB - 1; bj >= 0; bj--) {   // ymean: xs already holds what is stored, no step runs
         const double *D = A + (8 * bj) * ld + 8 * bj;
         double x[8];
 #pragma unroll
@@ -862,7 +863,7 @@ __device__ void chol_factor_solve_store(double *A, int Kp, int *bad, double *__r
         int i = e / Kp, j = e - i * Kp;
         if (j <= i) __stcs(Lc + e, isbad ? NAN : A[i * ld + j]);   // only the lower triangle is ever read; streaming stores
     }
-    for (int j = tid; j < Kp; j += NT) __stcs(muc + j, isbad ? NAN : xo[j]);
+    for (int j = tid; j < Kp; j += NT) __stcs(muc + j, isbad ? NAN : ymean ? xs[j] : xo[j]);
     if (tid == 0 && status) *status = isbad ? 1 : 0;
 }
 
@@ -870,7 +871,7 @@ __global__ void __launch_bounds__(kCh2Threads) k_cholesky_solve_mma(int K, int K
                                                                      const double *__restrict__ bvec,
                                                                      double *__restrict__ L, double *__restrict__ mu,
                                                                      const int *__restrict__ out_slot,
-                                                                     int *__restrict__ status) {
+                                                                     int *__restrict__ status, bool ymean) {
     extern __shared__ double sm[];
     const int ld = Kp + 4, NB = Kp >> 3, R = Kp + 8;
     double *A = sm;                         // [R][ld]
@@ -913,7 +914,7 @@ __global__ void __launch_bounds__(kCh2Threads) k_cholesky_solve_mma(int K, int K
     }
     __syncthreads();
     int oc = out_slot ? out_slot[c] : c;
-    chol_factor_solve_store<kCh2Threads>(A, Kp, &bad, L + (size_t)oc * Kp * Kp, mu + (size_t)oc * Kp, status ? status + c : nullptr);
+    chol_factor_solve_store<kCh2Threads>(A, Kp, &bad, L + (size_t)oc * Kp * Kp, mu + (size_t)oc * Kp, status ? status + c : nullptr, ymean);
     (void)K;
 }
 
@@ -971,7 +972,9 @@ constexpr int kCh3Threads = 128;
 // NT threads per matrix: 128 (four matrices per SM) for full batches; 256 when every matrix of the launch is resident anyway
 // (a few chains are latency-bound: the load, store and column-update phases get twice the threads; the arithmetic of every
 // element - and for Kp <= 128 the association of the final quadratic form - does not depend on NT)
-template <int NT>
+// YMEAN (the chain runner's form): the mean slot receives y = L^-1 b instead of mu = L^-T y, and the backward form is
+// |L^T w - y|^2 (= |L^T (w - mu)|^2). The back substitution and its scratch drop out; L and y are the same arithmetic.
+template <int NT, bool YMEAN>
 __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int Kp, const double *__restrict__ Mp,
                                                                     const double *__restrict__ bvec, double *__restrict__ M_out,
                                                                     double *__restrict__ L, double *__restrict__ mu,
@@ -982,8 +985,8 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
     double *A = sp;                  // [ntri][64]
     double *yv = A + ntri * 64;      // [Kp] b, then y = L^-1 b
     double *dinv = yv + Kp;          // [Kp] reciprocals of the diagonal of L
-    double *xs = dinv + Kp;          // [Kp] running right-hand side of the back substitution
-    double *xo = xs + Kp;            // [Kp] solution
+    double *xs = dinv + Kp;          // [Kp] running right-hand side of the back substitution (YMEAN: w of the backward form)
+    double *xo = xs + Kp;            // [Kp] solution (mu form only)
     __shared__ int bad;
     const int c = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int fr = lane >> 2, fc = lane & 3, sw = pk_swz(fr);
@@ -1144,31 +1147,33 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
     ICP_FT(if (tid == 0 && c < 8192) for (int k_ = 0; k_ < 5; k_++) g_ft[kFtStride * c + 1 + k_] = fph[k_];)
     // back substitution L^T x = y
     ICP_FT(const long long ftb = clock64(); if (tid == 0 && c < 8192) g_ft[kFtStride * c + 9] = ftb - ftf;)
-    for (int k = tid; k < Kp; k += NT) xs[k] = yv[k];
-    __syncthreads();
-    for (int bj = NB - 1; bj >= 0; bj--) {
-        const double *D = A + pk_blk(bj, bj);
-        double x[8];
-#pragma unroll
-        for (int i = 7; i >= 0; i--) {
-            double t = xs[8 * bj + i];
-#pragma unroll
-            for (int k = i + 1; k < 8; k++) t = fma(-D[k * 8 + (i ^ pk_swz(k))], x[k], t);
-            x[i] = t * dinv[8 * bj + i];
-        }
-        if (tid < 8) {
-#pragma unroll
-            for (int i = 0; i < 8; i++)
-                if (i == tid) xo[8 * bj + i] = x[i];
-        }
-        for (int k = tid; k < 8 * bj; k += NT) {
-            const double *blk = A + pk_blk(bj, k >> 3);   // elements (8 bj + p, k), p = 0..7
-            double t = xs[k];
-#pragma unroll
-            for (int p = 0; p < 8; p++) t = fma(-blk[p * 8 + ((k & 7) ^ pk_swz(p))], x[p], t);
-            xs[k] = t;
-        }
+    if (!YMEAN) {
+        for (int k = tid; k < Kp; k += NT) xs[k] = yv[k];
         __syncthreads();
+        for (int bj = NB - 1; bj >= 0; bj--) {
+            const double *D = A + pk_blk(bj, bj);
+            double x[8];
+#pragma unroll
+            for (int i = 7; i >= 0; i--) {
+                double t = xs[8 * bj + i];
+#pragma unroll
+                for (int k = i + 1; k < 8; k++) t = fma(-D[k * 8 + (i ^ pk_swz(k))], x[k], t);
+                x[i] = t * dinv[8 * bj + i];
+            }
+            if (tid < 8) {
+#pragma unroll
+                for (int i = 0; i < 8; i++)
+                    if (i == tid) xo[8 * bj + i] = x[i];
+            }
+            for (int k = tid; k < 8 * bj; k += NT) {
+                const double *blk = A + pk_blk(bj, k >> 3);   // elements (8 bj + p, k), p = 0..7
+                double t = xs[k];
+#pragma unroll
+                for (int p = 0; p < 8; p++) t = fma(-blk[p * 8 + ((k & 7) ^ pk_swz(p))], x[p], t);
+                xs[k] = t;
+            }
+            __syncthreads();
+        }
     }
     ICP_FT(const long long fts = clock64(); if (tid == 0 && c < 8192) g_ft[kFtStride * c + 10] = fts - ftb;)
     const bool isbad = bad != 0;
@@ -1187,14 +1192,18 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
             __stcs(reinterpret_cast<double2 *>(Lc + (size_t)i * Kp + j), v);
         }
     }
-    for (int j = tid; j < Kp; j += NT) __stcs(mu + (size_t)oc * Kp + j, isbad ? NAN : xo[j]);
+    for (int j = tid; j < Kp; j += NT) __stcs(mu + (size_t)oc * Kp + j, isbad ? NAN : YMEAN ? yv[j] : xo[j]);
     if (tid == 0 && status) status[c] = isbad ? 1 : 0;
     if (qa.out) {
         // chain runner: |L^T d|^2 of the transition theta_post -> theta_other while L is still here (k_chain_accept would
-        // otherwise read it back from HBM). d overwrites the right-hand side scratch.
+        // otherwise read it back from HBM). d = w - mu (YMEAN: w, and y is subtracted after the product) overwrites the
+        // right-hand side scratch.
         const int Lt = qa.K + kTheta0;
         const double *tp = qa.theta_post + (size_t)c * Lt + kTheta0, *to = qa.theta_other + (size_t)c * Lt + kTheta0;
-        for (int k = tid; k < Kp; k += NT) xs[k] = k < qa.K ? (tp[k] + ((to[k] - tp[k]) / qa.step)) - xo[k] : 0.0;
+        for (int k = tid; k < Kp; k += NT) {
+            const double w = k < qa.K ? tp[k] + ((to[k] - tp[k]) / qa.step) : 0.0;
+            xs[k] = YMEAN ? w : k < qa.K ? w - xo[k] : 0.0;
+        }
         __syncthreads();
         double part = 0.0;
         for (int j = tid; j < Kp; j += NT) {
@@ -1202,7 +1211,7 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
             int i = j;
             for (; i + 1 < Kp; i += 2) { v0 = fma(A[pk_at(i, j)], xs[i], v0); v1 = fma(A[pk_at(i + 1, j)], xs[i + 1], v1); }
             if (i < Kp) v0 = fma(A[pk_at(i, j)], xs[i], v0);
-            const double v = v0 + v1;
+            const double v = YMEAN ? (v0 + v1) - yv[j] : v0 + v1;
             part = fma(v, v, part);
         }
         // block sum through the (now free) dinv scratch
@@ -1219,17 +1228,24 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
     ICP_FT(if (tid == 0 && c < 8192) g_ft[kFtStride * c + 11] = clock64() - fts;)
 }
 
+template <int NT, bool YMEAN>
+static void launch_cholesky_packed_nt(int C, int Kp, size_t smem_c, const double *d_Mp, const double *d_b, double *d_M, double *d_L,
+                                      double *d_mu, const int *d_out_slot, int *d_status, const QuadArgs &q, cudaStream_t s) {
+    ICP_CUDA(cudaFuncSetAttribute(k_cholesky_packed<NT, YMEAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
+    k_cholesky_packed<NT, YMEAN><<<C, NT, smem_c, s>>>(Kp, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q);
+}
+
 static void run_cholesky_packed(int C, int Kp, size_t smem_c, const double *d_Mp, const double *d_b, double *d_M, double *d_L, double *d_mu,
-                                const int *d_out_slot, int *d_status, const QuadArgs *qa, cudaStream_t s) {
+                                const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s) {
     const QuadArgs q = qa ? *qa : QuadArgs{};
     // the two ICP posteriors of a step factorise concurrently: up to 148 chains all their matrices are resident at two per SM
     // (measured: 148 chains 605 k -> 646 k samples/s, one chain's round 0.179 -> 0.175 ms; at 296 chains 128 threads win)
     if (C <= 148 && Kp <= 128) {
-        ICP_CUDA(cudaFuncSetAttribute(k_cholesky_packed<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
-        k_cholesky_packed<256><<<C, 256, smem_c, s>>>(Kp, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q);
+        if (ymean) launch_cholesky_packed_nt<256, true>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
+        else launch_cholesky_packed_nt<256, false>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
     } else {
-        ICP_CUDA(cudaFuncSetAttribute(k_cholesky_packed<kCh3Threads>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
-        k_cholesky_packed<kCh3Threads><<<C, kCh3Threads, smem_c, s>>>(Kp, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q);
+        if (ymean) launch_cholesky_packed_nt<kCh3Threads, true>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
+        else launch_cholesky_packed_nt<kCh3Threads, false>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
     }
 }
 
@@ -1267,7 +1283,7 @@ __global__ void __launch_bounds__((NWC + kProdWarps) * 32, 2) k_posterior_fused(
                                                                              double gs_scale, double row_scale,
                                                                              double *__restrict__ L, double *__restrict__ mu,
                                                                              const int *__restrict__ out_slot,
-                                                                             int *__restrict__ status) {
+                                                                             int *__restrict__ status, bool ymean) {
     extern __shared__ __align__(16) double sm[];
     const int Kp = m.Kp, ld = Kp + 4, NB = Kp >> 3;
     const int bufsz = kMmaRows * ld;
@@ -1638,7 +1654,7 @@ __global__ void __launch_bounds__((NWC + kProdWarps) * 32, 2) k_posterior_fused(
     }
     const int oc = out_slot ? out_slot[c] : c;
     ICP_FT(long long ftc = clock64();)
-    chol_factor_solve_store<nthreads>(sA, Kp, &bad, L + (size_t)oc * Kp * Kp, mu + (size_t)oc * Kp, status ? status + c : nullptr);
+    chol_factor_solve_store<nthreads>(sA, Kp, &bad, L + (size_t)oc * Kp * Kp, mu + (size_t)oc * Kp, status ? status + c : nullptr, ymean);
     ICP_FT(if (tid == 0 && c < 8192) {
         unsigned smid;
         asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
@@ -1655,7 +1671,7 @@ extern "C" int icp_debug_fused_timing(long long *out, int n) {
 template <int NBLK, int NBMAX, int NWC>
 static void launch_fused(const ModelDev &m, int C, const ObsDev &o, double *d_M, int total, const GramFast *gf, double *d_L,
                          double *d_mu, const int *d_out_slot, int *d_status, double *d_Mp, double *d_b, cudaStream_t s,
-                         const QuadArgs *qa, bool *quad_done) {
+                         const QuadArgs *qa, bool *quad_done, bool ymean) {
     const int Kp = m.Kp, ld = Kp + 4;
     size_t stage = (size_t)2 * kMmaRows * ld + 8 * Kp + (std::min(o.n, kMaxStagedIds) + 3) / 4 * 2 + (size_t)kRawStages * kProdWarps * 32 * 3 * ((NBMAX + 1) / 2) * 2;
     size_t fact = (size_t)(Kp + 8) * ld + 3 * Kp;
@@ -1667,16 +1683,16 @@ static void launch_fused(const ModelDev &m, int C, const ObsDev &o, double *d_M,
             ProfScope _ps(ST_POSTERIOR_BUILD, s);
             if (gf) {
                 ICP_CUDA(cudaFuncSetAttribute(k_posterior_fused<NBLK, NBMAX, NWC, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                k_posterior_fused<NBLK, NBMAX, NWC, 1, false><<<C, nthr, smem, s>>>(m, o, d_Mp, total, gf->Gs, gf->gs_scale, gf->row_scale, nullptr, d_b, nullptr, nullptr);
+                k_posterior_fused<NBLK, NBMAX, NWC, 1, false><<<C, nthr, smem, s>>>(m, o, d_Mp, total, gf->Gs, gf->gs_scale, gf->row_scale, nullptr, d_b, nullptr, nullptr, false);
             } else {
                 ICP_CUDA(cudaFuncSetAttribute(k_posterior_fused<NBLK, NBMAX, NWC, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                k_posterior_fused<NBLK, NBMAX, NWC, 3, false><<<C, nthr, smem, s>>>(m, o, d_Mp, total, nullptr, 0.0, 1.0, nullptr, d_b, nullptr, nullptr);
+                k_posterior_fused<NBLK, NBMAX, NWC, 3, false><<<C, nthr, smem, s>>>(m, o, d_Mp, total, nullptr, 0.0, 1.0, nullptr, d_b, nullptr, nullptr, false);
             }
             ICP_CUDA(cudaGetLastError());
         }
         ProfScope _ps(ST_CHOLESKY, s);
         size_t smem_c = sizeof(double) * ((size_t)total * 64 + 4 * Kp);
-        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, qa, s);
+        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, qa, ymean, s);
         if (quad_done) *quad_done = qa != nullptr;
         return;
     }
@@ -1684,19 +1700,19 @@ static void launch_fused(const ModelDev &m, int C, const ObsDev &o, double *d_M,
     size_t smem = sizeof(double) * std::max(stage, fact);
     if (gf) {
         ICP_CUDA(cudaFuncSetAttribute(k_posterior_fused<NBLK, NBMAX, NWC, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_posterior_fused<NBLK, NBMAX, NWC, 1, true><<<C, nthr, smem, s>>>(m, o, d_M, total, gf->Gs, gf->gs_scale, gf->row_scale, d_L, d_mu, d_out_slot, d_status);
+        k_posterior_fused<NBLK, NBMAX, NWC, 1, true><<<C, nthr, smem, s>>>(m, o, d_M, total, gf->Gs, gf->gs_scale, gf->row_scale, d_L, d_mu, d_out_slot, d_status, ymean);
     } else {
         ICP_CUDA(cudaFuncSetAttribute(k_posterior_fused<NBLK, NBMAX, NWC, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_posterior_fused<NBLK, NBMAX, NWC, 3, true><<<C, nthr, smem, s>>>(m, o, d_M, total, nullptr, 0.0, 1.0, d_L, d_mu, d_out_slot, d_status);
+        k_posterior_fused<NBLK, NBMAX, NWC, 3, true><<<C, nthr, smem, s>>>(m, o, d_M, total, nullptr, 0.0, 1.0, d_L, d_mu, d_out_slot, d_status, ymean);
     }
 }
 
 void launch_cholesky_packed(int C, int Kp, const double *d_Mp, const double *d_b, double *d_M_or_null, double *d_L, double *d_mu,
-                            const int *d_out_slot, int *d_status, const QuadArgs *qa, cudaStream_t s) {
+                            const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s) {
     ProfScope _ps(ST_CHOLESKY, s);
     const int NB = Kp / 8, total = NB * (NB + 1) / 2;
     size_t smem_c = sizeof(double) * ((size_t)total * 64 + 4 * Kp);
-    run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M_or_null, d_L, d_mu, d_out_slot, d_status, qa, s);
+    run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M_or_null, d_L, d_mu, d_out_slot, d_status, qa, ymean, s);
     ICP_CUDA(cudaGetLastError());
 }
 
@@ -1706,7 +1722,7 @@ void launch_cholesky_packed(int C, int Kp, const double *d_Mp, const double *d_b
 // ICPCUDA_FUSE=1 (or d_Mp == nullptr): the single-launch variant, whose factorisation runs at two chains per SM.
 bool launch_posterior_fused(const ModelDev &m, int C, const ObsDev &o, const GramFast *gf, double *d_M_or_null, double *d_L,
                             double *d_mu, const int *d_out_slot, int *d_status, double *d_Mp, double *d_b, cudaStream_t s,
-                            const QuadArgs *qa, bool *quad_done) {
+                            const QuadArgs *qa, bool *quad_done, bool ymean) {
     if (quad_done) *quad_done = false;
     static const bool off = (getenv("ICPCUDA_NO_DMMA") && getenv("ICPCUDA_NO_DMMA")[0] == '1') ||
                             (getenv("ICPCUDA_NO_FUSE") && getenv("ICPCUDA_NO_FUSE")[0] == '1');
@@ -1714,9 +1730,9 @@ bool launch_posterior_fused(const ModelDev &m, int C, const ObsDev &o, const Gra
     const int NB = m.Kp / 8, total = NB * (NB + 1) / 2;
     if (off || NB > 13 || C <= 0) return false;   // NB <= 13: the 192-thread variants; the fused matrix must fit 2 CTAs / SM
     if (one_launch) d_Mp = nullptr;
-    if (NB <= 4) launch_fused<4, 4, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done);
-    else if (NB <= 7) launch_fused<8, 7, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done);
-    else launch_fused<24, 13, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done);
+    if (NB <= 4) launch_fused<4, 4, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done, ymean);
+    else if (NB <= 7) launch_fused<8, 7, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done, ymean);
+    else launch_fused<24, 13, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done, ymean);
     ICP_CUDA(cudaGetLastError());
     return true;
 }
@@ -1733,8 +1749,25 @@ __global__ void __launch_bounds__(128) k_pack_lower(int Kp, const double *__rest
     }
 }
 
+// mu -> y = L^T mu in place, for the factorisation path that solves for mu only (k_cholesky_solve)
+__global__ void __launch_bounds__(128) k_mean_to_ymean(int Kp, const double *__restrict__ L, double *__restrict__ mu,
+                                                       const int *__restrict__ slot) {
+    extern __shared__ double smu[];
+    const int sl = slot ? slot[blockIdx.x] : blockIdx.x;
+    const double *Lc = L + (size_t)sl * Kp * Kp;
+    double *m = mu + (size_t)sl * Kp;
+    for (int k = threadIdx.x; k < Kp; k += blockDim.x) smu[k] = m[k];
+    __syncthreads();
+    for (int j = threadIdx.x; j < Kp; j += blockDim.x) {
+        double v = 0.0;
+        for (int i = j; i < Kp; i++) v = fma(Lc[(size_t)i * Kp + j], smu[i], v);
+        m[j] = v;
+    }
+}
+
 void launch_cholesky_solve(int C, int K, int Kp, const double *d_M, const double *d_b, double *d_L, double *d_mu,
-                           const int *d_out_slot, int *d_status, cudaStream_t s, double *d_Mp, const QuadArgs *qa, bool *quad_done) {
+                           const int *d_out_slot, int *d_status, cudaStream_t s, double *d_Mp, const QuadArgs *qa, bool *quad_done,
+                           bool ymean) {
     ProfScope _ps(ST_CHOLESKY, s);
     if (quad_done) *quad_done = false;
     if (C <= 0) return;
@@ -1746,7 +1779,7 @@ void launch_cholesky_solve(int C, int K, int Kp, const double *d_M, const double
         ICP_REQUIRE(d_Mp != nullptr && smem_c <= 227 * 1024 - 64, "rank too large for the shared-memory Cholesky (K <= 224)");
         k_pack_lower<<<C, 128, 0, s>>>(Kp, d_M, d_Mp);
         ICP_CUDA(cudaGetLastError());
-        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, nullptr, d_L, d_mu, d_out_slot, d_status, qa, s);
+        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, nullptr, d_L, d_mu, d_out_slot, d_status, qa, ymean, s);
         ICP_CUDA(cudaGetLastError());
         if (quad_done) *quad_done = qa != nullptr;
         return;
@@ -1755,7 +1788,7 @@ void launch_cholesky_solve(int C, int K, int Kp, const double *d_M, const double
         size_t smem2 = sizeof(double) * ((size_t)(Kp + 8) * (Kp + 4) + 3 * Kp);
         ICP_REQUIRE(smem2 <= 227 * 1024, "rank too large for the shared-memory Cholesky (K <= 160)");
         ICP_CUDA(cudaFuncSetAttribute(k_cholesky_solve_mma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-        k_cholesky_solve_mma<<<C, kCh2Threads, smem2, s>>>(K, Kp, d_M, d_b, d_L, d_mu, d_out_slot, d_status);
+        k_cholesky_solve_mma<<<C, kCh2Threads, smem2, s>>>(K, Kp, d_M, d_b, d_L, d_mu, d_out_slot, d_status, ymean);
         ICP_CUDA(cudaGetLastError());
         return;
     }
@@ -1764,6 +1797,10 @@ void launch_cholesky_solve(int C, int K, int Kp, const double *d_M, const double
     ICP_CUDA(cudaFuncSetAttribute(k_cholesky_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_cholesky_solve<<<C, kChThreads, smem, s>>>(K, Kp, d_M, d_b, d_L, d_mu, d_out_slot, d_status);
     ICP_CUDA(cudaGetLastError());
+    if (ymean) {   // this path forms mu only: y = L^T mu
+        k_mean_to_ymean<<<C, 128, sizeof(double) * Kp, s>>>(Kp, d_L, d_mu, d_out_slot);
+        ICP_CUDA(cudaGetLastError());
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1829,12 +1866,14 @@ void launch_propose(const ModelDev &m, int C, double step, const double *d_theta
     ICP_CUDA(cudaGetLastError());
 }
 
-// |L^T d|^2 with d in shared memory; all threads of the block participate; red: >= 33 doubles
-__device__ double block_quad_LT(const double *__restrict__ Lc, int Kp, const double *d_sm, double *red) {
+// |L^T d - y|^2 with d in shared memory (y nullable: |L^T d|^2); all threads of the block participate; red: >= 33 doubles
+__device__ double block_quad_LT(const double *__restrict__ Lc, int Kp, const double *d_sm, double *red,
+                                const double *__restrict__ y = nullptr) {
     double part = 0.0;
     for (int j = threadIdx.x; j < Kp; j += blockDim.x) {
         double v = 0.0;
         for (int i = j; i < Kp; i++) v = fma(__ldg(&Lc[(size_t)i * Kp + j]), d_sm[i], v);
+        if (y) v -= y[j];
         part = fma(v, v, part);
     }
     return block_sum(part, red);
@@ -1861,23 +1900,28 @@ __global__ void __launch_bounds__(128) k_log_transition(int K, int Kp, double st
 }
 
 // |L^T d|^2 with L / mu read back from global memory: the factorisation paths that do not form it in their epilogue
+// ymean: the mean slot holds y = L^T mu, and the form is |L^T w - y|^2
 __global__ void __launch_bounds__(128) k_quad_form(int Kp, const double *__restrict__ L, const double *__restrict__ mu,
-                                                   const int *__restrict__ slot, QuadArgs qa) {
+                                                   const int *__restrict__ slot, QuadArgs qa, bool ymean) {
     extern __shared__ double sm[];
     double *sd = sm, *red = sm + Kp;
     const int c = blockIdx.x, Lt = qa.K + kTheta0;
     const int sl = slot ? slot[c] : c;
     const double *tp = qa.theta_post + (size_t)c * Lt + kTheta0, *to = qa.theta_other + (size_t)c * Lt + kTheta0;
-    for (int k = threadIdx.x; k < Kp; k += blockDim.x)
-        sd[k] = k < qa.K ? (tp[k] + ((to[k] - tp[k]) / qa.step)) - mu[(size_t)sl * Kp + k] : 0.0;
+    const double *mc = mu + (size_t)sl * Kp;
+    for (int k = threadIdx.x; k < Kp; k += blockDim.x) {
+        const double w = k < qa.K ? tp[k] + ((to[k] - tp[k]) / qa.step) : 0.0;
+        sd[k] = ymean ? w : k < qa.K ? w - mc[k] : 0.0;
+    }
     __syncthreads();
-    const double q = block_quad_LT(L + (size_t)sl * Kp * Kp, Kp, sd, red);
+    const double q = block_quad_LT(L + (size_t)sl * Kp * Kp, Kp, sd, red, ymean ? mc : nullptr);
     if (threadIdx.x == 0) qa.out[c] = q;
 }
 
-void launch_quad_form(int C, int Kp, const double *d_L, const double *d_mu, const int *d_slot, const QuadArgs &qa, cudaStream_t s) {
+void launch_quad_form(int C, int Kp, const double *d_L, const double *d_mu, const int *d_slot, const QuadArgs &qa, bool ymean,
+                      cudaStream_t s) {
     if (C <= 0) return;
-    k_quad_form<<<C, 128, sizeof(double) * (Kp + 40), s>>>(Kp, d_L, d_mu, d_slot, qa);
+    k_quad_form<<<C, 128, sizeof(double) * (Kp + 40), s>>>(Kp, d_L, d_mu, d_slot, qa, ymean);
     ICP_CUDA(cudaGetLastError());
 }
 
@@ -1889,3 +1933,69 @@ void launch_log_transition(int C, int K, int Kp, double step, const double *d_fr
 }
 
 }  // namespace icp
+
+// Factorises C symmetric matrices M (host, C x K x K) with right-hand sides b (C x K) on the device path the posterior
+// pipeline takes at this rank (Kp <= 104: k_cholesky_packed; above: launch_cholesky_solve), in the mu form (ymean = 0) or the
+// chain runner's form (ymean = 1). Out: L (C x K x K, lower triangle; the upper triangle is left as passed in), mean (mu or
+// y = L^-1 b), q (|L^T d|^2 of the transition theta_post -> theta_other, C x (K + 10) each; NULL: not formed), status.
+extern "C" int32_t icp_debug_factor(icp_ctx ctx, int32_t C, int32_t K, const double *M, const double *b, const double *theta_post,
+                                    const double *theta_other, double step, int32_t ymean, double *L, double *mean, double *q,
+                                    int32_t *status) {
+    using namespace icp;
+    icp_ctx _ctx = ctx;
+    try {
+        ICP_REQUIRE(ctx && C > 0 && K > 0 && M && b && L && mean && status, "null or empty argument");
+        ICP_REQUIRE(!q || (theta_post && theta_other), "q needs theta_post and theta_other");
+        CtxLock lock(ctx);
+        cudaStream_t s = ctx->stream;
+        const int Kp = (K + 7) / 8 * 8, NB = Kp / 8, Lt = K + kTheta0;
+        // padded exactly as the rank update pads: identity on the padded diagonal, zero right-hand side
+        std::vector<double> hM((size_t)C * Kp * Kp, 0.0), hb((size_t)C * Kp, 0.0);
+        for (int c = 0; c < C; c++) {
+            for (int i = 0; i < Kp; i++)
+                for (int j = 0; j < Kp; j++)
+                    hM[((size_t)c * Kp + i) * Kp + j] = i < K && j < K ? M[((size_t)c * K + i) * K + j] : i == j ? 1.0 : 0.0;
+            for (int i = 0; i < K; i++) hb[(size_t)c * Kp + i] = b[(size_t)c * K + i];
+        }
+        DevBuf<double> dM, db, dMp, dL, dmean, dtp, dto, dq;
+        DevBuf<int> dst;
+        dM.upload(hM.data(), hM.size(), s);
+        db.upload(hb.data(), hb.size(), s);
+        dMp.alloc((size_t)C * NB * (NB + 1) / 2 * 64);
+        dL.alloc((size_t)C * Kp * Kp);
+        ICP_CUDA(cudaMemsetAsync(dL.p, 0, sizeof(double) * dL.n, s));
+        dmean.alloc((size_t)C * Kp);
+        dst.alloc(C);
+        QuadArgs qa{};
+        if (q) {
+            dtp.upload(theta_post, (size_t)C * Lt, s);
+            dto.upload(theta_other, (size_t)C * Lt, s);
+            dq.alloc(C);
+            qa = QuadArgs{dtp.p, dto.p, step, K, dq.p};
+        }
+        bool quad_done = false;
+        if (NB <= 13) {
+            k_pack_lower<<<C, 128, 0, s>>>(Kp, dM.p, dMp.p);
+            ICP_CUDA(cudaGetLastError());
+            launch_cholesky_packed(C, Kp, dMp.p, db.p, nullptr, dL.p, dmean.p, nullptr, dst.p, q ? &qa : nullptr, ymean != 0, s);
+            quad_done = q != nullptr;
+        } else {
+            launch_cholesky_solve(C, K, Kp, dM.p, db.p, dL.p, dmean.p, nullptr, dst.p, s, dMp.p, q ? &qa : nullptr, &quad_done, ymean != 0);
+        }
+        if (q && !quad_done) launch_quad_form(C, Kp, dL.p, dmean.p, nullptr, qa, ymean != 0, s);
+        std::vector<double> hL((size_t)C * Kp * Kp), hm((size_t)C * Kp);
+        ICP_CUDA(cudaMemcpyAsync(hL.data(), dL.p, sizeof(double) * hL.size(), cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaMemcpyAsync(hm.data(), dmean.p, sizeof(double) * hm.size(), cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaMemcpyAsync(status, dst.p, sizeof(int) * C, cudaMemcpyDeviceToHost, s));
+        if (q) ICP_CUDA(cudaMemcpyAsync(q, dq.p, sizeof(double) * C, cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaStreamSynchronize(s));
+        for (int c = 0; c < C; c++)
+            for (int i = 0; i < K; i++) {
+                for (int j = 0; j <= i; j++) L[((size_t)c * K + i) * K + j] = hL[((size_t)c * Kp + i) * Kp + j];
+                mean[(size_t)c * K + i] = hm[(size_t)c * Kp + i];
+            }
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
+    }
+}

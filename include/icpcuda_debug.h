@@ -40,6 +40,14 @@ int32_t icp_debug_l2_bandwidth(icp_ctx ctx, int64_t working_set_bytes, double *g
  * tile shape M = 128, N = 112, K = 32). */
 int32_t icp_debug_i8_gram(icp_ctx ctx, int32_t rows, const int8_t *A, int32_t *D, int32_t iters, int32_t ctas, double *ms);
 
+/* Posterior factorisation of C host matrices M (C x K x K, symmetric) and right-hand sides b (C x K) on the device path the
+ * posterior pipeline takes at rank K. ymean = 0: mean = mu = M^-1 b (icp_posterior's form); ymean = 1: mean = y = L^-1 b, the
+ * chain runner's form, which skips the back substitution. L: lower triangle of the Cholesky factor (C x K x K). q (nullable):
+ * |L^T (w - mu)|^2 per matrix, w = theta_post + (theta_other - theta_post) / step over the coefficients (theta_* C x (K + 10)),
+ * formed as the chain runner forms its backward transition form. status[c] != 0: M_c was not positive definite. */
+int32_t icp_debug_factor(icp_ctx ctx, int32_t C, int32_t K, const double *M, const double *b, const double *theta_post,
+                         const double *theta_other, double step, int32_t ymean, double *L, double *mean, double *q, int32_t *status);
+
 #ifdef __cplusplus
 }
 #endif
