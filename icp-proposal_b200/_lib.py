@@ -50,6 +50,10 @@ class Component(C.Structure):
     _fields_ = [("kind", C.c_int32), ("axis", C.c_int32), ("weight", C.c_double), ("sd", C.c_double), ("proposal", _h)]
 
 
+class ChainTarget(C.Structure):
+    _fields_ = [("target", _h), ("components", C.POINTER(Component)), ("evaluator", _h)]
+
+
 class KernelTerm(C.Structure):
     _fields_ = [("scale", C.c_double), ("sigma", C.c_double), ("A", C.c_double * 9)]
 
@@ -133,6 +137,8 @@ _SIGS = {
     "icp_chainlog_gather": [_h, C.c_int32, C.c_int32, C.c_int32, C.POINTER(ChainIO), C.POINTER(ChainIO), _dp, _lp],
     "icp_variability_allreduce": [_h, _h, C.c_int32, _dp, C.c_int32, _dp, _dp, _dp, _dp, _dp, _lp],
     "icp_chain_create": [_h, _h, C.POINTER(Component), C.c_int32, _h, C.c_int32, C.POINTER(_h)],
+    "icp_chain_create_targets": [_h, C.c_int32, C.POINTER(ChainTarget), C.c_int32, C.c_int32, C.POINTER(_h)],
+    "icp_chain_set_target_index": [_h, C.c_int32, _ip],
     "icp_chain_destroy": [_h],
     "icp_chain_run": [_h, C.c_int32, C.c_int32, _dp, C.POINTER(ChainIO)],
     "icp_chain_run_device": [_h, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(ChainIO), C.c_int32],

@@ -565,25 +565,52 @@ class Comm:
 class Chain:
     """Fused Metropolis-Hastings runner (Scalismo MetropolisHastings + MixtureProposal on the device)."""
 
-    def __init__(self, model: Model, target: Target, components, evaluator: Evaluator, max_chains):
-        """components: list of dict(kind, weight, proposal=IcpProposal|None, sd=0, axis=0, name=...)."""
-        self.model, self.target, self.evaluator, self.lib, self.ctx = model, target, evaluator, model.lib, model.ctx
-        self.components = list(components)
-        arr = (_lib.Component * len(components))()
-        for i, c in enumerate(components):
-            arr[i].kind = int(c["kind"]); arr[i].axis = int(c.get("axis", 0)); arr[i].weight = float(c["weight"])
-            arr[i].sd = float(c.get("sd", 0.0))
-            arr[i].proposal = c["proposal"].h if c.get("proposal") is not None else None
-        self._arr = arr
+    def __init__(self, model: Model, target: Target = None, components=None, evaluator: Evaluator = None, max_chains=1,
+                 targets=None):
+        """components: list of dict(kind, weight, proposal=IcpProposal|None, sd=0, axis=0, name=...).
+        targets: instead of (target, components, evaluator), a list of such triples, one per target of the handle
+        (icp_chain_create_targets); run() then needs target_index."""
+        self.lib, self.ctx, self.model = model.lib, model.ctx, model
+        if targets is None:
+            targets = [(target, components, evaluator)]
+        elif target is not None or components is not None or evaluator is not None:
+            raise ValueError("pass either target, components and evaluator or targets")
+        self.targets = [(t, list(cs), e) for t, cs, e in targets]
+        self.target, self.components, self.evaluator = self.targets[0]
+        self.n_targets = len(self.targets)
+        self._arrs = []
+        for _, cs, _ in self.targets:
+            arr = (_lib.Component * len(cs))()
+            for i, c in enumerate(cs):
+                arr[i].kind = int(c["kind"]); arr[i].axis = int(c.get("axis", 0)); arr[i].weight = float(c["weight"])
+                arr[i].sd = float(c.get("sd", 0.0))
+                arr[i].proposal = c["proposal"].h if c.get("proposal") is not None else None
+            self._arrs.append(arr)
+        self._arr = self._arrs[0]
         self.max_chains = int(max_chains)
         self.h = C.c_void_p()
-        check(self.lib.icp_chain_create(model.h, target.h, arr, len(components), evaluator.h, self.max_chains,
-                                        C.byref(self.h)), self.ctx.h)
+        if len(self.targets) == 1:
+            check(self.lib.icp_chain_create(model.h, self.target.h, self._arr, len(self.components), self.evaluator.h,
+                                            self.max_chains, C.byref(self.h)), self.ctx.h)
+        else:
+            ents = (_lib.ChainTarget * len(self.targets))()
+            for g, (t, cs, e) in enumerate(self.targets):
+                ents[g].target, ents[g].components, ents[g].evaluator = t.h, self._arrs[g], e.h
+            check(self.lib.icp_chain_create_targets(model.h, len(self.targets), ents, len(self.components), self.max_chains,
+                                                    C.byref(self.h)), self.ctx.h)
+
+    def set_target_index(self, target_index):
+        """icp_chain_set_target_index: chain c of the next run from theta0 runs on targets[target_index[c]]."""
+        ti = np.ascontiguousarray(target_index, dtype=np.int32).reshape(-1)
+        check(self.lib.icp_chain_set_target_index(self.h, len(ti), ti.ctypes.data_as(_lib._ip)), self.ctx.h)
 
     def run(self, theta0, n_steps, seed=1024, chain_id_offset=0, u_comp=None, z=None, u_acc=None, log_theta=True,
-            raise_on_status=True, metrics_interval=0):
+            raise_on_status=True, metrics_interval=0, target_index=None):
         """raise_on_status=False: a per-chain status failure (empty set / not positive definite / NaN, the cases in which the
-        reference throws) does not raise; the result carries `status` (per-chain words) and `status_code` (the return code)."""
+        reference throws) does not raise; the result carries `status` (per-chain words) and `status_code` (the return code).
+        target_index: [C] target of every chain (set_target_index before the run)."""
+        if target_index is not None:
+            self.set_target_index(target_index)
         th, c = self.model._theta(theta0)
         K, L = self.model.K, self.model.K + THETA0
         io = _lib.ChainIO()
@@ -616,8 +643,10 @@ class Chain:
                     status=status, status_code=rc, theta_best=best, value_best=vbest, metrics=metrics)
 
     def run_device(self, C_, n_steps, theta0_ptr, seed=1024, chain_id_offset=0, log_component=0, log_accepted=0,
-                   log_values=0, log_theta=0, theta_final=0, n_accepted=0, async_=False):
-        """All pointers are raw device addresses (e.g. torch.Tensor.data_ptr())."""
+                   log_values=0, log_theta=0, theta_final=0, n_accepted=0, async_=False, target_index=None):
+        """All pointers are raw device addresses (e.g. torch.Tensor.data_ptr()); target_index is a host array as for run()."""
+        if target_index is not None:
+            self.set_target_index(target_index)
         io = _lib.ChainIO()
         io.seed, io.chain_id_offset = int(seed), int(chain_id_offset)
         io.log_component, io.log_accepted, io.log_values = log_component or None, log_accepted or None, log_values or None

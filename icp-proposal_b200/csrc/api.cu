@@ -763,10 +763,11 @@ void nearest_model_vertex(icp_model m, int C, const double *d_X, int64_t nq, con
 
 void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, double *d_L,
                         double *d_mu, const int *d_out_slot, cudaStream_t s, const SharedCp *shared, double *d_W,
-                        const QuadArgs *qa, bool ymean) {
+                        const QuadArgs *qa, bool ymean, const TargetSet *ts) {
     if (C <= 0) return;
     icp_model m = p->model;
     icp_target t = p->target;
+    const bool has_boundary = ts ? ts->has_boundary : t->has_boundary;
     const int Kp = m->Kp;
     ModelDev md = m->dev();
     if (!d_X) {
@@ -785,11 +786,12 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
         // :118 currentMesh.pointSet.findClosestPoint(targetPoint): vertex BVH refit to the current meshes
         w.prim.ensure(tot);
         if (w.seed.n < tot) { w.seed.ensure(tot); ICP_CUDA(cudaMemsetAsync(w.seed.p, 0xFF, sizeof(int) * tot, s)); }
-        nearest_model_vertex(m, C, d_X, n, p->tp.p, 0, w.seed.p, w.prim.p, s);
-        oa.tp = p->tp.p; oa.near_vid = w.prim.p;
+        const double *tp = ts ? ts->tp : p->tp.p;
+        nearest_model_vertex(m, C, d_X, n, tp, ts ? 1 : 0, w.seed.p, w.prim.p, s);
+        oa.tp = tp; oa.tp_per_chain = ts ? 1 : 0; oa.near_vid = w.prim.p;
     } else {
         // :97 target.operations.closestPointOnSurface(currentMeshPoint)
-        const bool need_flags = p->prm.boundary_aware && t->has_boundary;
+        const bool need_flags = p->prm.boundary_aware && has_boundary;
         if (shared && !need_flags) {
             oa.cp = shared->cp; oa.cp_stride = shared->stride; oa.cp_map = shared->map;
         } else {
@@ -797,6 +799,7 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
             NearestArgs a;
             a.bvh = &t->tri_bvh; a.prim_data = t->tri_data.p; a.wide = t->wide(); a.sm_count = t->ctx->sm_count; a.C = C; a.nq = n;
             a.Xq = d_X; a.q_ids = p->ids.p; a.Nq = m->N; a.out_cp = w.cp.p; a.perm = p->qperm.p;
+            if (ts) { a.mt_rec = ts->rec; a.mt_idx = ts->tidx; }
             if (w.seed.n < tot) { w.seed.ensure(tot); ICP_CUDA(cudaMemsetAsync(w.seed.p, 0xFF, sizeof(int) * tot, s)); }
             a.seed_slot = w.seed.p;
             launch_nearest(a, s);
@@ -809,8 +812,10 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
             NearestArgs v;
             v.bvh = &t->vert_bvh; v.prim_data = t->vert_data.p; v.C = C; v.nq = n; v.q = w.cp.p; v.q_per_chain = 1;
             v.out_prim = w.prim.p;
+            if (ts) { v.mt_rec = ts->rec; v.mt_idx = ts->tidx; }
             launch_nearest(v, s);
-            launch_lookup_flags((int64_t)C * n, w.prim.p, t->boundary.p, t->Nt, w.flags.p, s);
+            launch_lookup_flags((int64_t)C * n, w.prim.p, t->boundary.p, t->Nt, w.flags.p, s, ts ? ts->rec : nullptr,
+                                ts ? ts->tidx : nullptr, n);
             oa.cp_on_boundary = w.flags.p;
         }
     }
@@ -818,7 +823,7 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
     od.nrows = w.nobs.p + C;
     launch_observations(oa, od, s);
     // every observation is kept (no boundary filtering possible) -> the Gram part of M is the proposal's constant
-    const bool all_kept = !tsamp && !(p->prm.boundary_aware && t->has_boundary);
+    const bool all_kept = !tsamp && !(p->prm.boundary_aware && has_boundary);
     GramFast gf{p->Gs.p, 1.0 / (p->prm.tangential_noise * p->prm.tangential_noise),
                 std::sqrt(std::max(0.0, 1.0 - (p->prm.noise_along_normal * p->prm.noise_along_normal) /
                                                   (p->prm.tangential_noise * p->prm.tangential_noise)))};
@@ -1455,10 +1460,15 @@ extern "C" int32_t icp_evaluator_destroy(icp_evaluator e) {
 namespace icp {
 
 void evaluator_pipeline(icp_evaluator e, EvalWork &w, int C, const double *d_theta, const double *d_X, double *d_values,
-                        int *d_status, cudaStream_t s) {
+                        int *d_status, cudaStream_t s, const TargetSet *ts) {
     if (C <= 0) return;
     icp_model m = e->model;
     icp_target t = e->target;
+    const bool has_boundary = ts ? ts->has_boundary : t->has_boundary;
+    const TargetRec *mt_rec = ts ? ts->rec : nullptr;
+    const int *mt_idx = ts ? ts->tidx : nullptr;
+    // the target -> model lists: the evaluator's own, or every entry's copy of its target's list
+    const int n_tp = ts ? ts->n_tp : e->n_tp;
     ModelDev md = m->dev();
     const int kind = e->prm.kind, mode = e->prm.mode;
     EvalReduceArgs ra{};
@@ -1488,45 +1498,48 @@ void evaluator_pipeline(icp_evaluator e, EvalWork &w, int C, const double *d_the
             NearestArgs a;
             a.bvh = &t->tri_bvh; a.prim_data = t->tri_data.p; a.wide = t->wide(); a.sm_count = t->ctx->sm_count; a.C = C; a.nq = e->n_ids;
             a.Xq = d_X; a.q_ids = e->ids.p; a.Nq = m->N; a.out_d2 = w.d2_m2t.p; a.perm = e->qperm.p;
+            a.mt_rec = mt_rec; a.mt_idx = mt_idx;
             if (w.seed_m2t.n < tot) { w.seed_m2t.ensure(tot); ICP_CUDA(cudaMemsetAsync(w.seed_m2t.p, 0xFF, sizeof(int) * tot, s)); }
             a.seed_slot = w.seed_m2t.p;
             if (collective || w.force_cp_m2t) { w.cp_m2t.ensure(3 * tot); a.out_cp = w.cp_m2t.p; }
             a.chain_max = hd_max;
             launch_nearest(a, s);
-            if (collective && t->has_boundary) {
+            if (collective && has_boundary) {
                 // CollectiveAverage...:46-47: nearest target vertex of the closest point, dropped when on the boundary
                 w.prim.ensure(tot); w.skip_m2t.ensure(tot);
                 NearestArgs v;
                 v.bvh = &t->vert_bvh; v.prim_data = t->vert_data.p; v.C = C; v.nq = e->n_ids; v.q = w.cp_m2t.p;
                 v.q_per_chain = 1; v.out_prim = w.prim.p;
+                v.mt_rec = mt_rec; v.mt_idx = mt_idx;
                 launch_nearest(v, s);
-                launch_lookup_flags((int64_t)tot, w.prim.p, t->boundary.p, t->Nt, w.skip_m2t.p, s);
+                launch_lookup_flags((int64_t)tot, w.prim.p, t->boundary.p, t->Nt, w.skip_m2t.p, s, mt_rec, mt_idx, e->n_ids);
                 ra.skip_m2t = w.skip_m2t.p;
             }
         }
-        if (use_t && e->n_tp > 0) {
-            size_t tot = (size_t)C * e->n_tp;
+        if (use_t && n_tp > 0) {
+            size_t tot = (size_t)C * n_tp;
             w.d2_t2m.ensure(tot);
             bvh_refit(m->tri_bvh, C, d_X, m->N, m->tris.p, s);
             NearestArgs a;
-            a.bvh = &m->tri_bvh; a.X = d_X; a.tris = m->tris.p; a.N = m->N; a.C = C; a.nq = e->n_tp; a.q = e->tp.p;
+            a.bvh = &m->tri_bvh; a.X = d_X; a.tris = m->tris.p; a.N = m->N; a.C = C; a.nq = n_tp;
+            a.q = ts ? ts->tp : e->tp.p; a.q_per_chain = ts ? 1 : 0;
             a.out_d2 = w.d2_t2m.p;
             if (w.seed_t2m.n < tot) { w.seed_t2m.ensure(tot); ICP_CUDA(cudaMemsetAsync(w.seed_t2m.p, 0xFF, sizeof(int) * tot, s)); }
             a.seed_slot = w.seed_t2m.p;
             if (collective) { w.cp_t2m.ensure(3 * tot); a.out_cp = w.cp_t2m.p; }
             a.chain_max = hd_max;
             launch_nearest(a, s);
-            if (collective && t->has_boundary) {
+            if (collective && has_boundary) {
                 // CollectiveAverage...:58-59: id of the nearest vertex of the MODEL sample, looked up in the
                 // TARGET's boundary table (SURVEY Appendix B3)
                 w.prim.ensure(tot); w.skip_t2m.ensure(tot);
-                nearest_model_vertex(m, C, d_X, e->n_tp, w.cp_t2m.p, 1, nullptr, w.prim.p, s);
-                launch_lookup_flags((int64_t)tot, w.prim.p, t->boundary.p, t->Nt, w.skip_t2m.p, s);
+                nearest_model_vertex(m, C, d_X, n_tp, w.cp_t2m.p, 1, nullptr, w.prim.p, s);
+                launch_lookup_flags((int64_t)tot, w.prim.p, t->boundary.p, t->Nt, w.skip_t2m.p, s, mt_rec, mt_idx, n_tp);
                 ra.skip_t2m = w.skip_t2m.p;
             }
         }
         ra.n_m2t = use_m ? e->n_ids : 0; ra.d2_m2t = w.d2_m2t.p;
-        ra.n_t2m = use_t ? e->n_tp : 0; ra.d2_t2m = w.d2_t2m.p;
+        ra.n_t2m = use_t ? n_tp : 0; ra.d2_t2m = w.d2_t2m.p;
     }
     launch_eval_reduce(ra, s);
 }

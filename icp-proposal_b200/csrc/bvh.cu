@@ -326,7 +326,11 @@ constexpr int kDone = 0x7ffffffe;
 // upper bound <= the chain's maximum, so the maximum over the outputs stays the exact Hausdorff distance. The warps of a
 // launch rotate over the chains (warp w -> chain w % C, 32-query block (w / C) * blk_stride % n_blk of that chain), so the
 // first wave finishes a few blocks of EVERY chain and the following waves prune against those maxima.
-template <int PRIM, bool DYNAMIC, bool HDMAX>
+//
+// MT (several static targets, TargetRec): query row c first reads the leaf count, packed nodes, primitive ids and leaf data
+// of its own target, record mt_rec[mt_idx[c]]; the walk is the single-target one. The MT = false instantiations never read
+// the two trailing arguments.
+template <int PRIM, bool DYNAMIC, bool HDMAX, bool MT>
 __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int2 *__restrict__ children,
                                                  const float4 *__restrict__ nodes, const int *__restrict__ prim,
                                                  const double *__restrict__ prim_data, const double *__restrict__ X,
@@ -336,7 +340,8 @@ __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int
                                                  const int *__restrict__ perm, int *__restrict__ seed_slot,
                                                  int *__restrict__ out_prim, int *__restrict__ out_feat,
                                                  double *__restrict__ out_cp, double *__restrict__ out_d2,
-                                                 unsigned long long *__restrict__ chain_max, int n_blk, int blk_stride, int lpw) {
+                                                 unsigned long long *__restrict__ chain_max, int n_blk, int blk_stride, int lpw,
+                                                 const TargetRec *__restrict__ mt_rec, const int *__restrict__ mt_idx) {
     __shared__ int s_stack_n[kStackShared][kNearestThreads];
     __shared__ float s_stack_d[kStackShared][kNearestThreads];
     long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -361,6 +366,10 @@ __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int
         i = g % nq;
     }
     if (perm) { i = perm[i]; g = (long long)c * nq + i; }  // spatially sorted processing order, results in caller order
+    if (MT) {
+        const TargetRec &r = mt_rec[__ldg(mt_idx + c)];
+        n = r.n[PRIM]; nodes = r.nodes[PRIM]; prim = r.prim[PRIM]; prim_data = r.data[PRIM];
+    }
     double qx, qy, qz;
     if (q_ids) {
         const double *src = Xq + ((size_t)c * Nq + q_ids[i]) * 3;
@@ -452,7 +461,8 @@ __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int
 }
 
 void launch_nearest(const NearestArgs &a, cudaStream_t s) {
-    if (a.wide && launch_nearest_wide(a, a.sm_count, s)) return;
+    const bool mt = a.mt_rec != nullptr;
+    if (!mt && a.wide && launch_nearest_wide(a, a.sm_count, s)) return;
     ProfScope _ps(a.prim_data ? ST_NEAREST_STATIC : ST_NEAREST_DYNAMIC, s);
     long long total = a.nq * a.C;
     if (total <= 0) return;
@@ -474,12 +484,20 @@ void launch_nearest(const NearestArgs &a, cudaStream_t s) {
     static const int lpw_small = getenv("ICPCUDA_LPW") ? atoi(getenv("ICPCUDA_LPW")) : 8;   // (experiments: 4 / 8 / 16)
     const int lpw = (!a.chain_max && total <= 16384 && lpw_small >= 1 && lpw_small < 32) ? lpw_small : 32;
     if (lpw < 32) blocks = (unsigned)((((total + lpw - 1) / lpw) * 32 + threads - 1) / threads);
-#define ICP_LAUNCH_NEAREST(P, D, H)                                                                                  \
-    k_nearest<P, D, H><<<blocks, threads, 0, s>>>(b.n, b.children.p, (D) ? b.nodes.p : b.packed.p, b.prim.p, a.prim_data, a.X, a.tris, \
+#define ICP_LAUNCH_NEAREST_MT(P, D, H, M)                                                                            \
+    k_nearest<P, D, H, M><<<blocks, threads, 0, s>>>(b.n, b.children.p, (D) ? b.nodes.p : b.packed.p, b.prim.p, a.prim_data, a.X, a.tris, \
                                                a.N, a.C, (long long)a.nq, a.q, a.q_per_chain, a.Xq, a.q_ids,     \
                                                a.Nq, a.perm, a.seed_slot, a.out_prim, a.out_feat, a.out_cp, a.out_d2, \
-                                               a.chain_max, n_blk, blk_stride, lpw)
-    if (a.chain_max) {
+                                               a.chain_max, n_blk, blk_stride, lpw, a.mt_rec, a.mt_idx)
+#define ICP_LAUNCH_NEAREST(P, D, H) ICP_LAUNCH_NEAREST_MT(P, D, H, false)
+    if (mt) {
+        ICP_REQUIRE(!dynamic && a.mt_idx, "launch_nearest: several targets need static structures and a target index");
+        if (a.chain_max) {
+            ICP_REQUIRE(b.prim_kind == 0 && !a.out_cp && !a.out_prim && !a.out_feat, "launch_nearest: chain_max is for distance-only triangle queries");
+            ICP_LAUNCH_NEAREST_MT(0, false, true, true);
+        } else if (b.prim_kind == 0) ICP_LAUNCH_NEAREST_MT(0, false, false, true);
+        else ICP_LAUNCH_NEAREST_MT(1, false, false, true);
+    } else if (a.chain_max) {
         ICP_REQUIRE(b.prim_kind == 0 && !a.out_cp && !a.out_prim && !a.out_feat, "launch_nearest: chain_max is for distance-only triangle queries");
         if (dynamic) ICP_LAUNCH_NEAREST(0, true, true); else ICP_LAUNCH_NEAREST(0, false, true);
     } else if (b.prim_kind == 0) {
@@ -488,6 +506,7 @@ void launch_nearest(const NearestArgs &a, cudaStream_t s) {
         if (dynamic) ICP_LAUNCH_NEAREST(1, true, false); else ICP_LAUNCH_NEAREST(1, false, false);
     }
 #undef ICP_LAUNCH_NEAREST
+#undef ICP_LAUNCH_NEAREST_MT
     ICP_CUDA(cudaGetLastError());
 }
 
@@ -779,19 +798,24 @@ void launch_nearest_sorted(NearestArgs a, QuerySort &qs, const double lo[3], con
     launch_nearest(a, s);
 }
 
-// flags[i] = table[prim[i]] (0 when prim < 0)
+// flags[i] = table[prim[i]] (0 when prim < 0); with rec, row i / per reads the table of its own target
 __global__ void k_lookup_flags(long long n, const int *__restrict__ prim, const uint8_t *__restrict__ table, int table_n,
-                               uint8_t *__restrict__ flags) {
+                               uint8_t *__restrict__ flags, const TargetRec *__restrict__ rec, const int *__restrict__ tidx,
+                               long long per) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    if (rec) {
+        const TargetRec &r = rec[tidx[i / per]];
+        table = r.boundary; table_n = r.Nt;
+    }
     int p = prim[i];
     flags[i] = (p >= 0 && p < table_n) ? table[p] : 0;
 }
 
 void launch_lookup_flags(int64_t n, const int *d_prim, const uint8_t *d_table, int table_n, uint8_t *d_flags,
-                         cudaStream_t s) {
+                         cudaStream_t s, const TargetRec *rec, const int *tidx, int64_t per) {
     if (n <= 0) return;
-    k_lookup_flags<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(n, d_prim, d_table, table_n, d_flags);
+    k_lookup_flags<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(n, d_prim, d_table, table_n, d_flags, rec, tidx, per);
     ICP_CUDA(cudaGetLastError());
 }
 

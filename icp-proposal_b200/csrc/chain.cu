@@ -660,21 +660,115 @@ struct icp_chain_s {
     DevBuf<long long> sx_pending, sx_count, sx_flush_w, sx_flush_n;   // StatsDev
     DevBuf<double> sx_flush_theta, sx_mean, sx_m2, sx_nsum;          // StatsDev.flush_theta, StatsAcc
     DevBuf<int> sx_idx, sx_nlist;                                    // launch_stats_flush's list of flushed chains
+    // target set (icp_chain_create_targets). model / target / evaluator / icp_props above are those of entry 0, which every
+    // entry shares except for its target; with one target nothing below is used and the runner is the single-target one.
+    int n_targets = 1;
+    std::vector<icp_target> all_targets;       // [G] (references held)
+    std::vector<icp_evaluator> all_evals;      // [G]
+    std::vector<icp_proposal> all_props;       // every entry's ICP proposals
+    bool set_boundary = false;                 // OR of the targets' has_boundary
+    DevBuf<TargetRec> trec;                    // [G]
+    std::vector<DevBuf<double>> tp_all;        // per ICP component: [G][n_tp][3] the entries' target points (target sampling)
+    DevBuf<double> etp_all;                    // [G][etp_n][3] the evaluators' target -> model lists, padded to the longest
+    int etp_n = 0;
+    std::vector<int> tidx_req;                 // icp_chain_set_target_index: the target of every chain of the next run from theta0
+    DevBuf<int> tidx;                          // [C] target of every batch entry (look-ahead: lane v takes chain v % Cr's)
+    std::vector<DevBuf<double>> tp_lane;       // per ICP component: [C][n_tp][3]
+    DevBuf<double> etp_lane;                   // [C][etp_n][3]
 };
 
-extern "C" int32_t icp_chain_create(icp_model m, icp_target t, const icp_component *components, int32_t n_components,
-                                    icp_evaluator evaluator, int32_t max_chains, icp_chain *out) {
+namespace {
+
+// first difference between two entries of a target set that may only differ in their target ("" when none)
+std::string entry_difference(const icp_chain_target &a, const icp_chain_target &b, int n_components) {
+    auto ids_of = [](const DevBuf<int> &d, int n) {
+        std::vector<int> h(n);
+        if (n) ICP_CUDA(cudaMemcpy(h.data(), d.p, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost));
+        return h;
+    };
+    for (int i = 0; i < n_components; i++) {
+        const icp_component &x = a.components[i], &y = b.components[i];
+        const std::string c = "component " + std::to_string(i) + " ";
+        if (x.kind != y.kind) return c + "kind";
+        if (x.weight != y.weight) return c + "weight";
+        if (x.sd != y.sd) return c + "sd";
+        if (x.axis != y.axis) return c + "axis";
+        if (x.kind != ICP_PROP_ICP) continue;
+        if (!y.proposal) return c + "proposal (null)";
+        const icp_proposal_s &p = *x.proposal, &q = *y.proposal;
+        if (p.model != q.model) return c + "proposal model";
+        if (p.prm.step_length != q.prm.step_length) return c + "proposal step_length";
+        if (p.prm.tangential_noise != q.prm.tangential_noise) return c + "proposal tangential_noise";
+        if (p.prm.noise_along_normal != q.prm.noise_along_normal) return c + "proposal noise_along_normal";
+        if (p.prm.direction != q.prm.direction) return c + "proposal direction";
+        if (p.prm.boundary_aware != q.prm.boundary_aware) return c + "proposal boundary_aware";
+        if (p.prm.factor != q.prm.factor) return c + "proposal factor";
+        if (p.prm.rank_update != q.prm.rank_update) return c + "proposal rank_update";
+        if (p.n_ids != q.n_ids || ids_of(p.ids, p.n_ids) != ids_of(q.ids, q.n_ids)) return c + "proposal model point ids";
+        if (p.n_tp != q.n_tp) return c + "proposal n_tp";
+    }
+    const icp_evaluator_s &e = *a.evaluator, &f = *b.evaluator;
+    if (e.model != f.model) return "evaluator model";
+    if (e.prm.kind != f.prm.kind) return "evaluator kind";
+    if (e.prm.mode != f.prm.mode) return "evaluator mode";
+    if (e.prm.use_prior != f.prm.use_prior) return "evaluator use_prior";
+    if (e.prm.p0 != f.prm.p0) return "evaluator p0";
+    if (e.prm.p1 != f.prm.p1) return "evaluator p1";
+    if (e.prm.p2 != f.prm.p2) return "evaluator p2";
+    if (e.n_ids != f.n_ids || ids_of(e.ids, e.n_ids) != ids_of(f.ids, f.n_ids)) return "evaluator model point ids";
+    if (e.prm.kind != ICP_EVAL_HAUSDORFF && e.n_tp != f.n_tp) return "evaluator n_tp";   // Hausdorff: all of its target's vertices
+    return "";
+}
+
+__global__ void k_gather_target_rows(long long total, int row, const int *__restrict__ tidx, const double *__restrict__ src,
+                                     double *__restrict__ dst) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const long long c = i / row, k = i % row;
+    dst[i] = src[(size_t)tidx[c] * row + k];
+}
+
+}  // namespace
+
+extern "C" int32_t icp_chain_create_targets(icp_model m, int32_t n_targets, const icp_chain_target *targets, int32_t n_components,
+                                            int32_t max_chains, icp_chain *out) {
     icp_chain ch = nullptr;
     icp_ctx _ctx = m ? m->ctx : nullptr;
     try {
-        ICP_REQUIRE(m && t && components && evaluator && out, "null argument");
-        ICP_REQUIRE(m->ctx == t->ctx, "model and target belong to different contexts");
-        ICP_REQUIRE(evaluator->model == m && evaluator->target == t, "evaluator was built for another model / target");
+        ICP_REQUIRE(m && targets && out && n_targets >= 1, "null argument");
+        for (int g = 0; g < n_targets; g++) {
+            const icp_chain_target &e = targets[g];
+            ICP_REQUIRE(e.target && e.components && e.evaluator, "null argument (targets[" + std::to_string(g) + "])");
+            ICP_REQUIRE(m->ctx == e.target->ctx, "model and target belong to different contexts");
+            ICP_REQUIRE(e.evaluator->model == m && e.evaluator->target == e.target, "evaluator was built for another model / target");
+        }
         ICP_REQUIRE(n_components >= 1 && n_components <= kMaxComp, "1..16 mixture components supported");
         ICP_REQUIRE(max_chains >= 1, "max_chains must be >= 1");
         CtxLock lock(_ctx);
+        const icp_target t = targets[0].target;
+        const icp_component *components = targets[0].components;
+        const icp_evaluator evaluator = targets[0].evaluator;
+        for (int g = 0; g < n_targets; g++)
+            for (int i = 0; i < n_components; i++) {
+                const icp_component &ci = targets[g].components[i];
+                if (ci.kind == ICP_PROP_ICP)
+                    ICP_REQUIRE(ci.proposal && ci.proposal->model == m && ci.proposal->target == targets[g].target,
+                                "ICP component needs a proposal built for this model / target");
+            }
+        for (int g = 1; g < n_targets; g++) {
+            const std::string d = entry_difference(targets[0], targets[g], n_components);
+            ICP_REQUIRE(d.empty(), "targets[" + std::to_string(g) + "]: " + d + " differs from targets[0] (only the target may differ)");
+        }
         ch = new icp_chain_s();
         ch->model = m; ch->target = t; ch->evaluator = evaluator; ch->max_chains = max_chains;
+        ch->n_targets = n_targets;
+        for (int g = 0; g < n_targets; g++) {
+            ch->all_targets.push_back(targets[g].target);
+            ch->all_evals.push_back(targets[g].evaluator);
+            ch->set_boundary = ch->set_boundary || targets[g].target->has_boundary;
+        }
+        // with one target the boundary policy is that target's own
+        const bool has_boundary = n_targets > 1 ? ch->set_boundary : t->has_boundary;
         ChainParams &P = ch->P;
         P.n_comp = n_components; P.K = m->K; P.Kp = m->Kp; P.n_icp = 0;
         double wsum = 0;
@@ -692,8 +786,6 @@ extern "C" int32_t icp_chain_create(icp_model m, icp_target t, const icp_compone
             cd.cdf = i == n_components - 1 ? 1.0 : acc;
             switch (ci.kind) {
                 case ICP_PROP_ICP:
-                    ICP_REQUIRE(ci.proposal && ci.proposal->model == m && ci.proposal->target == t,
-                                "ICP component needs a proposal built for this model / target");
                     cd.icp_index = P.n_icp++;
                     cd.step = ci.proposal->prm.step_length;
                     cd.factor = ci.proposal->prm.factor;
@@ -732,7 +824,7 @@ extern "C" int32_t icp_chain_create(icp_model m, icp_target t, const icp_compone
                 for (int k = 0; k < P.n_icp; k++) {
                     icp_proposal pr = ch->icp_props[k];
                     if (pr->prm.direction != ICP_MODEL_SAMPLING || pr->n_ids == 0) continue;
-                    if (pr->prm.boundary_aware && t->has_boundary) continue;
+                    if (pr->prm.boundary_aware && has_boundary) continue;
                     std::vector<int> pids(pr->n_ids), map(pr->n_ids);
                     ICP_CUDA(cudaMemcpy(pids.data(), pr->ids.p, sizeof(int) * pids.size(), cudaMemcpyDeviceToHost));
                     bool ok = true;
@@ -752,14 +844,86 @@ extern "C" int32_t icp_chain_create(icp_model m, icp_target t, const icp_compone
         ICP_CUDA(cudaEventCreate(&ch->ev1));
         const char *env = getenv("ICPCUDA_NO_GRAPH");
         ch->use_graph = !(env && env[0] == '1');
-        m->refs++; t->refs++; evaluator->refs++;
-        for (icp_proposal pr : ch->icp_props) pr->refs++;
+        if (n_targets > 1) {
+            // the device table of the targets and every entry's point lists, laid end to end in entry order
+            cudaStream_t s = _ctx->stream;
+            std::vector<TargetRec> rec(n_targets);
+            for (int g = 0; g < n_targets; g++) {
+                const icp_target tg = targets[g].target;
+                rec[g] = TargetRec{{tg->tri_bvh.packed.p, tg->vert_bvh.packed.p}, {tg->tri_bvh.prim.p, tg->vert_bvh.prim.p},
+                                   {tg->tri_data.p, tg->vert_data.p}, {tg->tri_bvh.n, tg->vert_bvh.n}, tg->boundary.p, tg->Nt};
+            }
+            ch->trec.upload(rec.data(), rec.size(), s);
+            ch->tp_all.resize(P.n_icp);
+            ch->tp_lane.resize(P.n_icp);
+            for (int k = 0; k < P.n_icp; k++) {
+                const int n_tp = ch->icp_props[k]->n_tp;
+                if (ch->icp_props[k]->prm.direction != ICP_TARGET_SAMPLING || n_tp == 0) continue;
+                ch->tp_all[k].alloc((size_t)n_targets * n_tp * 3);
+                int j = 0;
+                for (int i = 0; i < n_components; i++) {   // the k-th ICP component of entry g
+                    if (components[i].kind != ICP_PROP_ICP || j++ != k) continue;
+                    for (int g = 0; g < n_targets; g++)
+                        ICP_CUDA(cudaMemcpyAsync(ch->tp_all[k].p + (size_t)g * n_tp * 3, targets[g].components[i].proposal->tp.p,
+                                                 sizeof(double) * n_tp * 3, cudaMemcpyDeviceToDevice, s));
+                }
+            }
+            for (int g = 0; g < n_targets; g++) ch->etp_n = std::max(ch->etp_n, targets[g].evaluator->n_tp);
+            if (ch->etp_n > 0) {
+                // Hausdorff targets may have different vertex counts: a shorter list is padded with repeats of its last
+                // vertex, which leaves the largest distance, the only one the evaluator keeps, unchanged
+                const int nm = ch->etp_n;
+                ch->etp_all.alloc((size_t)n_targets * nm * 3);
+                for (int g = 0; g < n_targets; g++) {
+                    const icp_evaluator eg = targets[g].evaluator;
+                    double *dst = ch->etp_all.p + (size_t)g * nm * 3;
+                    ICP_CUDA(cudaMemcpyAsync(dst, eg->tp.p, sizeof(double) * eg->n_tp * 3, cudaMemcpyDeviceToDevice, s));
+                    for (int r = eg->n_tp; r < nm; r++)
+                        ICP_CUDA(cudaMemcpyAsync(dst + (size_t)r * 3, eg->tp.p + (size_t)(eg->n_tp - 1) * 3, sizeof(double) * 3,
+                                                 cudaMemcpyDeviceToDevice, s));
+                }
+            }
+            ICP_CUDA(cudaStreamSynchronize(s));
+        }
+        m->refs++;
+        for (int g = 0; g < n_targets; g++) {
+            targets[g].target->refs++;
+            targets[g].evaluator->refs++;
+            for (int i = 0; i < n_components; i++)
+                if (targets[g].components[i].kind == ICP_PROP_ICP) {
+                    targets[g].components[i].proposal->refs++;
+                    ch->all_props.push_back(targets[g].components[i].proposal);
+                }
+        }
         *out = ch;
         return ICP_OK;
     } catch (...) {
         int32_t rc = translate_exception(_ctx);
         delete ch;
         return rc;
+    }
+}
+
+
+extern "C" int32_t icp_chain_create(icp_model m, icp_target t, const icp_component *components, int32_t n_components,
+                                    icp_evaluator evaluator, int32_t max_chains, icp_chain *out) {
+    const icp_chain_target one{t, components, evaluator};
+    return icp_chain_create_targets(m, 1, &one, n_components, max_chains, out);
+}
+
+extern "C" int32_t icp_chain_set_target_index(icp_chain c, int32_t C, const int32_t *target_index) {
+    icp_ctx _ctx = c ? c->model->ctx : nullptr;
+    try {
+        ICP_REQUIRE(_ctx != nullptr && target_index != nullptr, "null argument");
+        CtxLock lock(_ctx);
+        ICP_REQUIRE(C >= 1 && C <= c->max_chains, "C must be in [1, max_chains]");
+        for (int i = 0; i < C; i++)
+            ICP_REQUIRE(target_index[i] >= 0 && target_index[i] < c->n_targets,
+                        "target_index[" + std::to_string(i) + "] = " + std::to_string(target_index[i]) + " is outside [0, n_targets)");
+        c->tidx_req.assign(target_index, target_index + C);
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
     }
 }
 
@@ -775,8 +939,10 @@ extern "C" int32_t icp_chain_destroy(icp_chain c) {
         if (c->ev1) cudaEventDestroy(c->ev1);
         if (c->copy_ev) cudaEventDestroy(c->copy_ev);
         if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-        c->model->refs--; c->target->refs--; c->evaluator->refs--;
-        for (icp_proposal pr : c->icp_props) pr->refs--;
+        c->model->refs--;
+        for (icp_target t : c->all_targets) t->refs--;
+        for (icp_evaluator e : c->all_evals) e->refs--;
+        for (icp_proposal pr : c->all_props) pr->refs--;
         delete c;
         return ICP_OK;
     } catch (...) {
@@ -816,6 +982,13 @@ void enqueue_state_eval(RunCtx &r, const double *d_theta, double *d_values, cons
     static const bool forced_bvh = getenv("ICPCUDA_NEAREST_VERTEX") && std::string(getenv("ICPCUDA_NEAREST_VERTEX")) == "bvh";
     const bool fork = !g_prof && ch->use_streams && brute_ok && !forced_bvh;
     int n_side = 0;
+    // several targets: every consumer reads the batch entry's target from the table (TargetSet)
+    const bool multi = ch->n_targets > 1;
+    std::vector<TargetSet> tsv(ch->P.n_icp);
+    if (multi)
+        for (int i = 0; i < ch->P.n_icp; i++)
+            tsv[i] = TargetSet{ch->trec.p, ch->tidx.p, ch->set_boundary, ch->tp_lane[i].p, ch->icp_props[i]->n_tp};
+    const TargetSet ets{ch->trec.p, ch->tidx.p, ch->set_boundary, ch->etp_lane.p, ch->etp_n};
     if (fork) ICP_CUDA(cudaEventRecord(ctx->ev_fork, r.s));
     for (int i = 0; i < ch->P.n_icp; i++) {
         if (ch->cp_shared[i] || !fork || n_side >= icp_ctx_s::kAux) continue;
@@ -825,12 +998,12 @@ void enqueue_state_eval(RunCtx &r, const double *d_theta, double *d_values, cons
         double *Wb = ch->icp_props[i]->prm.factor == ICP_FACTOR_SVD ? r.st.W + (size_t)i * 2 * C * Kp * Kp : nullptr;
         QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
         posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, yb, d_slots, ss, nullptr, Wb, proposal ? &qa : nullptr,
-                           Wb == nullptr);
+                           Wb == nullptr, multi ? &tsv[i] : nullptr);
         ICP_CUDA(cudaEventRecord(ctx->ev_join[n_side], ss));
         ch->on_side[i] = 1;
         n_side++;
     }
-    evaluator_pipeline(ch->evaluator, ch->ework, Cn, d_theta, ch->X.p, d_values, ch->estatus.p, r.s);
+    evaluator_pipeline(ch->evaluator, ch->ework, Cn, d_theta, ch->X.p, d_values, ch->estatus.p, r.s, multi ? &ets : nullptr);
     for (int i = 0; i < ch->P.n_icp; i++) {
         if (ch->on_side[i]) { ch->on_side[i] = 0; continue; }
         double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *yb = r.st.ymean + (size_t)i * 2 * C * Kp;
@@ -838,7 +1011,7 @@ void enqueue_state_eval(RunCtx &r, const double *d_theta, double *d_values, cons
         double *Wb = ch->icp_props[i]->prm.factor == ICP_FACTOR_SVD ? r.st.W + (size_t)i * 2 * C * Kp * Kp : nullptr;
         QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
         posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, yb, d_slots, r.s, ch->cp_shared[i] ? &sh : nullptr, Wb,
-                           proposal ? &qa : nullptr, Wb == nullptr);
+                           proposal ? &qa : nullptr, Wb == nullptr, multi ? &tsv[i] : nullptr);
     }
     for (int k = 0; k < n_side; k++) ICP_CUDA(cudaStreamWaitEvent(r.s, ctx->ev_join[k], 0));   // join
 }
@@ -933,6 +1106,9 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
     ch->theta_best.ensure((size_t)C * Lt); ch->value_best.ensure(C);
     ch->qf.ensure((size_t)std::max(n_icp, 1) * C); ch->qb.ensure((size_t)std::max(n_icp, 1) * C);
     ICP_REQUIRE(io->metrics_interval >= 0, "metrics_interval must be >= 0");
+    ICP_REQUIRE(io->metrics_interval == 0 || ch->n_targets == 1,
+                "metrics_interval > 0 is not supported on a chain handle with several targets: measure each target's theta_best rows "
+                "with icp_registration_metrics after the run");
     ICP_REQUIRE(io->metrics_interval == 0 || io->log_metrics != nullptr, "metrics_interval > 0 needs log_metrics");
     ch->L.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp * Kp); ch->ymean.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp);
     ch->X.ensure((size_t)C * m->N * 3);
@@ -970,6 +1146,23 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
     r.rng = RngDev{io->seed, io->chain_id_offset, io->u_comp, io->z, io->u_acc, step_base};
     r.lg = LogDev{io->log_component, io->log_accepted, io->log_values, io->log_theta, step_base};
 
+    if (ch->n_targets > 1 && !resume) {
+        // the target of every batch entry (lane v of the look-ahead runs chain v % Cr) and the entries' own point lists
+        ICP_REQUIRE((int)ch->tidx_req.size() == Cr, "a chain handle with several targets needs icp_chain_set_target_index with C = " +
+                    std::to_string(Cr) + " entries before a run from theta0");
+        std::vector<int> lane(C);
+        for (int v = 0; v < C; v++) lane[v] = ch->tidx_req[v % Cr];
+        ch->tidx.upload(lane.data(), lane.size(), s);
+        auto gather = [&](const DevBuf<double> &all, DevBuf<double> &dst, int n) {
+            if (!all.p || n == 0) return;
+            const long long total = (long long)C * n * 3;
+            dst.ensure((size_t)total);
+            k_gather_target_rows<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(total, 3 * n, ch->tidx.p, all.p, dst.p);
+            ICP_CUDA(cudaGetLastError());
+        };
+        for (int k = 0; k < n_icp; k++) gather(ch->tp_all[k], ch->tp_lane[k], ch->icp_props[k]->n_tp);
+        gather(ch->etp_all, ch->etp_lane, ch->etp_n);
+    }
     ICP_CUDA(cudaEventRecord(ch->ev0, s));
     if (!resume && W > 1) {
         k_la_init<<<(C + 127) / 128, 128, 0, s>>>(Cr, W, Lt, theta0_dev, r.st);
@@ -1072,6 +1265,10 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
             const void *shared[] = {m->tri_bvh.nodes.p, m->tri_bvh.nodebox.p, m->tri_bvh.counters.p,
                                     m->vert_bvh.nodes.p, m->vert_bvh.nodebox.p, m->vert_bvh.counters.p};
             key.append((const char *)shared, sizeof shared);
+            // the target set: its table, the entries' target index and point lists
+            std::vector<const void *> tsp{ch->trec.p, ch->tidx.p, ch->etp_lane.p};
+            for (const DevBuf<double> &b : ch->tp_lane) tsp.push_back(b.p);
+            key.append((const char *)tsp.data(), sizeof(const void *) * tsp.size());
         }
         if (!(ch->exec && ch->exec_key == key)) {
             if (ch->exec) { cudaGraphExecDestroy(ch->exec); ch->exec = nullptr; }

@@ -146,6 +146,18 @@ struct WideBvh {
 };
 void wide_build(const Bvh &b, WideBvh &w, int L, cudaStream_t s);
 
+// One target of a chain handle's target set (icp_chain_create_targets) as the device reads it: the static triangle BVH
+// ([0]) and vertex BVH ([1]) of the target - packed nodes, leaf-slot -> primitive ids, Morton-ordered leaf data, leaf
+// count - and its boundary table. The chain runner uploads one record per target and a target index per batch entry.
+struct TargetRec {
+    const float4 *nodes[2];
+    const int *prim[2];
+    const double *data[2];
+    int n[2];
+    const uint8_t *boundary;   // [Nt]
+    int Nt;
+};
+
 struct NearestArgs {
     // structure
     const Bvh *bvh = nullptr;
@@ -177,6 +189,11 @@ struct NearestArgs {
     int *out_feat = nullptr;
     double *out_cp = nullptr;
     double *out_d2 = nullptr;
+    // several static targets in one launch: query row c walks the structure of record mt_rec[mt_idx[c]] (the triangle BVH
+    // for triangle queries, the vertex BVH for point queries) instead of bvh / prim_data, which then only give the
+    // primitive kind. Never takes the warp-cooperative kernel.
+    const TargetRec *mt_rec = nullptr;
+    const int *mt_idx = nullptr;
 };
 void launch_nearest(const NearestArgs &a, cudaStream_t s);
 // false: the arguments are outside the wide kernel's domain (nothing launched)
@@ -257,7 +274,8 @@ struct ObsArgs {
     const int *cp_map;
     const uint8_t *cp_on_boundary;  // [C][n] or nullptr
     // target sampling: nearest current-mesh vertex per target point
-    const double *tp;      // [n][3]
+    const double *tp;      // [n][3], or [C][n][3] when tp_per_chain
+    int tp_per_chain;
     const int *near_vid;   // [C][n]
     int iso;               // 1: isotropic noise sigma2 (deterministic ICP), frame = I / sqrt(sigma2)
     double iso_sigma2;
@@ -346,9 +364,10 @@ struct EvalReduceArgs {
 };
 void launch_eval_reduce(const EvalReduceArgs &a, cudaStream_t s);
 void launch_prior(int C, int K, const double *d_theta, double *d_out, cudaStream_t s);
-// flags[c][i] = table[prim[c][i]]
+// flags[c][i] = table[prim[c][i]]; with rec / tidx (several targets) the table of row c is rec[tidx[c]].boundary, rows of
+// `per` entries
 void launch_lookup_flags(int64_t n, const int *d_prim, const uint8_t *d_table, int table_n, uint8_t *d_flags,
-                         cudaStream_t s);
+                         cudaStream_t s, const TargetRec *rec = nullptr, const int *tidx = nullptr, int64_t per = 1);
 
 }  // namespace icp
 
@@ -621,14 +640,24 @@ struct SharedCp {
     int stride;
     const int *map;     // [n_ids] index into the shared list
 };
+// Several targets in one batch (the chain runner of a target set): entry c of the batch fits target rec[tidx[c]], and a
+// consumer whose point list belongs to the target reads the entry's own copy tp [C][n_tp][3]. has_boundary is the OR over
+// the targets: it decides the boundary path (no closest-point sharing, no constant-Gram path) for every entry.
+struct TargetSet {
+    const TargetRec *rec;   // [G]
+    const int *tidx;        // [C]
+    bool has_boundary;
+    const double *tp;       // [C][n_tp][3] (target sampling / the evaluator's target -> model queries), else null
+    int n_tp;               // entries per row of tp (the Hausdorff evaluator: the largest Nt, shorter lists padded)
+};
 // d_W (nullable, [slot][Kp][Kp]): also the reference's SVD-based covariance factor (ICP_FACTOR_SVD)
 // ymean: d_mu receives y = L^-1 b instead of mu (see launch_posterior_fused); only the chain runner asks for it
 void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, double *d_L,
                         double *d_mu, const int *d_out_slot, cudaStream_t s, const SharedCp *shared = nullptr,
-                        double *d_W = nullptr, const QuadArgs *qa = nullptr, bool ymean = false);
-// distance evaluator pipeline: values [C][3] = {product, prior, distance}
+                        double *d_W = nullptr, const QuadArgs *qa = nullptr, bool ymean = false, const TargetSet *ts = nullptr);
+// distance evaluator pipeline: values [C][3] = {product, prior, distance}; ts: see TargetSet
 void evaluator_pipeline(icp_evaluator e, EvalWork &w, int C, const double *d_theta, const double *d_X, double *d_values,
-                        int *d_status, cudaStream_t s);
+                        int *d_status, cudaStream_t s, const TargetSet *ts = nullptr);
 // RAII: selects the context device, serialises calls on the context
 struct CtxLock {
     std::unique_lock<std::mutex> lk;

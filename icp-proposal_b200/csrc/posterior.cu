@@ -69,6 +69,7 @@ __device__ __forceinline__ void observations_grouped(const ObsArgs &a, const Obs
     int *s_cnt = s_int, *s_off = s_cnt + N, *s_slot = s_off + N, *s_cur = s_slot + N, *s_seg = s_cur + N;
     __shared__ int s_part[2][256], s_tot[2];
     const int *near = a.near_vid + (size_t)c * n;
+    const double *tp = a.tp + (a.tp_per_chain ? (size_t)c * n * 3 : 0);
     for (int v = tid; v < N; v += nt) { s_cnt[v] = 0; s_cur[v] = 0; }
     __syncthreads();
     for (int i = tid; i < n; i += nt) {
@@ -116,8 +117,8 @@ __device__ __forceinline__ void observations_grouped(const ObsArgs &a, const Obs
         for (int p = 0; p < mv; p++) {
             const int i = seg[p];
             double ix, iy, iz;
-            if (a.world_frame) { ix = a.tp[3 * i]; iy = a.tp[3 * i + 1]; iz = a.tp[3 * i + 2]; }
-            else inverse_pose(th, R, a.tp[3 * i], a.tp[3 * i + 1], a.tp[3 * i + 2], ix, iy, iz);  // :129
+            if (a.world_frame) { ix = tp[3 * i]; iy = tp[3 * i + 1]; iz = tp[3 * i + 2]; }
+            else inverse_pose(th, R, tp[3 * i], tp[3 * i + 1], tp[3 * i + 2], ix, iy, iz);  // :129
             s0 += (ix - m.ref[3 * v]) - m.mean[3 * v];
             s1 += (iy - m.ref[3 * v + 1]) - m.mean[3 * v + 1];
             s2 += (iz - m.ref[3 * v + 2]) - m.mean[3 * v + 2];
@@ -192,7 +193,8 @@ __global__ void __launch_bounds__(256) k_observations(ObsArgs a, ObsDev o) {
         bool drop = false;
         if (a.prm.direction == ICP_TARGET_SAMPLING) {
             id = a.near_vid[g];                                         // :118 findClosestPoint on the current mesh
-            tx = a.tp[3 * i]; ty = a.tp[3 * i + 1]; tz = a.tp[3 * i + 2];
+            const double *tpi = a.tp + ((a.tp_per_chain ? (size_t)c * o.n : 0) + i) * 3;
+            tx = tpi[0]; ty = tpi[1]; tz = tpi[2];
             if (id < 0) drop = true;
             else if (a.prm.boundary_aware && m.boundary[id]) drop = true;  // :119,124
         } else {

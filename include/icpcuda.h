@@ -298,6 +298,30 @@ int32_t icp_chain_create(icp_model m, icp_target t, const icp_component *compone
                          icp_evaluator evaluator, int32_t max_chains, icp_chain *out);
 int32_t icp_chain_destroy(icp_chain c);
 
+/* Several targets in one chain handle: every chain names its own target, and the chains of all targets run in the same
+ * batched launches (icp_chain_create is the one-target case). Entry g holds a target, the mixture built for it and its
+ * evaluator. Only the targets may differ: every entry has the same component kinds, weights, sd and axes; the ICP
+ * proposals share the model, every icp_proposal_params field, the model point ids and n_tp; the evaluators share kind,
+ * mode, use_prior, p0 - p2, the model point ids and n_tp (not the Hausdorff evaluator, whose list is all vertices of its
+ * target: shorter lists are padded with repeats of their last vertex, which does not change the maximum). Any other
+ * difference is refused with ICP_ERR_INVALID_ARGUMENT and a message naming the field. The handle holds references on
+ * every target, proposal and evaluator.
+ * Boundary policy: the boundary path (no closest-point sharing with the evaluator, no constant-Gram posterior) is taken
+ * for every chain when any target has a boundary, so a chain on a closed target of such a set agrees with its
+ * single-target run to rounding, not bit for bit. Runs with metrics_interval > 0 are refused when n_targets > 1
+ * (icp_registration_metrics on each target's rows of theta_best afterwards gives the same measures). */
+typedef struct {
+    icp_target target;
+    const icp_component *components;  /* n_components entries */
+    icp_evaluator evaluator;          /* built for (model, target) */
+} icp_chain_target;
+int32_t icp_chain_create_targets(icp_model m, int32_t n_targets, const icp_chain_target *targets, int32_t n_components,
+                                 int32_t max_chains, icp_chain *out);
+/* target_index [C] (host): chain c runs on targets[target_index[c]]. Takes effect at the next run from theta0; resumed runs
+ * keep the assignment. Required before the first run of a handle with n_targets > 1 (and again whenever a run from theta0
+ * has a different C). Sharded runs pass the indices of their own chains. */
+int32_t icp_chain_set_target_index(icp_chain c, int32_t C, const int32_t *target_index);
+
 typedef struct {
     /* randomness: either counter-based on the device (Philox4x32-10 keyed by seed and the global
      * chain id chain_id_offset + c, so results do not depend on how chains are sharded over GPUs)
