@@ -314,6 +314,17 @@ constexpr int kStackShared = 12;   // stack entries per thread kept in shared me
 constexpr int kNearestThreads = 128;
 constexpr int kDone = 0x7ffffffe;
 
+#ifdef ICP_CP_TIMING
+// experiment build only (ICPCUDA_LIB_TAG=timing ICPCUDA_NVCC_EXTRA=-DICP_CP_TIMING, tools/cp_chain_major.py): k_nearest
+// adds up, over all its launches since the last reset, [0] warp iterations and [1] lane iterations of the descent phase,
+// [2] warp rounds and [3] lane tests of the leaf phase, [4] warps and [5] live queries. [1] / [0] is the number of lanes
+// active per node visit, [3] / [2] per leaf test.
+__device__ unsigned long long g_cp_count[6];
+#define ICP_CPT(...) __VA_ARGS__
+#else
+#define ICP_CPT(...)
+#endif
+
 // Traversal in two alternating phases per warp ("while-while" with postponed leaves): every lane first descends through
 // internal nodes until it holds a leaf (or has nothing left), then the warp reconverges and all lanes holding a leaf run
 // the exact FP64 primitive test together. Static structures read one 64-byte packed node (child boxes + child links);
@@ -362,10 +373,15 @@ __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int
         if (lpw < 32) g = (g >> 5) * lpw + (threadIdx.x & 31);
         live = (lpw >= 32 || (int)(threadIdx.x & 31) < lpw) && g < nq * C;
         if (!live) g = nq * C - 1;   // idle lanes stay in the warp-synchronous loop, write nothing
-        c = (int)(g / nq);
-        i = g % nq;
+        // chain-major: consecutive lanes take the same query row of consecutive chains. The same model point in different
+        // chains lies a few mm apart (a quarter of a target edge), so the lanes of a warp walk nearly the same nodes to the
+        // same leaves and finish together; 32 consecutive rows of one chain spread over ~40 mm of the surface. With C = 1
+        // this is the row order itself.
+        if (nq * C <= 0x7fffffffLL) { const int gi = (int)g; c = gi % C; i = gi / C; }
+        else { c = (int)(g % C); i = g / C; }
     }
-    if (perm) { i = perm[i]; g = (long long)c * nq + i; }  // spatially sorted processing order, results in caller order
+    if (perm) i = perm[i];   // spatially sorted processing order, results in caller order
+    if (!HDMAX) g = (long long)c * nq + i;
     if (MT) {
         const TargetRec &r = mt_rec[__ldg(mt_idx + c)];
         n = r.n[PRIM]; nodes = r.nodes[PRIM]; prim = r.prim[PRIM]; prim_data = r.data[PRIM];
@@ -414,8 +430,11 @@ __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int
         }
         return nn;
     };
+    ICP_CPT(unsigned cnt_desc = 0, cnt_leaf = 0, cnt_wdesc = 0, cnt_wleaf = 0;)
     while (true) {
+        ICP_CPT(unsigned cnt_round = 0;)
         while ((unsigned)node < (unsigned)kDone) {   // internal node
+            ICP_CPT(cnt_round++;)
             int2 ch;
             float4 a, b, cc;
             if (DYNAMIC) {
@@ -442,6 +461,8 @@ __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int
             else node = pop();
         }
         const bool at_leaf = node != kDone;
+        ICP_CPT(cnt_desc += cnt_round; cnt_wdesc += __reduce_max_sync(0xffffffffu, cnt_round);
+                cnt_leaf += at_leaf; cnt_wleaf += __any_sync(0xffffffffu, at_leaf);)
         if (!__any_sync(0xffffffffu, at_leaf)) break;
         if (at_leaf) {
             leaf_test<PRIM, DYNAMIC>(~node, prim, prim_data, Xi, tris, qx, qy, qz, h);
@@ -450,6 +471,15 @@ __global__ void __launch_bounds__(kNearestThreads, 7) k_nearest(int n, const int
             if (HDMAX && node != kDone && __double_as_longlong(h.d2) <= (long long)__ldcg(cmax)) { node = kDone; pruned = true; }
         }
     }
+    ICP_CPT({
+        const unsigned sd = __reduce_add_sync(0xffffffffu, cnt_desc), sl = __reduce_add_sync(0xffffffffu, cnt_leaf),
+                       nl = __reduce_add_sync(0xffffffffu, live ? 1u : 0u);
+        if ((threadIdx.x & 31) == 0) {
+            atomicAdd(&g_cp_count[0], (unsigned long long)cnt_wdesc); atomicAdd(&g_cp_count[1], (unsigned long long)sd);
+            atomicAdd(&g_cp_count[2], (unsigned long long)cnt_wleaf); atomicAdd(&g_cp_count[3], (unsigned long long)sl);
+            atomicAdd(&g_cp_count[4], 1ull); atomicAdd(&g_cp_count[5], (unsigned long long)nl);
+        }
+    })
     if (!live) return;
     if (HDMAX && !pruned && h.d2 == h.d2 && h.prim != 0x7fffffff) atomicMax(chain_max + c, (unsigned long long)__double_as_longlong(h.d2));
     if (h.prim == 0x7fffffff) { h.d2 = NAN; h.x = h.y = h.z = NAN; h.prim = -1; }
@@ -820,3 +850,16 @@ void launch_lookup_flags(int64_t n, const int *d_prim, const uint8_t *d_table, i
 }
 
 }  // namespace icp
+
+#ifdef ICP_CP_TIMING
+// copies the six k_nearest counters to out (host memory); reset != 0 then clears them
+extern "C" int32_t icp_debug_cp_counters(unsigned long long *out, int32_t reset) {
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e == cudaSuccess && out) e = cudaMemcpyFromSymbol(out, icp::g_cp_count, sizeof(icp::g_cp_count));
+    if (e == cudaSuccess && reset) {
+        const unsigned long long zero[6] = {0, 0, 0, 0, 0, 0};
+        e = cudaMemcpyToSymbol(icp::g_cp_count, zero, sizeof(zero));
+    }
+    return (int32_t)e;
+}
+#endif
