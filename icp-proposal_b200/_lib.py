@@ -76,6 +76,10 @@ class StdIcpIO(C.Structure):
                 ("log_alpha", C.c_void_p), ("log_direction", C.c_void_p), ("status", C.c_void_p), ("iterations_done", C.c_void_p)]
 
 
+class StdIcpTarget(C.Structure):
+    _fields_ = [("target", _h), ("target_points", _dp)]
+
+
 class ChainStatsParams(C.Structure):
     _fields_ = [("burn_in", C.c_int64), ("take_every_n", C.c_int64), ("end", C.c_int64), ("normals", C.c_int32),
                 ("reserved", C.c_int32)]
@@ -109,6 +113,9 @@ _SIGS = {
     "icp_std_icp_iteration": [_h, _h, C.c_int32, _ip, C.c_int32, _dp, C.c_int32, C.c_double, C.c_double, C.c_int32, _dp, _dp],
     "icp_std_icp_iteration_theta": [_h, _h, C.c_int32, _ip, C.c_int32, _dp, C.c_int32, C.c_double, C.c_double, C.c_int32, _dp, _dp],
     "icp_std_icp_create": [_h, _h, _ip, C.c_int32, _dp, C.c_int32, C.c_double, C.c_int32, C.c_int32, C.POINTER(_h)],
+    "icp_std_icp_create_targets": [_h, C.c_int32, C.POINTER(StdIcpTarget), _ip, C.c_int32, C.c_int32, C.c_double, C.c_int32,
+                                   C.c_int32, C.POINTER(_h)],
+    "icp_std_icp_set_target_index": [_h, C.c_int32, _ip],
     "icp_std_icp_destroy": [_h],
     "icp_std_icp_run": [_h, C.c_int32, _dp, C.c_int32, _dp, C.c_int32, C.POINTER(StdIcpIO)],
     "icp_std_icp_run_device": [_h, C.c_int32, C.c_void_p, C.c_int32, _dp, C.c_int32, C.POINTER(StdIcpIO), C.c_int32],

@@ -793,10 +793,8 @@ class IcpBasedSurfaceFitting:
         self.ids = (self.rand.integers(0, model.N, numOfSamplePoints) if model_point_ids is None else np.asarray(model_point_ids)).astype(np.int32)
         self.tp = _decimated_points(target, numOfSamplePoints) if target_points is None else np.asarray(target_points, float)
 
-    def runfitting(self, numIterations, iterationSeq=(1.0, 0.1, 0.01), initialCoefficients=None, directions=None):
-        """The whole loop on the device (core.StdIcp). initialCoefficients of shape (C, K) runs C independent fits and returns
-        C instances (self.coefficients becomes C x K); directions is then (iterations, C) or (iterations,) for all fits. With
-        ModelAndTargetSampling and no directions the coin is self.rand, drawn iteration by iteration (fit by fit) as before."""
+    def _plan(self, numIterations, iterationSeq, initialCoefficients, directions):
+        """(batched, theta0 (C, K + 10), directions (iters, C)) of runfitting's arguments; draws the coins from self.rand."""
         K = self.model.K
         batched = initialCoefficients is not None and np.ndim(initialCoefficients) == 2
         alpha = np.zeros((1, K)) if initialCoefficients is None else np.asarray(initialCoefficients, float).reshape(-1, K)
@@ -811,17 +809,61 @@ class IcpBasedSurfaceFitting:
         else:
             target = np.full((iters, n_fits), self.projectionDirection == TargetSampling)
         theta0 = np.stack([self.model.theta(alpha=a, center=(0, 0, 0)) for a in alpha])
-        runner = core.StdIcp(self.model, self.target, self.ids, self.tp, self.stepLength, _lib.MODEL_SAMPLING, n_fits)
+        return batched, theta0, np.where(target, _lib.TARGET_SAMPLING, _lib.MODEL_SAMPLING).astype(np.int32)
+
+    def _finish(self, batched, alpha_final):
+        if batched:
+            self.coefficients = alpha_final
+            return [self.model.instance(a) for a in alpha_final]
+        self.coefficients = alpha_final[0]
+        return self.model.instance(alpha_final[0])
+
+    def runfitting(self, numIterations, iterationSeq=(1.0, 0.1, 0.01), initialCoefficients=None, directions=None):
+        """The whole loop on the device (core.StdIcp). initialCoefficients of shape (C, K) runs C independent fits and returns
+        C instances (self.coefficients becomes C x K); directions is then (iterations, C) or (iterations,) for all fits. With
+        ModelAndTargetSampling and no directions the coin is self.rand, drawn iteration by iteration (fit by fit) as before."""
+        batched, theta0, dirs = self._plan(numIterations, iterationSeq, initialCoefficients, directions)
+        runner = core.StdIcp(self.model, self.target, self.ids, self.tp, self.stepLength, _lib.MODEL_SAMPLING, len(theta0))
         try:
-            out = runner.run(theta0, np.asarray(iterationSeq, float), numIterations,
-                             directions=np.where(target, _lib.TARGET_SAMPLING, _lib.MODEL_SAMPLING), log=False)
+            out = runner.run(theta0, np.asarray(iterationSeq, float), numIterations, directions=dirs, log=False)
         finally:
             runner.close()
-        if batched:
-            self.coefficients = out["alpha_final"]
-            return [self.model.instance(a) for a in out["alpha_final"]]
-        self.coefficients = out["alpha_final"][0]
-        return self.model.instance(out["alpha_final"][0])
+        return self._finish(batched, out["alpha_final"])
+
+    @staticmethod
+    def runfittings(fittings, numIterations, iterationSeq=(1.0, 0.1, 0.01), initialCoefficients=None, directions=None):
+        """runfitting of several fittings of one model, typically one per target, as one device run (a core.StdIcp target
+        set). initialCoefficients and directions hold one entry per fitting, each as runfitting takes it (None: runfitting's
+        default for every fitting). Each fitting draws its coins from its own self.rand and gets its own coefficients, so its
+        result equals its own runfitting. Returns the list of what each fitting's runfitting returns."""
+        fittings = list(fittings)
+        if not fittings:
+            raise ValueError("runfittings needs at least one fitting")
+        f0 = fittings[0]
+        for g, f in enumerate(fittings[1:], 1):
+            for field, same in (("model", f.model is f0.model), ("model_point_ids", np.array_equal(f.ids, f0.ids)),
+                                ("stepLength", f.stepLength == f0.stepLength),
+                                ("projectionDirection", f.projectionDirection == f0.projectionDirection)):
+                if not same:
+                    raise ValueError(f"fittings[{g}].{field} differs from fittings[0]: only the target may differ")
+        inits = [None] * len(fittings) if initialCoefficients is None else list(initialCoefficients)
+        dirs_in = [None] * len(fittings) if directions is None else list(directions)
+        if len(inits) != len(fittings) or len(dirs_in) != len(fittings):
+            raise ValueError("initialCoefficients and directions need one entry per fitting")
+        plans = [f._plan(numIterations, iterationSeq, a, d) for f, a, d in zip(fittings, inits, dirs_in)]
+        counts = [len(p[1]) for p in plans]
+        theta0 = np.concatenate([p[1] for p in plans])
+        dirs = np.concatenate([p[2] for p in plans], axis=1)
+        tidx = np.repeat(np.arange(len(fittings)), counts)
+        runner = core.StdIcp(f0.model, model_point_ids=f0.ids, step_length=f0.stepLength, direction=_lib.MODEL_SAMPLING,
+                             max_fits=len(theta0), targets=[(f.target, f.tp) for f in fittings])
+        try:
+            out = runner.run(theta0, np.asarray(iterationSeq, float), numIterations, directions=dirs, log=False,
+                             target_index=tidx if len(fittings) > 1 else None)
+        finally:
+            runner.close()
+        ends = np.cumsum(counts)
+        return [f._finish(p[0], out["alpha_final"][e - n:e]) for f, p, n, e in zip(fittings, plans, counts, ends)]
 
 
 class RegistrationComparison:

@@ -263,19 +263,46 @@ def std_icp_iteration_theta(model: Model, target: Target, direction, model_point
 class StdIcp:
     """Device-resident IcpBasedSurfaceFitting.runfitting for batches of independent fits (icp_std_icp_*)."""
 
-    def __init__(self, model: Model, target: Target, model_point_ids, target_points, step_length=1.0,
-                 direction=_lib.MODEL_SAMPLING, max_fits=1):
-        self.model, self.target, self.lib, self.ctx = model, target, model.lib, model.ctx
+    def __init__(self, model: Model, target: Target = None, model_point_ids=None, target_points=None, step_length=1.0,
+                 direction=_lib.MODEL_SAMPLING, max_fits=1, targets=None):
+        """targets: instead of (target, target_points), a list of such pairs, one per target of the handle
+        (icp_std_icp_create_targets); run() then needs target_index."""
+        self.model, self.lib, self.ctx = model, model.lib, model.ctx
+        if targets is None:
+            targets = [(target, target_points)]
+        elif target is not None or target_points is not None:
+            raise ValueError("pass either target and target_points or targets")
+        self.targets = [(t, f64(np.asarray(tp, dtype=np.float64).reshape(-1, 3))) for t, tp in targets]
+        self.target, self.tp = self.targets[0]
+        self.n_targets = len(self.targets)
+        for g, (_, tp) in enumerate(self.targets):
+            if len(tp) != len(self.tp):   # the C ABI takes one n_tp for every entry
+                raise ValueError(f"targets[{g}] has {len(tp)} target points, targets[0] has {len(self.tp)}")
         self.ids = i32(np.asarray(model_point_ids).reshape(-1))
-        self.tp = f64(np.asarray(target_points, dtype=np.float64).reshape(-1, 3))
         self.max_fits = int(max_fits)
         self.h = C.c_void_p()
-        check(self.lib.icp_std_icp_create(model.h, target.h, iptr(self.ids), len(self.ids), dptr(self.tp), len(self.tp),
-                                          float(step_length), int(direction), self.max_fits, C.byref(self.h)), self.ctx.h)
+        if self.n_targets == 1:
+            check(self.lib.icp_std_icp_create(model.h, self.target.h, iptr(self.ids), len(self.ids), dptr(self.tp), len(self.tp),
+                                              float(step_length), int(direction), self.max_fits, C.byref(self.h)), self.ctx.h)
+        else:
+            ents = (_lib.StdIcpTarget * self.n_targets)()
+            for g, (t, tp) in enumerate(self.targets):
+                ents[g].target, ents[g].target_points = t.h, dptr(tp)
+            check(self.lib.icp_std_icp_create_targets(model.h, self.n_targets, ents, iptr(self.ids), len(self.ids), len(self.tp),
+                                                      float(step_length), int(direction), self.max_fits, C.byref(self.h)),
+                  self.ctx.h)
 
-    def run(self, theta0, sigma2, num_iterations, directions=None, seed=1024, fit_id_offset=0, log=True):
-        """theta0 (C, K + 10); sigma2: iterationSeq; directions (iters, C) or None. Returns dict(alpha_final (C, K), status (C,),
-        iterations_done (C,), and with log=True log_alpha (iters, C, K) and log_direction (iters, C))."""
+    def set_target_index(self, target_index):
+        """icp_std_icp_set_target_index: fit c of every later run with this C runs on targets[target_index[c]]."""
+        ti = np.ascontiguousarray(target_index, dtype=np.int32).reshape(-1)
+        check(self.lib.icp_std_icp_set_target_index(self.h, len(ti), ti.ctypes.data_as(_lib._ip)), self.ctx.h)
+
+    def run(self, theta0, sigma2, num_iterations, directions=None, seed=1024, fit_id_offset=0, log=True, target_index=None):
+        """theta0 (C, K + 10); sigma2: iterationSeq; directions (iters, C) or None; target_index (C,): the target of every fit
+        (set_target_index before the run). Returns dict(alpha_final (C, K), status (C,), iterations_done (C,), and with log=True
+        log_alpha (iters, C, K) and log_direction (iters, C))."""
+        if target_index is not None:
+            self.set_target_index(target_index)
         th, c = self.model._theta(theta0)
         s2 = f64(np.atleast_1d(sigma2))
         K, iters = self.model.K, len(s2) * (int(num_iterations) + 1)
@@ -294,8 +321,10 @@ class StdIcp:
         return out
 
     def run_device(self, C_, theta0_ptr, sigma2, num_iterations, directions=0, seed=1024, fit_id_offset=0, alpha_final=0,
-                   log_alpha=0, log_direction=0, status=0, iterations_done=0, async_=False):
-        """All pointers are raw device addresses (e.g. torch.Tensor.data_ptr()); sigma2 is a host sequence."""
+                   log_alpha=0, log_direction=0, status=0, iterations_done=0, async_=False, target_index=None):
+        """All pointers are raw device addresses (e.g. torch.Tensor.data_ptr()); sigma2 and target_index are host sequences."""
+        if target_index is not None:
+            self.set_target_index(target_index)
         s2 = f64(np.atleast_1d(sigma2))
         io = _lib.StdIcpIO()
         io.seed, io.fit_id_offset, io.directions = int(seed), int(fit_id_offset), directions or None

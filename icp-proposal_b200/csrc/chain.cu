@@ -720,6 +720,10 @@ std::string entry_difference(const icp_chain_target &a, const icp_chain_target &
     return "";
 }
 
+}  // namespace
+
+namespace icp {
+
 __global__ void k_gather_target_rows(long long total, int row, const int *__restrict__ tidx, const double *__restrict__ src,
                                      double *__restrict__ dst) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -728,7 +732,24 @@ __global__ void k_gather_target_rows(long long total, int row, const int *__rest
     dst[i] = src[(size_t)tidx[c] * row + k];
 }
 
-}  // namespace
+void launch_gather_target_rows(int C, int row, const int *d_tidx, const double *d_src, double *d_dst, cudaStream_t s) {
+    const long long total = (long long)C * row;
+    if (total <= 0) return;
+    k_gather_target_rows<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(total, row, d_tidx, d_src, d_dst);
+    ICP_CUDA(cudaGetLastError());
+}
+
+void upload_target_table(const std::vector<icp_target> &targets, DevBuf<TargetRec> &table, cudaStream_t s) {
+    std::vector<TargetRec> rec(targets.size());
+    for (size_t g = 0; g < targets.size(); g++) {
+        const icp_target tg = targets[g];
+        rec[g] = TargetRec{{tg->tri_bvh.packed.p, tg->vert_bvh.packed.p}, {tg->tri_bvh.prim.p, tg->vert_bvh.prim.p},
+                           {tg->tri_data.p, tg->vert_data.p}, {tg->tri_bvh.n, tg->vert_bvh.n}, tg->boundary.p, tg->Nt};
+    }
+    table.upload(rec.data(), rec.size(), s);
+}
+
+}  // namespace icp
 
 extern "C" int32_t icp_chain_create_targets(icp_model m, int32_t n_targets, const icp_chain_target *targets, int32_t n_components,
                                             int32_t max_chains, icp_chain *out) {
@@ -847,13 +868,7 @@ extern "C" int32_t icp_chain_create_targets(icp_model m, int32_t n_targets, cons
         if (n_targets > 1) {
             // the device table of the targets and every entry's point lists, laid end to end in entry order
             cudaStream_t s = _ctx->stream;
-            std::vector<TargetRec> rec(n_targets);
-            for (int g = 0; g < n_targets; g++) {
-                const icp_target tg = targets[g].target;
-                rec[g] = TargetRec{{tg->tri_bvh.packed.p, tg->vert_bvh.packed.p}, {tg->tri_bvh.prim.p, tg->vert_bvh.prim.p},
-                                   {tg->tri_data.p, tg->vert_data.p}, {tg->tri_bvh.n, tg->vert_bvh.n}, tg->boundary.p, tg->Nt};
-            }
-            ch->trec.upload(rec.data(), rec.size(), s);
+            upload_target_table(ch->all_targets, ch->trec, s);
             ch->tp_all.resize(P.n_icp);
             ch->tp_lane.resize(P.n_icp);
             for (int k = 0; k < P.n_icp; k++) {
@@ -1155,10 +1170,8 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
         ch->tidx.upload(lane.data(), lane.size(), s);
         auto gather = [&](const DevBuf<double> &all, DevBuf<double> &dst, int n) {
             if (!all.p || n == 0) return;
-            const long long total = (long long)C * n * 3;
-            dst.ensure((size_t)total);
-            k_gather_target_rows<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(total, 3 * n, ch->tidx.p, all.p, dst.p);
-            ICP_CUDA(cudaGetLastError());
+            dst.ensure((size_t)C * n * 3);
+            launch_gather_target_rows(C, 3 * n, ch->tidx.p, all.p, dst.p, s);
         };
         for (int k = 0; k < n_icp; k++) gather(ch->tp_all[k], ch->tp_lane[k], ch->icp_props[k]->n_tp);
         gather(ch->etp_all, ch->etp_lane, ch->etp_n);

@@ -146,9 +146,10 @@ struct WideBvh {
 };
 void wide_build(const Bvh &b, WideBvh &w, int L, cudaStream_t s);
 
-// One target of a chain handle's target set (icp_chain_create_targets) as the device reads it: the static triangle BVH
-// ([0]) and vertex BVH ([1]) of the target - packed nodes, leaf-slot -> primitive ids, Morton-ordered leaf data, leaf
-// count - and its boundary table. The chain runner uploads one record per target and a target index per batch entry.
+// One target of a target set (icp_chain_create_targets, icp_std_icp_create_targets) as the device reads it: the static
+// triangle BVH ([0]) and vertex BVH ([1]) of the target - packed nodes, leaf-slot -> primitive ids, Morton-ordered leaf
+// data, leaf count - and its boundary table. A runner uploads one record per target (upload_target_table) and a target
+// index per batch entry.
 struct TargetRec {
     const float4 *nodes[2];
     const int *prim[2];
@@ -368,6 +369,8 @@ void launch_prior(int C, int K, const double *d_theta, double *d_out, cudaStream
 // `per` entries
 void launch_lookup_flags(int64_t n, const int *d_prim, const uint8_t *d_table, int table_n, uint8_t *d_flags,
                          cudaStream_t s, const TargetRec *rec = nullptr, const int *tidx = nullptr, int64_t per = 1);
+// dst[c][k] = src[tidx[c]][k] for C rows of `row` doubles: every batch entry's copy of its target's point list
+void launch_gather_target_rows(int C, int row, const int *d_tidx, const double *d_src, double *d_dst, cudaStream_t s);
 
 }  // namespace icp
 
@@ -439,6 +442,9 @@ struct icp_target_s {
 };
 
 namespace icp {
+
+// the device table of a target set: record g describes targets[g] (TargetRec), uploaded on s
+void upload_target_table(const std::vector<icp_target> &targets, DevBuf<TargetRec> &table, cudaStream_t s);
 
 // per-batch workspace of the correspondence + posterior pipeline of one ICP proposal
 struct PosteriorWork {

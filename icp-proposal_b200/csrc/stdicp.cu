@@ -11,6 +11,9 @@
 // Each iteration sorts its fits into a model-sampling range and a target-sampling range (k_si_gather, k_si_scatter); the
 // split is known on the host before the run (caller directions, or the Philox coin, a pure function of seed, fit, iteration),
 // and one CUDA graph per (C, split, sigma) is captured and replayed.
+// A handle may hold several targets (icp_std_icp_create_targets): every fit names its own, a model-sampling slot walks its
+// target's BVH (the multi-target k_nearest) and a target-sampling slot reads its target's point list. G_s, the projectors
+// and the graphs depend on the model and the model point ids only, so every fit equals its single-target run bit for bit.
 #include <cmath>
 #include <cstring>
 #include <map>
@@ -53,13 +56,14 @@ __global__ void k_si_init(int C, int Lt, const double *__restrict__ theta0, doub
 }
 
 // work slot p <- fit perm[iter][p]: parameters (a stopped fit runs on the identity instance so that every query stays finite;
-// its result is discarded) and its closest-point traversal seeds
+// its result is discarded), its closest-point traversal seeds and, on a target set (tidx != nullptr), its target
 __global__ void k_si_gather(int C, int Lt, int nm, int n_ids, int n_tp, const int *__restrict__ iter, const RunIo *__restrict__ io,
                             const double *__restrict__ theta, const int *__restrict__ status, double *__restrict__ theta_w,
                             const int *__restrict__ seed_m, const int *__restrict__ seed_t, int *__restrict__ wseed_m,
-                            int *__restrict__ wseed_t) {
+                            int *__restrict__ wseed_t, const int *__restrict__ tidx, int *__restrict__ wtidx) {
     const int p = blockIdx.x, c = io->perm[(size_t)(*iter) * C + p];
     const bool stopped = status[c] != 0;
+    if (tidx && threadIdx.x == 0) wtidx[p] = tidx[c];
     for (int e = threadIdx.x; e < Lt; e += blockDim.x)
         theta_w[(size_t)p * Lt + e] = stopped ? (e == 0 ? 1.0 : 0.0) : theta[(size_t)c * Lt + e];
     if (p < nm) for (int i = threadIdx.x; i < n_ids; i += blockDim.x) wseed_m[(size_t)p * n_ids + i] = seed_m[(size_t)c * n_ids + i];
@@ -258,11 +262,19 @@ void host_philox(uint64_t seed, uint64_t chain, uint32_t step, uint32_t block, u
 // ---------------------------------------------------------------------------------------------------
 struct icp_std_icp_s {
     icp_model model = nullptr;
-    icp_target target = nullptr;
+    icp_target target = nullptr;              // targets[0]: the primitive kind and the single-target structures
     int n_ids = 0, n_tp = 0, max_fits = 0, direction = 0;
     double step = 1.0;
     DevBuf<int> ids;
-    DevBuf<double> tp, Gs;
+    DevBuf<double> tp, Gs;                    // tp: [G][n_tp][3], the entries' point lists end to end
+    // target set (icp_std_icp_create_targets); with one target nothing below is allocated and every launch is the
+    // single-target one
+    int n_targets = 1;
+    std::vector<icp_target> targets;          // [G] (references held)
+    DevBuf<TargetRec> trec;                   // [G]
+    std::vector<int> tidx_req;                // icp_std_icp_set_target_index: the target of every fit of the next runs
+    DevBuf<int> tidx, wtidx;                  // [max_fits] target of every fit / of every work slot
+    DevBuf<double> tp_w;                      // [max_fits][n_tp][3] point lists of the target-sampling work slots
     // workspaces, sized for max_fits at the first run (graph capture cannot allocate)
     bool sized = false;
     DevBuf<double> theta, theta_w, theta0, X, cp, F, y, L, mu, b, Mp, M;
@@ -288,35 +300,52 @@ struct icp_std_icp_s {
     }
 };
 
-extern "C" int32_t icp_std_icp_create(icp_model m, icp_target t, const int32_t *model_point_ids, int32_t n_ids,
-                                      const double *target_points, int32_t n_tp, double step_length, int32_t direction,
-                                      int32_t max_fits, icp_std_icp *out) {
+extern "C" int32_t icp_std_icp_create_targets(icp_model m, int32_t n_targets, const icp_std_icp_target *targets,
+                                              const int32_t *model_point_ids, int32_t n_ids, int32_t n_tp, double step_length,
+                                              int32_t direction, int32_t max_fits, icp_std_icp *out) {
     icp_std_icp h = nullptr;
     icp_ctx _ctx = m ? m->ctx : nullptr;
     try {
-        ICP_REQUIRE(m && t && out, "null argument");
-        ICP_REQUIRE(m->ctx == t->ctx, "model and target belong to different contexts");
+        ICP_REQUIRE(m && targets && out && n_targets >= 1, "null argument");
         ICP_REQUIRE(direction == ICP_MODEL_SAMPLING || direction == ICP_TARGET_SAMPLING || direction == ICP_MODEL_AND_TARGET_SAMPLING,
                     "bad direction");
         ICP_REQUIRE(max_fits >= 1, "max_fits must be >= 1");
         ICP_REQUIRE(std::isfinite(step_length), "step_length must be finite");
         ICP_REQUIRE(n_ids >= 1 && model_point_ids, "model sampling needs at least one model point id");
-        ICP_REQUIRE(n_tp >= 1 && target_points, "target sampling needs at least one target point");
+        ICP_REQUIRE(n_tp >= 1, "target sampling needs at least one target point");
         for (int i = 0; i < n_ids; i++) ICP_REQUIRE(model_point_ids[i] >= 0 && model_point_ids[i] < m->N, "model point id out of range");
-        for (int i = 0; i < 3 * n_tp; i++) ICP_REQUIRE(std::isfinite(target_points[i]), "target points must be finite");
+        for (int g = 0; g < n_targets; g++) {
+            const std::string e = "targets[" + std::to_string(g) + "]";
+            ICP_REQUIRE(targets[g].target, e + ".target is null");
+            ICP_REQUIRE(targets[g].target_points, e + ".target_points is null");
+            ICP_REQUIRE(targets[g].target->ctx == m->ctx, e + ".target: model and target belong to different contexts");
+            for (int i = 0; i < 3 * n_tp; i++)
+                ICP_REQUIRE(std::isfinite(targets[g].target_points[i]), e + ".target_points must be finite");
+        }
         CtxLock lock(_ctx);
         cudaStream_t s = _ctx->stream;
         h = new icp_std_icp_s();
-        h->model = m; h->target = t; h->n_ids = n_ids; h->n_tp = n_tp; h->max_fits = max_fits; h->direction = direction;
-        h->step = step_length;
+        h->model = m; h->target = targets[0].target; h->n_ids = n_ids; h->n_tp = n_tp; h->max_fits = max_fits;
+        h->direction = direction; h->step = step_length; h->n_targets = n_targets;
+        for (int g = 0; g < n_targets; g++) h->targets.push_back(targets[g].target);
         h->ids.upload(model_point_ids, n_ids, s);
-        h->tp.upload(target_points, (size_t)3 * n_tp, s);
+        h->tp.alloc((size_t)n_targets * n_tp * 3);
+        for (int g = 0; g < n_targets; g++)
+            ICP_CUDA(cudaMemcpyAsync(h->tp.p + (size_t)g * n_tp * 3, targets[g].target_points, sizeof(double) * n_tp * 3,
+                                     cudaMemcpyHostToDevice, s));
+        if (n_targets > 1) {
+            upload_target_table(h->targets, h->trec, s);
+            // fixed addresses: the iteration graphs read them
+            h->tidx.alloc(max_fits); h->wtidx.alloc(max_fits);
+            h->tp_w.alloc((size_t)max_fits * n_tp * 3);
+        }
         h->Gs.alloc((size_t)m->Kp * m->Kp);
         launch_gram_rows(m->dev(), n_ids, h->ids.p, h->Gs.p, s);
         ICP_CUDA(cudaEventCreate(&h->ev0));
         ICP_CUDA(cudaEventCreate(&h->ev1));
         ICP_CUDA(cudaStreamSynchronize(s));
-        m->refs++; t->refs++;
+        m->refs++;
+        for (icp_target t : h->targets) t->refs++;
         *out = h;
         return ICP_OK;
     } catch (...) {
@@ -326,13 +355,37 @@ extern "C" int32_t icp_std_icp_create(icp_model m, icp_target t, const int32_t *
     }
 }
 
+extern "C" int32_t icp_std_icp_create(icp_model m, icp_target t, const int32_t *model_point_ids, int32_t n_ids,
+                                      const double *target_points, int32_t n_tp, double step_length, int32_t direction,
+                                      int32_t max_fits, icp_std_icp *out) {
+    const icp_std_icp_target one{t, target_points};
+    return icp_std_icp_create_targets(m, 1, &one, model_point_ids, n_ids, n_tp, step_length, direction, max_fits, out);
+}
+
+extern "C" int32_t icp_std_icp_set_target_index(icp_std_icp h, int32_t C, const int32_t *target_index) {
+    icp_ctx _ctx = h ? h->model->ctx : nullptr;
+    try {
+        ICP_REQUIRE(_ctx != nullptr && target_index != nullptr, "null argument");
+        CtxLock lock(_ctx);
+        ICP_REQUIRE(C >= 1 && C <= h->max_fits, "C must be in [1, max_fits]");
+        for (int i = 0; i < C; i++)
+            ICP_REQUIRE(target_index[i] >= 0 && target_index[i] < h->n_targets,
+                        "target_index[" + std::to_string(i) + "] = " + std::to_string(target_index[i]) + " is outside [0, n_targets)");
+        h->tidx_req.assign(target_index, target_index + C);
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
+    }
+}
+
 extern "C" int32_t icp_std_icp_destroy(icp_std_icp h) {
     if (!h) return ICP_OK;
     icp_ctx _ctx = h->model->ctx;
     try {
         CtxLock lock(_ctx);
         ICP_CUDA(cudaStreamSynchronize(_ctx->stream));
-        h->model->refs--; h->target->refs--;
+        h->model->refs--;
+        for (icp_target t : h->targets) t->refs--;
         delete h;
         return ICP_OK;
     } catch (...) {
@@ -365,8 +418,9 @@ void enqueue_iteration(icp_std_icp h, int C, int nm, int si, double sigma2, cuda
     icp_target t = h->target;
     const ModelDev md = m->dev();
     const int K = m->K, Kp = m->Kp, Lt = K + kTheta0, nt = C - nm, ni = h->n_ids, ntp = h->n_tp;
+    const bool multi = h->n_targets > 1;
     k_si_gather<<<C, 128, 0, s>>>(C, Lt, nm, ni, ntp, h->iter.p, h->io.p, h->theta.p, h->status.p, h->theta_w.p, h->seed_m.p,
-                                  h->seed_t.p, h->wseed_m.p, h->wseed_t.p);
+                                  h->seed_t.p, h->wseed_m.p, h->wseed_t.p, multi ? h->tidx.p : nullptr, h->wtidx.p);
     ICP_CUDA(cudaGetLastError());
     launch_reconstruct(md, C, h->theta_w.p, h->X.p, s);
     if (nm > 0) {
@@ -374,6 +428,7 @@ void enqueue_iteration(icp_std_icp h, int C, int nm, int si, double sigma2, cuda
         NearestArgs a;
         a.bvh = &t->tri_bvh; a.prim_data = t->tri_data.p; a.wide = t->wide(); a.sm_count = t->ctx->sm_count; a.C = nm; a.nq = ni;
         a.Xq = h->X.p; a.q_ids = h->ids.p; a.Nq = m->N; a.out_cp = h->cp.p; a.seed_slot = h->wseed_m.p;
+        if (multi) { a.mt_rec = h->trec.p; a.mt_idx = h->wtidx.p; }   // slot p walks the BVH of its own target
         launch_nearest(a, s);
         const int NB = Kp / 8, grid = (nm + kSiFits - 1) / kSiFits;
         const double *T = h->T.p + (size_t)si * Kp * Kp;
@@ -387,13 +442,19 @@ void enqueue_iteration(icp_std_icp h, int C, int nm, int si, double sigma2, cuda
         // :118 currentMesh.pointSet.findClosestPoint(targetPoint), then model.posterior(corr, sigma2) (:81) with isotropic noise
         double *th_t = h->theta_w.p + (size_t)nm * Lt;
         const double *X_t = h->X.p + (size_t)nm * m->N * 3;
-        nearest_model_vertex(m, nt, X_t, ntp, h->tp.p, 0, h->wseed_t.p, h->prim.p, s);
+        // on a target set every slot reads its own target's point list, gathered into [nt][n_tp][3]
+        const double *tp = h->tp.p;
+        if (multi) {
+            launch_gather_target_rows(nt, 3 * ntp, h->wtidx.p + nm, h->tp.p, h->tp_w.p, s);
+            tp = h->tp_w.p;
+        }
+        nearest_model_vertex(m, nt, X_t, ntp, tp, multi ? 1 : 0, h->wseed_t.p, h->prim.p, s);
         ObsArgs oa{};
         oa.m = md; oa.C = nt; oa.theta = th_t; oa.X = X_t;
         oa.prm.step_length = h->step; oa.prm.tangential_noise = 1; oa.prm.noise_along_normal = 1;
         oa.prm.direction = ICP_TARGET_SAMPLING; oa.prm.boundary_aware = 0; oa.prm.factor = ICP_FACTOR_CHOLESKY;
         oa.prm.rank_update = ICP_RANK_UPDATE_FP64;
-        oa.tp = h->tp.p; oa.near_vid = h->prim.p; oa.iso = 1; oa.iso_sigma2 = sigma2; oa.world_frame = 1;
+        oa.tp = tp; oa.tp_per_chain = multi ? 1 : 0; oa.near_vid = h->prim.p; oa.iso = 1; oa.iso_sigma2 = sigma2; oa.world_frame = 1;
         ObsDev od{ntp, h->vid.p, h->F.p, h->y.p, h->nobs.p};
         od.nrows = h->nobs.p + nt;
         launch_observations(oa, od, s);
@@ -453,6 +514,8 @@ void std_icp_run(icp_std_icp h, int C, const double *theta0_dev, int n_sigma, co
     ICP_CUDA(cudaMemcpyAsync(h->perm.p, perm.data(), sizeof(int) * perm.size(), cudaMemcpyHostToDevice, s));
     RunIo rio{h->perm.p, log_alpha, log_direction};
     ICP_CUDA(cudaMemcpyAsync(h->io.p, &rio, sizeof rio, cudaMemcpyHostToDevice, s));
+    if (h->n_targets > 1)
+        ICP_CUDA(cudaMemcpyAsync(h->tidx.p, h->tidx_req.data(), sizeof(int) * (size_t)C, cudaMemcpyHostToDevice, s));
     ICP_CUDA(cudaMemsetAsync(h->seed_m.p, 0xFF, sizeof(int) * (size_t)C * h->n_ids, s));   // no traversal seed yet
     ICP_CUDA(cudaMemsetAsync(h->seed_t.p, 0xFF, sizeof(int) * (size_t)C * h->n_tp, s));
     k_si_init<<<C, 128, 0, s>>>(C, Lt, theta0_dev, h->theta.p, h->status.p, h->done.p, h->iter.p);
@@ -473,7 +536,8 @@ void std_icp_run(icp_std_icp h, int C, const double *theta0_dev, int n_sigma, co
     // iterations: one graph per (C, split, sigma), captured at its first use and replayed
     std::string base;
     {
-        const void *bufs[] = {m->vert_bvh.nodes.p, m->vert_bvh.nodebox.p, m->vert_bvh.counters.p, h->T.p, h->pstatus.p};
+        const void *bufs[] = {m->vert_bvh.nodes.p, m->vert_bvh.nodebox.p, m->vert_bvh.counters.p, h->T.p, h->pstatus.p, h->trec.p,
+                              h->wtidx.p};
         base.append((const char *)bufs, sizeof bufs);
         base.append((const char *)&C, sizeof C);
     }
@@ -528,6 +592,8 @@ void check_run_args(icp_std_icp h, int C, const void *theta0, int n_sigma, const
     for (int i = 0; i < n_sigma; i++) ICP_REQUIRE(std::isfinite(sigma2[i]) && sigma2[i] > 0, "every sigma2 must be finite and > 0");
     ICP_REQUIRE(num_iterations >= 0, "num_iterations must be >= 0");
     ICP_REQUIRE((long long)n_sigma * (num_iterations + 1) <= (1LL << 30), "too many iterations");
+    ICP_REQUIRE(h->n_targets == 1 || (int)h->tidx_req.size() == C,
+                "a handle with several targets needs icp_std_icp_set_target_index with C = " + std::to_string(C) + " entries before a run");
 }
 
 }  // namespace

@@ -192,6 +192,24 @@ typedef struct icp_std_icp_s *icp_std_icp;
 int32_t icp_std_icp_create(icp_model m, icp_target t, const int32_t *model_point_ids, int32_t n_ids, const double *target_points,
                            int32_t n_tp, double step_length, int32_t direction, int32_t max_fits, icp_std_icp *out);
 int32_t icp_std_icp_destroy(icp_std_icp h);
+/* Several targets in one handle: every fit names its own target, and the fits of all targets run in the same batched
+ * launches (icp_std_icp_create is the one-target case). Entry g holds a target and its n_tp target points
+ * (randomPointsOnTarget, :51-53); the model, the model point ids, n_tp, the step and the direction are shared by
+ * construction. Target meshes may have different vertex and triangle counts. Every fit equals, bit for bit, the run of a
+ * single-target handle on its own target with the same seed and global fit id. Refused with ICP_ERR_INVALID_ARGUMENT and a
+ * message naming the entry: a null target or point list, a target of another context, non-finite points. The handle holds
+ * a reference on every target. */
+typedef struct {
+    icp_target target;
+    const double *target_points;   /* n_tp x 3, points on this target */
+} icp_std_icp_target;
+int32_t icp_std_icp_create_targets(icp_model m, int32_t n_targets, const icp_std_icp_target *targets,
+                                   const int32_t *model_point_ids, int32_t n_ids, int32_t n_tp, double step_length,
+                                   int32_t direction, int32_t max_fits, icp_std_icp *out);
+/* target_index [C] (host), entries in [0, n_targets): fit c runs on targets[target_index[c]] in every later run with this C.
+ * Required before a run of a handle with n_targets > 1, and again whenever a run has a different C (refused otherwise).
+ * Sharded runs pass the indices of their own fits, with their fit_id_offset as usual. */
+int32_t icp_std_icp_set_target_index(icp_std_icp h, int32_t C, const int32_t *target_index);
 /* per-fit status words (icp_std_icp_io.status): where the reference catches an exception and returns the last coefficients
  * (:94-104), that fit stops: it keeps its coefficients for the rest of the run, its later log rows repeat them and
  * iterations_done stops counting. The other fits are unaffected and the run returns ICP_OK. */

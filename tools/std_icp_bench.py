@@ -8,8 +8,15 @@
 - The ICP arm of config 4 (StdIcpVsChainICPrandomInitComparisonAll.scala:148): 100 random inits x 101 iterations, Philox coin,
   GPMM-100 and GPMM-200.
 - 2368 fits of GPMM-100 in one batch: fits/s.
+- config4_icp_arm_targets: the ICP arm of config 4 over G = 1, 8, 24 and 47 targets (the perturbed femur-twin targets of
+  tools/multi_target_bench.py, each with its own 1622 target points) x 100 fits, GPMM-100 and GPMM-200, measured three ways:
+    multi   one run of a target-set handle (icp_std_icp_create_targets) with G x 100 fits
+    loop    G single-target runs of 100 fits back to back (one handle per target: the only way before target sets)
+    single  one single-target run of G x 100 fits (the rate at equal fit count on one target)
+  fits/s from device time (the loop: the sum of its runs' device times; its wall time adds the per-run synchronisations),
+  launches per iteration, and whether every multi fit equals its loop fit bit for bit.
 
-Usage: python tools/std_icp_bench.py [--out FILE] [--repeats R]
+Usage: python tools/std_icp_bench.py [--out FILE] [--repeats R] [--groups 1,8,24,47]
 """
 import argparse
 import json
@@ -58,10 +65,78 @@ def _timed(runner, th0, sig, n_it, repeats, **kw):
     return out, float(np.median(ms)), float(np.median(wall)), launches
 
 
+INITS = 100
+
+
+def targets_section(ctx, fx, models, ids, groups, repeats):
+    """config4_icp_arm_targets (see the module docstring)."""
+    base = dict(ref=fx["ref"], basis=fx["100"][0], variance=fx["100"][1])
+    K100 = len(base["variance"])
+    tgts, tps = [], []
+    for g in range(max(groups)):
+        # the perturbed targets of tools/multi_target_bench.py
+        tv = synth.model_instance(base, np.random.default_rng(100 + g).normal(0, 1.0, K100))
+        tv = tv + np.random.default_rng(7 + g).normal(0, 0.5, tv.shape)
+        tgts.append(core.Target(ctx, tv, fx["cells"]))
+        tps.append(synth.near_surface_queries(tv, fx["cells"], N, seed=1024, sd=0.0))
+    out = []
+    for k in ("100", "200"):
+        m = models[k]
+        for G in groups:
+            C = G * INITS
+            th = np.zeros((C, m.K + 10)); th[:, 0] = 1.0
+            th[:, 10:] = np.random.default_rng(4).normal(0, 1.0, (C, m.K))     # random inits
+            tidx = np.repeat(np.arange(G), INITS)
+            row = dict(K=m.K, targets=G, fits=C, iterations=ITERS)
+            multi = core.StdIcp(m, model_point_ids=ids, direction=_lib.MODEL_AND_TARGET_SAMPLING, max_fits=C,
+                                targets=list(zip(tgts[:G], tps[:G]))) if G > 1 else \
+                core.StdIcp(m, tgts[0], ids, tps[0], 1.0, _lib.MODEL_AND_TARGET_SAMPLING, max_fits=C)
+            kw = dict(seed=7, log=False, target_index=tidx) if G > 1 else dict(seed=7, log=False)
+            mo, ms, wall, launches = _timed(multi, th, (1e-15,), ITERS - 1, repeats, **kw)
+            multi.close()
+            row["multi"] = dict(device_ms=ms, fits_per_s=C / (ms * 1e-3), launches_per_iteration=launches / ITERS, wall_ms=wall * 1e3)
+            # the loop: one handle per target, each warmed up, then the G runs back to back
+            hs = [core.StdIcp(m, tgts[g], ids, tps[g], 1.0, _lib.MODEL_AND_TARGET_SAMPLING, max_fits=INITS) for g in range(G)]
+            for g, h in enumerate(hs):
+                h.run(th[g * INITS:(g + 1) * INITS], (1e-15,), ITERS - 1, seed=7, fit_id_offset=g * INITS, log=False)
+            best = None
+            for _ in range(repeats):
+                t = time.perf_counter()
+                lo, lms, ll = [], 0.0, 0
+                for g, h in enumerate(hs):
+                    lo.append(h.run(th[g * INITS:(g + 1) * INITS], (1e-15,), ITERS - 1, seed=7, fit_id_offset=g * INITS, log=False))
+                    d, n = h.last_run_stats()
+                    lms += d; ll += n
+                lwall = time.perf_counter() - t
+                if best is None or lms < best[0]:
+                    best = (lms, lwall, ll)
+            for h in hs:
+                h.close()
+            lms, lwall, ll = best
+            row["loop"] = dict(device_ms=lms, fits_per_s=C / (lms * 1e-3), launches_per_iteration=ll / ITERS, wall_ms=lwall * 1e3,
+                               wall_fits_per_s=C / lwall)
+            row["multi_equals_loop"] = bool(np.array_equal(mo["alpha_final"], np.concatenate([o["alpha_final"] for o in lo])) and
+                                            np.array_equal(mo["status"], np.concatenate([o["status"] for o in lo])))
+            one = core.StdIcp(m, tgts[0], ids, tps[0], 1.0, _lib.MODEL_AND_TARGET_SAMPLING, max_fits=C)
+            _, sms, swall, sl = _timed(one, th, (1e-15,), ITERS - 1, repeats, seed=7, log=False)
+            one.close()
+            row["single"] = dict(device_ms=sms, fits_per_s=C / (sms * 1e-3), launches_per_iteration=sl / ITERS, wall_ms=swall * 1e3)
+            row["multi_vs_loop_device"] = lms / ms
+            row["multi_vs_loop_wall"] = lwall / wall
+            row["multi_vs_single_device"] = sms / ms
+            row["failed_fits"] = int((mo["status"] != 0).sum())
+            print(json.dumps(row), file=sys.stderr, flush=True)
+            out.append(row)
+    for t in tgts:
+        t.close()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None)
     ap.add_argument("--repeats", type=int, default=5)
+    ap.add_argument("--groups", default="1,8,24,47")
     a = ap.parse_args()
     fx = _load()
     ctx = core.Context(0)
@@ -120,6 +195,7 @@ def main():
 
     res["config4_icp_arm"] = [batch("100", 100), batch("200", 100)]
     res["fits_2368"] = batch("100", 2368)
+    res["config4_icp_arm_targets"] = targets_section(ctx, fx, models, ids, [int(g) for g in a.groups.split(",")], a.repeats)
     for m in models.values():
         m.close()
     tgt.close(); ctx.close()
