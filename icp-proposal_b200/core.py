@@ -63,6 +63,16 @@ class Context:
                                         float(step), int(bool(ymean)), dptr(L), dptr(mean), None if q is None else dptr(q), iptr(st)), self.h)
         return L, mean, q, st
 
+    def svd_factor(self, L, variance, tol=0.0):
+        """The SVD factor W of C posteriors from their Cholesky factors L (C x K x K) on the device path of ICP_FACTOR_SVD
+        (icp_debug_svd_factor): W and the Jacobi sweeps that rotated per posterior (40: the cap ended the loop). tol <= 0: the
+        library's stopping threshold."""
+        L = f64(L); c, K = L.shape[0], L.shape[1]
+        var = f64(variance).reshape(K)
+        W = np.empty((c, K, K)); sw = np.empty(c, np.int32)
+        check(self.lib.icp_debug_svd_factor(self.h, c, K, dptr(L), dptr(var), float(tol), dptr(W), iptr(sw)), self.h)
+        return W, sw
+
     def philox(self, seed, chain, step, block):
         out = (C.c_uint32 * 4)()
         check(self.lib.icp_debug_philox(self.h, seed, chain, step, block, out), self.h)

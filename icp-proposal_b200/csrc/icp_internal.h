@@ -340,9 +340,10 @@ void launch_propose(const ModelDev &m, int C, double step, const double *d_theta
                     const double *d_L, const double *d_mu, const int *d_slot, double *d_theta_out, cudaStream_t s,
                     const double *d_W = nullptr);
 // the reference's covariance factor W = D^-1 Ubar diag(sqrt(lambda')) of C posteriors from their Cholesky factors
-// (svdfactor.cu); L / W addressed through d_slot (nullable); scratch is grown when the matrices do not fit shared memory
+// (svdfactor.cu); L / W addressed through d_slot (nullable); scratch is grown when the matrices do not fit shared memory.
+// tol <= 0: the library's stopping threshold of the Jacobi sweeps; d_sweeps (nullable): sweeps that rotated, per posterior
 void launch_svd_factor(int C, int K, int Kp, const double *d_L, const double *d_sqrt_var, const int *d_slot, double *d_W,
-                       DevBuf<double> &scratch, cudaStream_t s);
+                       DevBuf<double> &scratch, cudaStream_t s, double tol = 0.0, int *d_sweeps = nullptr);
 // -1/2 (K ln 2pi + |L^T (alpha_c - mu)|^2), -inf unless only alpha changed
 void launch_log_transition(int C, int K, int Kp, double step, const double *d_from, const double *d_to,
                            const double *d_L, const double *d_mu, const int *d_slot, double *d_out, cudaStream_t s);

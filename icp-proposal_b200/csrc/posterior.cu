@@ -686,7 +686,7 @@ __global__ void __launch_bounds__(kChThreads) k_cholesky_solve(int K, int Kp, co
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
     for (int j = 0; j < Kp; j++) {
         double ajj = A[j * ld + j];
-        if (!(ajj > 0.0)) { if (threadIdx.x == 0) bad = 1; }
+        if (!(ajj > 0.0 && ajj < INFINITY)) { if (threadIdx.x == 0) bad = 1; }   // an infinite pivot only yields NaN
         double inv = 1.0 / sqrt(ajj);
         __syncthreads();  // everyone has read the pivot before it is overwritten
         for (int i = j + threadIdx.x; i < R; i += kChThreads) A[i * ld + j] *= inv;  // i == j: a/sqrt(a) = sqrt(a)
@@ -787,11 +787,13 @@ __device__ void chol_factor_solve_store(double *A, int Kp, int *bad, double *__r
 #pragma unroll
         for (int j = 0; j < 8; j++) {
             double s = l[j][j];
-            if (!(s > 0.0)) mybad = true;
             // 1/sqrt(s) by rsqrt + one Newton step (full double accuracy), sqrt(s) = s * inv: one short dependent
             // chain instead of a software sqrt followed by a software divide
             double r = rsqrt(s);
             r = fma(r * 0.5, fma(-s * r, r, 1.0), r);
+            // r > 0 exactly for finite s > 0: s <= 0 and NaN give NaN, and so does s = +Inf (rsqrt 0, the Newton step
+            // 0 * Inf), which a test of s > 0 lets through - with no later pivot to catch it when it is the last one
+            if (!(r > 0.0)) mybad = true;
             inv[j] = r;
             double d = s * r;
             d = fma(fma(-d, d, s), 0.5 * r, d);
@@ -1088,10 +1090,10 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
 #pragma unroll
             for (int j = 0; j < 8; j++) {
                 double s = l[j][j];
-                if (!(s > 0.0)) mybad = true;
                 // 1/sqrt(s) by rsqrt + one Newton step (full double accuracy), sqrt(s) = s * inv
                 double r = rsqrt(s);
                 r = fma(r * 0.5, fma(-s * r, r, 1.0), r);
+                if (!(r > 0.0)) mybad = true;   // finite s > 0 only: +Inf gives NaN here (see chol_factor_solve_store)
                 inv[j] = r;
                 double d = s * r;
                 d = fma(fma(-d, d, s), 0.5 * r, d);
@@ -1947,6 +1949,9 @@ extern "C" int32_t icp_debug_factor(icp_ctx ctx, int32_t C, int32_t K, const dou
     icp_ctx _ctx = ctx;
     try {
         ICP_REQUIRE(ctx && C > 0 && K > 0 && M && b && L && mean && status, "null or empty argument");
+        // the ranks of icp_model_create: 225..232 would still fit the packed factorisation (Kp = 232), but no posterior
+        // pipeline runs there, so a result at those ranks would describe nothing the library computes
+        ICP_REQUIRE(K <= 224, "rank K must be in [1, 224]");
         ICP_REQUIRE(!q || (theta_post && theta_other), "q needs theta_post and theta_other");
         CtxLock lock(ctx);
         cudaStream_t s = ctx->stream;

@@ -14,6 +14,9 @@
 // Order: lambda' descending (ties: lower column index first). Sign: the entry of largest magnitude of every vector is
 // positive (lowest index on ties) - a documented convention of this library (the test checkers adopt it); what LAPACK's
 // dgesdd would return inside Breeze is not knowable without a JVM.
+#include <cmath>
+#include <vector>
+
 #include "icp_device.cuh"
 #include "icp_internal.h"
 
@@ -21,6 +24,9 @@ namespace icp {
 
 constexpr int kSvdThreads = 256;
 constexpr int kSvdMaxSweeps = 40;
+// a pair rotates while |a.b| > kSvdTol |a| |b|; the femur-like posteriors of rank 31 to 224 stop after 8 or 9 sweeps
+// (tests/test_gpu_posterior_ranks.py::test_svd_factor asserts that the cap is not reached)
+constexpr double kSvdTol = 1e-15;
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
@@ -31,7 +37,8 @@ __device__ __forceinline__ double warp_sum(double v) {
 __global__ void __launch_bounds__(kSvdThreads) k_svd_factor(int K, int Kp, const double *__restrict__ L,
                                                             const double *__restrict__ sqrt_var,
                                                             const int *__restrict__ slot, double *__restrict__ W,
-                                                            double *__restrict__ scratch, int mats_in_smem) {
+                                                            double *__restrict__ scratch, int mats_in_smem, double tol,
+                                                            int *__restrict__ sweeps) {
     extern __shared__ __align__(16) double sm[];
     __shared__ double s_n2[256];     // squared column norms (K <= 224)
     __shared__ int s_rank[256];
@@ -53,8 +60,8 @@ __global__ void __launch_bounds__(kSvdThreads) k_svd_factor(int K, int Kp, const
     }
     __syncthreads();
     const int n = (K + 1) & ~1;       // tournament size (even); an index >= K is a bye
-    const double tol = 1e-15;
-    for (int sweep = 0; sweep < kSvdMaxSweeps; sweep++) {
+    int sweep = 0;                    // sweeps that rotated; kSvdMaxSweeps: the cap ended the loop
+    for (; sweep < kSvdMaxSweeps; sweep++) {
         int rotated = 0;
         for (int r = 0; r < n - 1; r++) {
             for (int k = warp; k < n / 2; k += nw) {
@@ -88,6 +95,7 @@ __global__ void __launch_bounds__(kSvdThreads) k_svd_factor(int K, int Kp, const
         }
         if (!__syncthreads_or(rotated)) break;
     }
+    if (sweeps && tid == 0) sweeps[c] = sweep;
     // column norms, sign of every vector
     for (int j = warp; j < K; j += nw) {
         const double *g = G + (size_t)j * ld, *u = J + (size_t)j * ld;
@@ -126,7 +134,7 @@ __global__ void __launch_bounds__(kSvdThreads) k_svd_factor(int K, int Kp, const
 }
 
 void launch_svd_factor(int C, int K, int Kp, const double *d_L, const double *d_sqrt_var, const int *d_slot, double *d_W,
-                       DevBuf<double> &scratch, cudaStream_t s) {
+                       DevBuf<double> &scratch, cudaStream_t s, double tol, int *d_sweeps) {
     if (C <= 0) return;
     ProfScope _ps(ST_OTHER, s);
     ICP_REQUIRE(K <= 256, "rank too large for the SVD factor kernel");
@@ -137,8 +145,46 @@ void launch_svd_factor(int C, int K, int Kp, const double *d_L, const double *d_
     if (mats < 2) scratch.ensure((size_t)C * 2 * KK);
     const size_t smem = sizeof(double) * KK * mats;
     ICP_CUDA(cudaFuncSetAttribute(k_svd_factor, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_svd_factor<<<C, kSvdThreads, smem, s>>>(K, Kp, d_L, d_sqrt_var, d_slot, d_W, scratch.p, mats);
+    k_svd_factor<<<C, kSvdThreads, smem, s>>>(K, Kp, d_L, d_sqrt_var, d_slot, d_W, scratch.p, mats, tol > 0.0 ? tol : kSvdTol,
+                                              d_sweeps);
     ICP_CUDA(cudaGetLastError());
 }
 
 }  // namespace icp
+
+// The SVD factor of C posteriors from their Cholesky factors (host, C x K x K, lower triangle read) and the model variances:
+// W (C x K x K) and the Jacobi sweeps that rotated per posterior (kSvdMaxSweeps: the cap ended the loop). tol <= 0: the
+// pipeline's threshold.
+extern "C" int32_t icp_debug_svd_factor(icp_ctx ctx, int32_t C, int32_t K, const double *L, const double *variance, double tol,
+                                        double *W, int32_t *sweeps) {
+    using namespace icp;
+    icp_ctx _ctx = ctx;
+    try {
+        ICP_REQUIRE(ctx && C > 0 && K >= 1 && K <= 224 && L && variance && W && sweeps, "null or empty argument");
+        for (int j = 0; j < K; j++) ICP_REQUIRE(variance[j] > 0.0 && std::isfinite(variance[j]), "variances must be finite and > 0");
+        CtxLock lock(ctx);
+        cudaStream_t s = ctx->stream;
+        const int Kp = (K + 7) / 8 * 8;
+        std::vector<double> hL((size_t)C * Kp * Kp, 0.0), hs(Kp, 1.0), hW((size_t)C * Kp * Kp);
+        for (int c = 0; c < C; c++)
+            for (int i = 0; i < K; i++)
+                for (int j = 0; j <= i; j++) hL[((size_t)c * Kp + i) * Kp + j] = L[((size_t)c * K + i) * K + j];
+        for (int j = 0; j < K; j++) hs[j] = std::sqrt(variance[j]);
+        DevBuf<double> dL, ds, dW, scratch;
+        DevBuf<int> dsw;
+        dL.upload(hL.data(), hL.size(), s);
+        ds.upload(hs.data(), hs.size(), s);
+        dW.alloc(hW.size());
+        dsw.alloc(C);
+        launch_svd_factor(C, K, Kp, dL.p, ds.p, nullptr, dW.p, scratch, s, tol, dsw.p);
+        ICP_CUDA(cudaMemcpyAsync(hW.data(), dW.p, sizeof(double) * hW.size(), cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaMemcpyAsync(sweeps, dsw.p, sizeof(int) * C, cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaStreamSynchronize(s));
+        for (int c = 0; c < C; c++)
+            for (int i = 0; i < K; i++)
+                for (int j = 0; j < K; j++) W[((size_t)c * K + i) * K + j] = hW[((size_t)c * Kp + i) * Kp + j];
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
+    }
+}

@@ -517,7 +517,10 @@ __global__ void __launch_bounds__(kRuThreads, 1) k_rank_update_i8(ModelDev m, Ob
                 // steps of this chain the team still owes, then - while the tensor core finishes the chain - its first step
                 // of the next chain (one call site of the step body: two would double its register footprint)
                 int st = ((h - (int)S) & 1) + 2 * pre_done;
-                const bool had_pre = pre_done != 0;
+                // the team's first step of every chain is reduced and parked in shared memory on its own, whether it ran early
+                // (the previous chain's tail) or runs here: b then sums in the same order in every chain, so a chain's b does not
+                // depend on whether it is the first chain of its CTA
+                bool had_pre = pre_done != 0;
                 pre_done = 0;
                 bool published = false;
                 for (;;) {
@@ -547,6 +550,16 @@ __global__ void __launch_bounds__(kRuThreads, 1) k_rank_update_i8(ModelDev m, Ob
                     } else break;
                     convert_step(Sg);
                     if (published) break;
+                    if (!had_pre) {
+                        reduce_b();
+                        if (live && (lane & 23) == 0) {
+#pragma unroll
+                            for (int k = 0; k < 8; k++) sb[h * Kp + 8 * g + k] = bacc[k];
+                        }
+#pragma unroll
+                        for (int k = 0; k < 8; k++) bacc[k] = 0.0;
+                        had_pre = true;
+                    }
                 }
                 if (pre_done) {
                     // the early step's share of the next chain's b goes to that chain's buffer now

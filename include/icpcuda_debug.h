@@ -48,6 +48,13 @@ int32_t icp_debug_i8_gram(icp_ctx ctx, int32_t rows, const int8_t *A, int32_t *D
 int32_t icp_debug_factor(icp_ctx ctx, int32_t C, int32_t K, const double *M, const double *b, const double *theta_post,
                          const double *theta_other, double step, int32_t ymean, double *L, double *mean, double *q, int32_t *status);
 
+/* The reference's covariance factor W = D^-1 Ubar diag(sqrt(lambda')) (ICP_FACTOR_SVD) of C posteriors from their Cholesky factors
+ * L (C x K x K, lower triangle read) and the model variances (K), on the device path the proposal takes: W (C x K x K) and per
+ * posterior the one-sided Jacobi sweeps that rotated (40, the cap, means the loop did not converge). tol <= 0: the library's
+ * stopping threshold; > 0: that threshold instead. */
+int32_t icp_debug_svd_factor(icp_ctx ctx, int32_t C, int32_t K, const double *L, const double *variance, double tol, double *W,
+                             int32_t *sweeps);
+
 #ifdef __cplusplus
 }
 #endif
