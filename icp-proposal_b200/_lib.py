@@ -164,6 +164,7 @@ _SIGS = {
     "icp_debug_i8_gram": [_h, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, _dp],
     "icp_debug_factor": [_h, C.c_int32, C.c_int32, _dp, _dp, _dp, _dp, C.c_double, C.c_int32, _dp, _dp, _dp, _ip],
     "icp_debug_svd_factor": [_h, C.c_int32, C.c_int32, _dp, _dp, C.c_double, _dp, _ip],
+    "icp_debug_chain_schedule": [_h, C.c_int32, _ip, _lp],
 }
 EXPORTED_SYMBOLS = sorted(list(_SIGS) + ["icp_stage_name"])
 

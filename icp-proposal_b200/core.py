@@ -706,6 +706,17 @@ class Chain:
         check(self.lib.icp_chain_last_run_rounds(self.h, C.byref(n)))
         return n.value
 
+    def schedule(self, mode=None):
+        """icp_debug_chain_schedule: mode "eager" makes later runs from theta0 factor both posteriors of every proposal, "lazy"
+        factor them lazily wherever that applies, "auto" lets the runner choose; None leaves the setting. Returns (lazy,
+        counters) of the resident run: whether it factors lazily, and [posteriors factored when picked, fallback chain-steps,
+        certified chain-steps] of the last call."""
+        lazy = C.c_int32(0)
+        cnt = (C.c_int64 * 3)()
+        code = -1 if mode is None else {"auto": 0, "eager": 1, "lazy": 2}[mode]
+        check(self.lib.icp_debug_chain_schedule(self.h, code, C.byref(lazy), cnt), self.ctx.h)
+        return bool(lazy.value), [int(v) for v in cnt]
+
     def set_statistics(self, burn_in, take_every_n=1, end=0, normals=True):
         """icp_chain_set_statistics: accumulate the posterior variability maps of the records burn_in, burn_in + take_every_n, ...
         below `end` (<= 0: no limit) inside the run, from the next run from theta0 on. burn_in=None switches them off."""

@@ -761,25 +761,19 @@ void nearest_model_vertex(icp_model m, int C, const double *d_X, int64_t nq, con
     launch_nearest(a, s);
 }
 
-void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, double *d_L,
-                        double *d_mu, const int *d_out_slot, cudaStream_t s, const SharedCp *shared, double *d_W,
-                        const QuadArgs *qa, bool ymean, const TargetSet *ts) {
-    if (C <= 0) return;
+// the observation half of posterior_pipeline: closest points + observations of C chains. store (nullable): write them
+// there (ObsDev::row / nonfinite) instead of into the work buffers; returns the list the factorisation reads.
+ObsDev posterior_observe(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, cudaStream_t s,
+                         const SharedCp *shared, const TargetSet *ts, const ObsDev *store) {
     icp_model m = p->model;
     icp_target t = p->target;
     const bool has_boundary = ts ? ts->has_boundary : t->has_boundary;
-    const int Kp = m->Kp;
     ModelDev md = m->dev();
-    if (!d_X) {
-        w.X.ensure((size_t)C * m->N * 3);
-        launch_reconstruct(md, C, d_theta, w.X.p, s);
-        d_X = w.X.p;
-    }
     const bool tsamp = p->prm.direction == ICP_TARGET_SAMPLING;
     int n = tsamp ? p->n_tp : p->n_ids;
     size_t tot = (size_t)C * std::max(n, 1);
-    w.vid.ensure(tot); w.F.ensure(9 * tot); w.y.ensure(3 * tot); w.nobs.ensure(2 * (size_t)C);
-    w.M.ensure((size_t)C * Kp * Kp); w.b.ensure((size_t)C * Kp); w.status.ensure(C);
+    if (!store) { w.vid.ensure(tot); w.F.ensure(9 * tot); w.y.ensure(3 * tot); }
+    w.nobs.ensure(2 * (size_t)C);
     ObsArgs oa{};
     oa.m = md; oa.prm = p->prm; oa.C = C; oa.theta = d_theta; oa.X = d_X;
     if (tsamp) {
@@ -821,7 +815,33 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
     }
     ObsDev od{n, w.vid.p, w.F.p, w.y.p, w.nobs.p};
     od.nrows = w.nobs.p + C;
+    if (store) {
+        od.vid = store->vid; od.F = store->F; od.y = store->y; od.nrows = store->nrows;
+        od.row = store->row; od.nonfinite = store->nonfinite;
+    }
     launch_observations(oa, od, s);
+    od.nonfinite = nullptr;
+    return od;
+}
+
+// grouped observations (target sampling on at least half the vertices) scale their rows by sqrt(multiplicity)
+static bool obs_grouped(icp_proposal p) {
+    const int n = p->prm.direction == ICP_TARGET_SAMPLING ? p->n_tp : p->n_ids;
+    return p->prm.direction == ICP_TARGET_SAMPLING && 2 * (long long)n >= p->model->N;
+}
+
+bool posterior_listable(icp_proposal p) {
+    return p->prm.factor == ICP_FACTOR_CHOLESKY && !obs_grouped(p) && posterior_packed_path(p->model->Kp);
+}
+
+// the factorisation half: rank update + Cholesky of the observations od (od.list / count: only the listed entries)
+void posterior_factor(icp_proposal p, int C, const ObsDev &od, PosteriorWork &w, double *d_L, double *d_mu, const int *d_out_slot,
+                      int *d_status, cudaStream_t s, double *d_W, const QuadArgs *qa, bool ymean, bool has_boundary) {
+    icp_model m = p->model;
+    const int Kp = m->Kp;
+    ModelDev md = m->dev();
+    const bool tsamp = p->prm.direction == ICP_TARGET_SAMPLING;
+    w.M.ensure((size_t)C * Kp * Kp); w.b.ensure((size_t)C * Kp);
     // every observation is kept (no boundary filtering possible) -> the Gram part of M is the proposal's constant
     const bool all_kept = !tsamp && !(p->prm.boundary_aware && has_boundary);
     GramFast gf{p->Gs.p, 1.0 / (p->prm.tangential_noise * p->prm.tangential_noise),
@@ -835,7 +855,7 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
     // scaled by sqrt(multiplicity), outside the column bound).
     static const std::string ru_env = getenv("ICPCUDA_RANK_UPDATE") ? getenv("ICPCUDA_RANK_UPDATE") : "";
     const bool want_i8 = ru_env == "int8" || (ru_env != "fp64" && p->prm.rank_update == ICP_RANK_UPDATE_INT8);
-    const bool grouped = tsamp && 2 * (long long)n >= m->N;
+    const bool grouped = obs_grouped(p);
     I8Scale sc{0.0, 0.0, 0.0};
     if (want_i8 && !grouped) {
         // whitened rows |F_d . Qhat_v[:, j]| <= max(1 / sd_n, 1 / sd_t) resp. sqrt(kappa) (constant-Gram rows): scaled to 2^30
@@ -850,16 +870,32 @@ void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const doub
     }
     if (want_i8 && !grouped &&
         launch_rank_update_i8(md, C, od, gfp, I8Model{m->Qhat.p, m->col_norm.p, p->Qsub.p}, sc, w.Mp.p, w.b.p, m->ctx->sm_count, s)) {
-        launch_cholesky_packed(C, Kp, w.Mp.p, w.b.p, w.want_M ? w.M.p : nullptr, d_L, d_mu, d_out_slot, w.status.p, qa, ymean, s);
+        launch_cholesky_packed(C, Kp, w.Mp.p, w.b.p, w.want_M ? w.M.p : nullptr, d_L, d_mu, d_out_slot, d_status, qa, ymean, s,
+                               od.list, od.count);
         quad_done = qa != nullptr;
     } else
-    if (!launch_posterior_fused(md, C, od, gfp, w.want_M ? w.M.p : nullptr, d_L, d_mu, d_out_slot, w.status.p, w.Mp.p, w.b.p, s, qa,
+    if (!launch_posterior_fused(md, C, od, gfp, w.want_M ? w.M.p : nullptr, d_L, d_mu, d_out_slot, d_status, w.Mp.p, w.b.p, s, qa,
                                 &quad_done, ymean)) {
         launch_posterior_build(md, C, od, w.M.p, w.b.p, s, gfp);
-        launch_cholesky_solve(C, m->K, Kp, w.M.p, w.b.p, d_L, d_mu, d_out_slot, w.status.p, s, w.Mp.p, qa, &quad_done, ymean);
+        launch_cholesky_solve(C, m->K, Kp, w.M.p, w.b.p, d_L, d_mu, d_out_slot, d_status, s, w.Mp.p, qa, &quad_done, ymean);
     }
     if (qa && !quad_done) launch_quad_form(C, Kp, d_L, d_mu, d_out_slot, *qa, ymean, s);
     if (d_W) launch_svd_factor(C, m->K, Kp, d_L, m->sqrt_var.p, d_out_slot, d_W, w.svd_scratch, s);
+}
+
+void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, double *d_L,
+                        double *d_mu, const int *d_out_slot, cudaStream_t s, const SharedCp *shared, double *d_W,
+                        const QuadArgs *qa, bool ymean, const TargetSet *ts) {
+    if (C <= 0) return;
+    icp_model m = p->model;
+    if (!d_X) {
+        w.X.ensure((size_t)C * m->N * 3);
+        launch_reconstruct(m->dev(), C, d_theta, w.X.p, s);
+        d_X = w.X.p;
+    }
+    w.status.ensure(C);
+    const ObsDev od = posterior_observe(p, C, d_theta, d_X, w, s, shared, ts, nullptr);
+    posterior_factor(p, C, od, w, d_L, d_mu, d_out_slot, w.status.p, s, d_W, qa, ymean, ts ? ts->has_boundary : p->target->has_boundary);
 }
 
 }  // namespace icp

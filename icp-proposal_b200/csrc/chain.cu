@@ -72,6 +72,18 @@ __device__ __forceinline__ int stats_selected(const StatsDev &x, long long i) {
     return i >= x.burn_in && (x.end <= 0 || i < x.end) && (i - x.burn_in) % x.every == 0;
 }
 
+// Lazy factorisation (step-by-step runner, DESIGN.md section 5): the posterior of a state is factored when a proposal from that
+// state picks its component, or when the step cannot be decided without it; every pointer is null under the eager schedule.
+struct LazyDev {
+    uint8_t *valid;       // [n_icp][2 C] L and y of the posterior slot are factored
+    uint8_t *nonfin;      // [n_icp][2 C] some observation (F, y~) of the slot is not finite
+    int *cnt;             // [2 n_icp + 1] list lengths: factor on pick (per component), fallback factorisations of the current
+                          // state (per component), fallback chains
+    int *list;            // [2 n_icp + 1][C] the lists (chain indices)
+    uint8_t *cert;        // [C] this step's ICP transition terms are certified negligible (k_lazy_certify)
+    long long *tally;     // [3] of the run: posteriors factored on pick, fallback chain-steps, certified chain-steps
+};
+
 struct StateDev {
     double *theta_cur, *theta_prop;     // [C][L]
     double *values_cur, *values_prop;   // [C][3]
@@ -93,6 +105,7 @@ struct StateDev {
     // look-ahead only: the lanes' accept decisions and status words of this round, the first step the run must not take
     int *lane_ok, *lane_status, *step_end;
     StatsDev sx;
+    LazyDev lz;
 };
 
 // per-chain status bits of a run (icp_chain_io.status)
@@ -108,10 +121,11 @@ struct StatusSrc {
     int n_post;
 };
 
-__device__ __forceinline__ int fold_status(const StatusSrc &ss, int c) {
+// post = false: this step factored no posterior of the chain (a certified step of the lazy schedule)
+__device__ __forceinline__ int fold_status(const StatusSrc &ss, int c, bool post = true) {
     int st = 0;
     if (ss.eval && ss.eval[c] != 0) st |= kStEmptySet;
-    for (int i = 0; i < ss.n_post; i++)
+    for (int i = 0; i < ss.n_post && post; i++)
         if (ss.post[i] && ss.post[i][c] != 0) st |= kStNotPD;
     return st;
 }
@@ -129,7 +143,7 @@ __global__ void k_chain_status0(int C, int Lt, StateDev st, StatusSrc ss) {
     for (int j = 0; j < Lt; j++) st.theta_best[(size_t)c * Lt + j] = st.theta_cur[(size_t)c * Lt + j];
 }
 
-__global__ void k_chain_init(int C, StateDev st) {
+__global__ void k_chain_init(int C, int n_icp, StateDev st) {
     int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c == 0) *st.step = 0;
     if (c >= C) return;
@@ -138,6 +152,8 @@ __global__ void k_chain_init(int C, StateDev st) {
     st.slot_prop[c] = C + c;
     st.n_acc[c] = 0;
     st.status[c] = 0;
+    if (st.lz.valid)   // the posteriors of theta0 are factored with its evaluation
+        for (int i = 0; i < n_icp; i++) { st.lz.valid[(size_t)i * 2 * C + c] = 1; st.lz.nonfin[(size_t)i * 2 * C + c] = 0; }
 }
 
 // standard normals of chain `chain` at step `step`: Philox block 1 + k/2 -> Box-Muller pair
@@ -149,6 +165,25 @@ __device__ __forceinline__ double chain_normal(unsigned long long seed, unsigned
     double sn, cs;
     sincospi(2.0 * u2, &sn, &cs);
     return (k & 1) ? rad * sn : rad * cs;
+}
+
+// MixtureProposal.propose's pick: the first component whose cumulative weight reaches the step's uniform; *ua: the step's
+// acceptance uniform
+__device__ __forceinline__ int pick_component(const ChainParams &P, const RngDev &rng, unsigned long long chain, unsigned int step,
+                                              int cr, int Cr, double *ua) {
+    double uc;
+    if (rng.u_comp) {
+        uc = rng.u_comp[(size_t)(step - rng.step_base) * Cr + cr];
+        *ua = rng.u_acc[(size_t)(step - rng.step_base) * Cr + cr];
+    } else {
+        uint4 r = chain_philox(rng.seed, chain, step, 0u);
+        uc = u53(r.x, r.y);
+        *ua = u53(r.z, r.w);
+    }
+    int ci = P.n_comp - 1;
+    for (int i = 0; i < P.n_comp; i++)
+        if (P.comp[i].cdf >= uc) { ci = i; break; }
+    return ci;
 }
 
 // w = L^-T z, one warp, registers + shuffles; L staged in shared memory with
@@ -216,6 +251,26 @@ __device__ __forceinline__ double block_quad_packed(const double *sL, int Kp, co
     return block_sum(part, red);
 }
 
+// forward transition form |L_cur,i^T s - y_cur,i|^2 of ICP component ci of chain c, s = alpha + (alpha' - alpha) / step_i
+// (SVD-factor components: |L^T (s - mu)|^2), from sdl = alpha' - alpha in shared memory. stage: copy the factor into sL first
+// (else sL holds it). Block-wide, 256 threads (the association of the block sum depends on the block size).
+__device__ void forward_form(const ChainParams &P, const StateDev &st, int c, const CompDev &ci, bool stage, const double *th,
+                             const double *sdl, double *sL, double *sd, double *red) {
+    const int K = P.K, Kp = P.Kp, C = P.C;
+    const size_t pslot = (size_t)ci.icp_index * 2 * C + st.slot_cur[c];
+    if (stage) stage_packed_L(st.L + pslot * Kp * Kp, Kp, sL);
+    const double *mean = st.ymean + pslot * Kp;
+    const bool ym = ci.factor != ICP_FACTOR_SVD;
+    for (int k = threadIdx.x; k < Kp; k += blockDim.x) {
+        const double s = k < K ? th[kTheta0 + k] + (sdl[k] / ci.step) : 0.0;
+        sd[k] = ym ? s : k < K ? s - mean[k] : 0.0;
+    }
+    __syncthreads();
+    const double qf = block_quad_packed(sL, Kp, sd, red, ym ? mean : nullptr);
+    if (threadIdx.x == 0) st.qf[(size_t)ci.icp_index * C + c] = qf;
+    __syncthreads();
+}
+
 // MixtureProposal.propose (pick the first component whose cumulative weight reaches r) + the component's propose, then the
 // forward transition form |L_cur^T d|^2 of EVERY ICP component (MixtureProposal.logTransitionProbability sums over all of
 // them): the factors of the current state are staged here anyway, so k_chain_accept never reads a factor back.
@@ -241,18 +296,8 @@ __global__ void __launch_bounds__(256) k_chain_propose(ChainParams P, ModelDev m
     }
     unsigned long long chain = rng.chain_offset + (unsigned long long)cr;
     if (threadIdx.x == 0) {
-        double uc, ua;
-        if (rng.u_comp) {
-            uc = rng.u_comp[(size_t)(step - rng.step_base) * Cr + cr];
-            ua = rng.u_acc[(size_t)(step - rng.step_base) * Cr + cr];
-        } else {
-            uint4 r = chain_philox(rng.seed, chain, step, 0u);
-            uc = u53(r.x, r.y);
-            ua = u53(r.z, r.w);
-        }
-        int ci = P.n_comp - 1;
-        for (int i = 0; i < P.n_comp; i++)
-            if (P.comp[i].cdf >= uc) { ci = i; break; }
+        double ua;
+        const int ci = pick_component(P, rng, chain, step, cr, Cr, &ua);
         s_ci = ci;
         st.comp_sel[c] = ci;
         st.u_acc[c] = ua;
@@ -328,28 +373,17 @@ __global__ void __launch_bounds__(256) k_chain_propose(ChainParams P, ModelDev m
     // the components in index order formed the selected component's form from an overwritten factor whenever an ICP
     // component with a smaller index came before it - invisible next to a random-walk component, whose density dominates
     // the mixture's at these step sizes, and wrong in an ICP-only mixture: tools/check_forward_forms.py.)
+    // The lazy schedule forms them in k_lazy_forward, for the steps that need them.
+    if (st.lz.valid) return;
     for (int pass = 0; pass < P.n_comp + 1; pass++) {
         const int i = pass == 0 ? s_ci : pass - 1;
         if (pass == 0 && !staged) continue;
         if (pass > 0 && staged && i == s_ci) continue;
         const CompDev ci = P.comp[i];
         if (ci.kind != ICP_PROP_ICP) continue;
-        const size_t pslot = (size_t)ci.icp_index * 2 * C + st.slot_cur[c];
-        if (pass == 0) {
+        if (pass == 0)
             for (int k = threadIdx.x; k < Kp; k += blockDim.x) sL[(k * (k + 1)) / 2 + k] = sdg[k];   // the true diagonal again
-        } else {
-            stage_packed_L(st.L + pslot * Kp * Kp, Kp, sL);
-        }
-        const double *mean = st.ymean + pslot * Kp;
-        const bool ym = ci.factor != ICP_FACTOR_SVD;
-        for (int k = threadIdx.x; k < Kp; k += blockDim.x) {
-            const double s = k < K ? th[kTheta0 + k] + (sdl[k] / ci.step) : 0.0;
-            sd[k] = ym ? s : k < K ? s - mean[k] : 0.0;
-        }
-        __syncthreads();
-        const double qf = block_quad_packed(sL, Kp, sd, red, ym ? mean : nullptr);
-        if (threadIdx.x == 0) st.qf[(size_t)ci.icp_index * C + c] = qf;
-        __syncthreads();
+        forward_form(P, st, c, ci, pass > 0, th, sdl, sL, sd, red);
     }
 }
 
@@ -357,15 +391,12 @@ __device__ __forceinline__ double gauss1_logpdf(double x, double sd) {
     return -(x * x) / (2.0 * sd * sd) - log(sd * sqrt(2.0 * 3.14159265358979323846));
 }
 
-// log transition densities of every mixture component in both directions, log-sum-exp, acceptance, log append
-__global__ void __launch_bounds__(128) k_chain_accept(ChainParams P, StateDev st, LogDev lg, StatusSrc stsrc) {
-    extern __shared__ double sm[];
-    const int K = P.K, Kp = P.Kp, Lt = K + kTheta0, C = P.C;
-    double *red = sm;
-    __shared__ double s_fwd[kMaxComp], s_bwd[kMaxComp];
-    __shared__ int s_flags[3];  // [0] any of theta[0..9] differs, [1] outside rotation group, [2] outside translation group
-    int c = blockIdx.x;
-    int step = *st.step;
+// log transition densities of every mixture component of chain c in both directions into s_fwd / s_bwd; icp = false: the ICP
+// components' terms are -inf instead of their forms. Block-wide, 128 threads (the association of |alpha' - alpha|^2 depends on
+// the block size): k_chain_accept and k_lazy_certify must see the same bits.
+__device__ void transition_terms(const ChainParams &P, const StateDev &st, int c, bool icp, double *red, double *s_fwd, double *s_bwd,
+                                 int *s_flags) {
+    const int K = P.K, Lt = K + kTheta0, C = P.C;
     const double *cur = st.theta_cur + (size_t)c * Lt, *prp = st.theta_prop + (size_t)c * Lt;
     if (threadIdx.x < 3) s_flags[threadIdx.x] = 0;
     __syncthreads();
@@ -386,7 +417,7 @@ __global__ void __launch_bounds__(128) k_chain_accept(ChainParams P, StateDev st
         const CompDev cd = P.comp[i];
         double fwd, bwd;
         if (cd.kind == ICP_PROP_ICP) {
-            if (s_flags[0]) { fwd = bwd = -INFINITY; }                          // NonRigidIcpProposal.scala:72-74
+            if (s_flags[0] || !icp) { fwd = bwd = -INFINITY; }                  // NonRigidIcpProposal.scala:72-74
             else {
                 // the two quadratic forms were formed where the factors were on chip: forward by k_chain_propose (L_cur),
                 // backward by the factorisation of the proposal's posterior (L_prop)
@@ -407,6 +438,21 @@ __global__ void __launch_bounds__(128) k_chain_accept(ChainParams P, StateDev st
         if (threadIdx.x == 0) { s_fwd[i] = fwd; s_bwd[i] = bwd; }
     }
     __syncthreads();
+}
+
+// log transition densities of every mixture component in both directions, log-sum-exp, acceptance, log append
+__global__ void __launch_bounds__(128) k_chain_accept(ChainParams P, StateDev st, LogDev lg, StatusSrc stsrc) {
+    extern __shared__ double sm[];
+    const int K = P.K, Lt = K + kTheta0, C = P.C;
+    double *red = sm;
+    __shared__ double s_fwd[kMaxComp], s_bwd[kMaxComp];
+    __shared__ int s_flags[3];  // [0] any of theta[0..9] differs, [1] outside rotation group, [2] outside translation group
+    int c = blockIdx.x;
+    int step = *st.step;
+    const double *cur = st.theta_cur + (size_t)c * Lt, *prp = st.theta_prop + (size_t)c * Lt;
+    // a certified step of the lazy schedule: the ICP terms cannot change the log-sum-exps (k_lazy_certify), and none was formed
+    const bool certified = st.lz.cert && st.lz.cert[c];
+    transition_terms(P, st, c, !certified, red, s_fwd, s_bwd, s_flags);
     __shared__ int s_acc;
     if (threadIdx.x == 0) {
         // MixtureProposal.logTransitionProbability: ln sum_i w_i exp(l_i)
@@ -426,7 +472,7 @@ __global__ void __launch_bounds__(128) k_chain_accept(ChainParams P, StateDev st
         s_acc = ok;
         // the reference throws where these happen (CollectiveAverage...Evaluator.scala:51,63; Scalismo's mixture on a NaN
         // transition); here the step is rejected and the chain's sticky status word records it
-        const int stw = fold_status(stsrc, c) | (nan ? kStNanTransition : 0);
+        const int stw = fold_status(stsrc, c, !certified) | (nan ? kStNanTransition : 0);
         if (P.W > 1) { st.lane_ok[c] = ok; st.lane_status[c] = stw; }   // k_la_resolve decides which lanes happened
         else if (stw) st.status[c] |= stw;
     }
@@ -484,7 +530,119 @@ __global__ void __launch_bounds__(128) k_chain_accept(ChainParams P, StateDev st
     }
 }
 
-__global__ void k_step_increment(int *step) { *step += 1; }
+// ---- lazy factorisation (step-by-step runner) --------------------------------------------------------------------------
+// Appends chain c to list `l` when `want` (warp-aggregated: one atomic per warp and list). Every lane of the warp calls it.
+__device__ __forceinline__ void lazy_append(const LazyDev &lz, int C, int l, int c, bool want) {
+    const unsigned mask = __ballot_sync(0xffffffffu, want);
+    if (!mask) return;
+    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
+    int base = 0;
+    if (lane == leader) base = atomicAdd(&lz.cnt[l], __popc(mask));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (want) lz.list[(size_t)l * C + base + __popc(mask & ((1u << lane) - 1u))] = c;
+}
+
+// step 1: the step's component, as k_chain_propose picks it; a chain that picked ICP component i goes to list i when the
+// posterior of its current state is not factored yet. The proposal slots are cleared for this step's observations.
+__global__ void __launch_bounds__(128) k_lazy_pick(ChainParams P, StateDev st, RngDev rng) {
+    const int C = P.C;
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool live = c < C;
+    int ci = -1;
+    if (live) {
+        double ua;
+        ci = pick_component(P, rng, rng.chain_offset + (unsigned long long)c, (unsigned int)*st.step, c, C, &ua);
+    }
+    for (int i = 0; i < P.n_icp; i++) {
+        bool want = false;
+        if (live) {
+            const size_t base = (size_t)i * 2 * C;
+            st.lz.valid[base + st.slot_prop[c]] = 0;
+            st.lz.nonfin[base + st.slot_prop[c]] = 0;
+            want = P.comp[ci].kind == ICP_PROP_ICP && P.comp[ci].icp_index == i && !st.lz.valid[base + st.slot_cur[c]];
+            if (want) st.lz.valid[base + st.slot_cur[c]] = 1;
+        }
+        lazy_append(st.lz, C, i, c, want);
+    }
+}
+
+// step 5: are the ICP terms of this step negligible in both directions (DESIGN.md section 2)? Each ICP term is
+// -(K ln 2 pi + q) / 2 <= U = -K ln 2 pi / 2. With m_N the largest other term (finite, > U), D the first non-zero summand
+// w_i exp(l_i - m_N) of the others in component order and T = sum_ICP w_i exp(U - m_N) < 2^-56 D, k_chain_accept's
+// log-sum-exp has the same maximum and the same bits with the ICP terms as -inf. The skipped posteriors must have finite
+// observations (then M = I + A^T A >= I: no status bit, no NaN form). A chain that is not certified goes to the fallback list,
+// with every component whose current posterior is not factored.
+__global__ void __launch_bounds__(128) k_lazy_certify(ChainParams P, StateDev st) {
+    extern __shared__ double sm[];
+    const int C = P.C, c = blockIdx.x;
+    __shared__ double s_fwd[kMaxComp], s_bwd[kMaxComp];
+    __shared__ int s_flags[3];
+    transition_terms(P, st, c, false, sm, s_fwd, s_bwd, s_flags);
+    if (threadIdx.x != 0) return;
+    const int sc = st.slot_cur[c], sp = st.slot_prop[c];
+    bool ok = true;
+    for (int i = 0; i < P.n_icp; i++) {
+        const size_t base = (size_t)i * 2 * C;
+        ok = ok && !st.lz.nonfin[base + sc] && !st.lz.nonfin[base + sp];
+    }
+    if (ok && !s_flags[0]) {   // (theta[0..9] differ: k_chain_accept takes the ICP terms as -inf anyway)
+        const double U = -0.5 * (P.K * ICP_LOG_2PI);
+        for (int dir = 0; dir < 2 && ok; dir++) {
+            const double *l = dir ? s_bwd : s_fwd;
+            double mN = -INFINITY;
+            bool nan = false;
+            for (int i = 0; i < P.n_comp; i++)
+                if (P.comp[i].kind != ICP_PROP_ICP) { nan = nan || l[i] != l[i]; mN = fmax(mN, l[i]); }
+            if (nan || !(mN < INFINITY) || !(U < mN)) { ok = false; break; }
+            double D = 0.0, T = 0.0;
+            for (int i = 0; i < P.n_comp; i++) {
+                if (P.comp[i].kind == ICP_PROP_ICP) T += P.comp[i].weight * exp(U - mN);
+                else if (D == 0.0) D = P.comp[i].weight * exp(l[i] - mN);
+            }
+            // D normal with room to spare: half an ulp of every partial sum from D on is then above 2^-54 D
+            ok = D >= 0x1p-1000 && T < 0x1p-56 * D;
+        }
+    }
+    st.lz.cert[c] = ok;
+    if (ok) return;
+    const int nl = 2 * P.n_icp;   // the fallback list
+    st.lz.list[(size_t)nl * C + atomicAdd(&st.lz.cnt[nl], 1)] = c;
+    for (int i = 0; i < P.n_icp; i++) {
+        const size_t base = (size_t)i * 2 * C;
+        st.lz.valid[base + sp] = 1;
+        if (!st.lz.valid[base + sc]) {
+            st.lz.valid[base + sc] = 1;
+            st.lz.list[(size_t)(P.n_icp + i) * C + atomicAdd(&st.lz.cnt[P.n_icp + i], 1)] = c;
+        }
+    }
+}
+
+// step 6, after the fallback factorisations: the forward forms of every ICP component of the fallback chains, as k_chain_propose
+// forms them under the eager schedule (same code, same block size)
+__global__ void __launch_bounds__(256) k_lazy_forward(ChainParams P, StateDev st) {
+    extern __shared__ double sm[];
+    const int K = P.K, Kp = P.Kp, Lt = K + kTheta0, C = P.C;
+    const int nl = 2 * P.n_icp;
+    if ((int)blockIdx.x >= st.lz.cnt[nl]) return;
+    const int c = st.lz.list[(size_t)nl * C + blockIdx.x];
+    // the propose kernel's layout: sdl: alpha' - alpha | sd: transition argument | red | sL
+    double *sdl = sm + 2 * Kp, *sd = sm + 3 * Kp, *red = sm + 7 * Kp, *sL = sm + 7 * Kp + 40;
+    const double *th = st.theta_cur + (size_t)c * Lt, *to = st.theta_prop + (size_t)c * Lt;
+    for (int k = threadIdx.x; k < K; k += blockDim.x) sdl[k] = to[kTheta0 + k] - th[kTheta0 + k];
+    __syncthreads();
+    for (int i = 0; i < P.n_comp; i++)
+        if (P.comp[i].kind == ICP_PROP_ICP) forward_form(P, st, c, P.comp[i], true, th, sdl, sL, sd, red);
+}
+
+// tally (nullable, lazy schedule): adds this step's list lengths to the run's counters
+__global__ void k_step_increment(int *step, LazyDev lz, int n_icp, int C) {
+    *step += 1;
+    if (!lz.tally) return;
+    long long picked = 0;
+    for (int i = 0; i < n_icp; i++) picked += lz.cnt[i];
+    const int fb = lz.cnt[2 * n_icp];
+    lz.tally[0] += picked; lz.tally[1] += fb; lz.tally[2] += C - fb;
+}
 
 // ---- rejection look-ahead ("prefetching" Metropolis-Hastings) ---------------------------------------------------------
 // A single chain is a chain of dependent latencies (SamplingRegistration.scala:60-85 is sequential), but a REJECTED step leaves
@@ -675,6 +833,15 @@ struct icp_chain_s {
     DevBuf<int> tidx;                          // [C] target of every batch entry (look-ahead: lane v takes chain v % Cr's)
     std::vector<DevBuf<double>> tp_lane;       // per ICP component: [C][n_tp][3]
     DevBuf<double> etp_lane;                   // [C][etp_n][3]
+    // lazy factorisation (LazyDev): the schedule of the resident run, the debug switch to the eager one, and per ICP component
+    // the observations of every posterior slot ([2 C][n] vid, [2 C][n][9] F, [2 C][n][3] y~, [2 C] rows in use)
+    bool resident_lazy = false;
+    int schedule = 0;        // icp_debug_chain_schedule: 0 automatic, 1 eager, 2 lazy wherever it applies
+    DevBuf<uint8_t> lz_valid, lz_nonfin, lz_cert;
+    DevBuf<int> lz_cnt, lz_list;
+    DevBuf<long long> lz_tally;
+    std::vector<DevBuf<int>> obs_vid, obs_nrows;
+    std::vector<DevBuf<double>> obs_F, obs_y;
 };
 
 namespace {
@@ -969,6 +1136,7 @@ namespace {
 
 struct RunCtx {
     icp_chain ch;
+    bool lazy = false;   // the lazy factorisation schedule (st.lz)
     int C;            // stride of the per-chain arrays (lanes in look-ahead mode: Cr * W)
     int Cn = 0;       // entries the kernels of this step / round process (C, or Cr * Wa with Wa active lanes)
     int W = 1, Cr = 0, Wa = 1;
@@ -978,6 +1146,29 @@ struct RunCtx {
     cudaStream_t s;
     int64_t launches = 0;
 };
+
+// the observation store of ICP component i (lazy schedule), rows addressed through `rows` ([C] slot indices)
+ObsDev lazy_store(icp_chain ch, int i, int C, const int *rows) {
+    const icp_proposal p = ch->icp_props[i];
+    ObsDev o{p->prm.direction == ICP_TARGET_SAMPLING ? p->n_tp : p->n_ids, ch->obs_vid[i].p, ch->obs_F[i].p, ch->obs_y[i].p,
+             ch->pwork[i].nobs.p};
+    o.nrows = ch->obs_nrows[i].p;
+    o.row = rows;
+    o.nonfinite = ch->lz_nonfin.p + (size_t)i * 2 * C;
+    return o;
+}
+
+// factorisation of the posteriors of ICP component i listed in lazy list `l`, from the stored observations of slot rows[c]
+void lazy_factor(RunCtx &r, int i, int l, const int *rows, const QuadArgs *qa, int *status) {
+    icp_chain ch = r.ch;
+    const int C = r.C, Kp = ch->model->Kp;
+    ObsDev od = lazy_store(ch, i, C, rows);
+    od.nonfinite = nullptr;
+    od.list = r.st.lz.list + (size_t)l * C;
+    od.count = r.st.lz.cnt + l;
+    posterior_factor(ch->icp_props[i], C, od, ch->pwork[i], r.st.L + (size_t)i * 2 * C * Kp * Kp, r.st.ymean + (size_t)i * 2 * C * Kp,
+                     rows, status, r.s, nullptr, qa, true, ch->n_targets > 1 ? ch->set_boundary : ch->icp_props[i]->target->has_boundary);
+}
 
 // evaluator + ICP posteriors of the parameter vectors in `theta` (all chains), written to the
 // posterior state selected by `slots`
@@ -1004,16 +1195,29 @@ void enqueue_state_eval(RunCtx &r, const double *d_theta, double *d_values, cons
         for (int i = 0; i < ch->P.n_icp; i++)
             tsv[i] = TargetSet{ch->trec.p, ch->tidx.p, ch->set_boundary, ch->tp_lane[i].p, ch->icp_props[i]->n_tp};
     const TargetSet ets{ch->trec.p, ch->tidx.p, ch->set_boundary, ch->etp_lane.p, ch->etp_n};
+    // ICP component i on stream ss. The lazy schedule keeps the observations in the component's slot store and factors only the
+    // posteriors of theta0 here; the proposal's are factored when needed (enqueue_step).
+    auto icp_posterior = [&](int i, cudaStream_t ss, const SharedCp *sh) {
+        double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *yb = r.st.ymean + (size_t)i * 2 * C * Kp;
+        if (r.lazy) {
+            const ObsDev store = lazy_store(ch, i, C, d_slots);
+            const ObsDev od = posterior_observe(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], ss, sh, multi ? &tsv[i] : nullptr, &store);
+            if (!proposal)
+                posterior_factor(ch->icp_props[i], Cn, od, ch->pwork[i], Lb, yb, d_slots, ch->pwork[i].status.p, ss, nullptr, nullptr, true,
+                                 multi ? ch->set_boundary : ch->icp_props[i]->target->has_boundary);
+            return;
+        }
+        double *Wb = ch->icp_props[i]->prm.factor == ICP_FACTOR_SVD ? r.st.W + (size_t)i * 2 * C * Kp * Kp : nullptr;
+        QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
+        posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, yb, d_slots, ss, sh, Wb, proposal ? &qa : nullptr,
+                           Wb == nullptr, multi ? &tsv[i] : nullptr);
+    };
     if (fork) ICP_CUDA(cudaEventRecord(ctx->ev_fork, r.s));
     for (int i = 0; i < ch->P.n_icp; i++) {
         if (ch->cp_shared[i] || !fork || n_side >= icp_ctx_s::kAux) continue;
         cudaStream_t ss = ctx->aux[n_side];
         ICP_CUDA(cudaStreamWaitEvent(ss, ctx->ev_fork, 0));
-        double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *yb = r.st.ymean + (size_t)i * 2 * C * Kp;
-        double *Wb = ch->icp_props[i]->prm.factor == ICP_FACTOR_SVD ? r.st.W + (size_t)i * 2 * C * Kp * Kp : nullptr;
-        QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
-        posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, yb, d_slots, ss, nullptr, Wb, proposal ? &qa : nullptr,
-                           Wb == nullptr, multi ? &tsv[i] : nullptr);
+        icp_posterior(i, ss, nullptr);
         ICP_CUDA(cudaEventRecord(ctx->ev_join[n_side], ss));
         ch->on_side[i] = 1;
         n_side++;
@@ -1021,12 +1225,8 @@ void enqueue_state_eval(RunCtx &r, const double *d_theta, double *d_values, cons
     evaluator_pipeline(ch->evaluator, ch->ework, Cn, d_theta, ch->X.p, d_values, ch->estatus.p, r.s, multi ? &ets : nullptr);
     for (int i = 0; i < ch->P.n_icp; i++) {
         if (ch->on_side[i]) { ch->on_side[i] = 0; continue; }
-        double *Lb = r.st.L + (size_t)i * 2 * C * Kp * Kp, *yb = r.st.ymean + (size_t)i * 2 * C * Kp;
         SharedCp sh{ch->ework.cp_m2t.p, ch->evaluator->n_ids, ch->cp_map[i].p};
-        double *Wb = ch->icp_props[i]->prm.factor == ICP_FACTOR_SVD ? r.st.W + (size_t)i * 2 * C * Kp * Kp : nullptr;
-        QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
-        posterior_pipeline(ch->icp_props[i], Cn, d_theta, ch->X.p, ch->pwork[i], Lb, yb, d_slots, r.s, ch->cp_shared[i] ? &sh : nullptr, Wb,
-                           proposal ? &qa : nullptr, Wb == nullptr, multi ? &tsv[i] : nullptr);
+        icp_posterior(i, r.s, ch->cp_shared[i] ? &sh : nullptr);
     }
     for (int k = 0; k < n_side; k++) ICP_CUDA(cudaStreamWaitEvent(r.s, ctx->ev_join[k], 0));   // join
 }
@@ -1046,18 +1246,47 @@ void enqueue_step(RunCtx &r) {
     ChainParams P = ch->P;
     P.C = C; P.W = r.W; P.Cr = r.Cr; P.Wa = r.Wa;
     size_t smem_p = sizeof(double) * ((size_t)7 * Kp + 40 + (size_t)Kp * (Kp + 1) / 2);
+    const int n_icp = P.n_icp;
+    if (r.lazy) {
+        // 1. pick, 2. factor the current posteriors the picked ICP components need
+        {
+            ProfScope ps(ST_OTHER, r.s);
+            ICP_CUDA(cudaMemsetAsync(r.st.lz.cnt, 0, sizeof(int) * (2 * n_icp + 1), r.s));
+            k_lazy_pick<<<(C + 127) / 128, 128, 0, r.s>>>(P, r.st, r.rng);
+            ICP_CUDA(cudaGetLastError());
+        }
+        for (int i = 0; i < n_icp; i++) lazy_factor(r, i, i, r.st.slot_cur, nullptr, nullptr);
+    }
     {
         ProfScope ps(ST_PROPOSE, r.s);
         k_chain_propose<<<Cn, 256, smem_p, r.s>>>(P, m->dev(), r.st, r.rng);
         ICP_CUDA(cudaGetLastError());
     }
     enqueue_state_eval(r, r.st.theta_prop, r.st.values_prop, r.st.slot_prop, true);
+    if (r.lazy) {
+        // 5. certify, 6. factor what the eager schedule would have used for the chains that are not certified
+        {
+            ProfScope ps(ST_OTHER, r.s);
+            k_lazy_certify<<<C, 128, sizeof(double) * 40, r.s>>>(P, r.st);
+            ICP_CUDA(cudaGetLastError());
+        }
+        for (int i = 0; i < n_icp; i++) {
+            QuadArgs qa{r.st.theta_prop, r.st.theta_cur, ch->icp_props[i]->prm.step_length, m->K, r.st.qb + (size_t)i * C};
+            lazy_factor(r, i, 2 * n_icp, r.st.slot_prop, &qa, ch->pwork[i].status.p);
+            lazy_factor(r, i, n_icp + i, r.st.slot_cur, nullptr, nullptr);
+        }
+        {
+            ProfScope ps(ST_PROPOSE, r.s);
+            k_lazy_forward<<<C, 256, smem_p, r.s>>>(P, r.st);
+            ICP_CUDA(cudaGetLastError());
+        }
+    }
     {
         ProfScope ps(ST_ACCEPT, r.s);
         k_chain_accept<<<Cn, 128, sizeof(double) * 40, r.s>>>(P, r.st, r.lg, status_sources(ch));
         ICP_CUDA(cudaGetLastError());
         if (r.W > 1) k_la_resolve<<<r.Cr, 128, 0, r.s>>>(P, r.st, r.lg);   // one round of the look-ahead: 1 .. W steps per chain
-        else k_step_increment<<<1, 1, 0, r.s>>>(r.st.step);
+        else k_step_increment<<<1, 1, 0, r.s>>>(r.st.step, r.st.lz, n_icp, C);
         ICP_CUDA(cudaGetLastError());
     }
     if (r.st.sx.pending) {
@@ -1083,6 +1312,18 @@ int lookahead_width(icp_chain ch, int C, const icp_chain_io *io, bool resume, bo
     if (w < 0) w = C <= 8 ? 8 : C <= 32 ? 4 : C <= 148 ? 2 : 1;
     if (w > 32) w = 32;
     return w < 2 ? 1 : w;
+}
+
+// The lazy factorisation schedule applies to the step-by-step runner when every ICP component can factor a list of posteriors
+// (Cholesky factor, packed rank-update path, ungrouped observations) and the mixture has a component that is not ICP (its
+// terms are what can make the ICP terms negligible). Below two chains per SM the eager schedule is faster: its two ICP
+// pipelines run side by side, where the lazy step puts its list factorisations one after the other on the critical path
+// (tools/chains_sweep.py: 0.21 against 0.15 ms per step at 8 chains, 0.29 against 0.30 at 296; profiles/r2t_lazy_posterior.md).
+bool lazy_schedule(icp_chain ch, int W, int C) {
+    if (W != 1 || ch->schedule == 1 || ch->P.n_icp == 0 || ch->P.n_icp == ch->P.n_comp) return false;
+    for (icp_proposal p : ch->icp_props)
+        if (!posterior_listable(p)) return false;
+    return ch->schedule == 2 || C >= 2 * ch->model->ctx->sm_count;
 }
 
 // on_step(k): called on the host right after step k (1-based) of this call has been enqueued on the library stream
@@ -1127,15 +1368,37 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
     ICP_REQUIRE(io->metrics_interval == 0 || io->log_metrics != nullptr, "metrics_interval > 0 needs log_metrics");
     ch->L.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp * Kp); ch->ymean.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp);
     ch->X.ensure((size_t)C * m->N * 3);
+    // the schedule is part of the resident state: a resumed run keeps it
+    const bool lazy = resume ? ch->resident_lazy : lazy_schedule(ch, W, C);
+    LazyDev lz{};
+    if (lazy) {
+        const size_t slots = (size_t)n_icp * 2 * C;
+        ch->lz_valid.ensure(slots); ch->lz_nonfin.ensure(slots); ch->lz_cert.ensure(C);
+        ch->lz_cnt.ensure(2 * n_icp + 1); ch->lz_list.ensure((size_t)(2 * n_icp + 1) * C); ch->lz_tally.ensure(3);
+        ch->obs_vid.resize(n_icp); ch->obs_nrows.resize(n_icp); ch->obs_F.resize(n_icp); ch->obs_y.resize(n_icp);
+        for (int i = 0; i < n_icp; i++) {
+            const icp_proposal p = ch->icp_props[i];
+            const size_t n = (size_t)std::max(p->prm.direction == ICP_TARGET_SAMPLING ? p->n_tp : p->n_ids, 1);
+            ch->obs_vid[i].ensure(2 * C * n); ch->obs_F[i].ensure(2 * C * n * 9); ch->obs_y[i].ensure(2 * C * n * 3);
+            ch->obs_nrows[i].ensure(2 * C);
+            ch->pwork[i].status.ensure(C);
+        }
+        ICP_CUDA(cudaMemsetAsync(ch->lz_tally.p, 0, sizeof(long long) * 3, s));
+        lz = LazyDev{ch->lz_valid.p, ch->lz_nonfin.p, ch->lz_cnt.p, ch->lz_list.p, ch->lz_cert.p, ch->lz_tally.p};
+    } else if (!resume) {   // allocated only while the lazy schedule is resident
+        ch->lz_valid.release(); ch->lz_nonfin.release(); ch->lz_cert.release(); ch->lz_cnt.release(); ch->lz_list.release();
+        ch->obs_vid.clear(); ch->obs_nrows.clear(); ch->obs_F.clear(); ch->obs_y.clear();
+    }
 
     RunCtx r;
-    r.ch = ch; r.C = C; r.Cn = C; r.s = s; r.W = W; r.Cr = Cr; r.Wa = W;
+    r.ch = ch; r.C = C; r.Cn = C; r.s = s; r.W = W; r.Cr = Cr; r.Wa = W; r.lazy = lazy;
     r.st = StateDev{ch->theta_cur.p, ch->theta_prop.p, ch->values_cur.p, ch->values_prop.p, ch->cur_sel.p,
                     ch->slot_cur.p, ch->slot_prop.p, ch->comp_sel.p, ch->u_acc.p, ch->n_acc.p, ch->step.p, ch->L.p,
                     ch->ymean.p, ch->any_svd ? ch->W.p : nullptr, ch->status.p, ch->theta_best.p, ch->value_best.p,
                     ch->qf.p, ch->qb.p, ch->lane_ok.p, ch->lane_status.p, ch->step_end.p};
     if (!resume) { ch->stats_on = ch->stats_req_on; ch->stats_run = ch->stats_req; }
     r.st.sx = StatsDev{};
+    r.st.lz = lz;
     if (ch->stats_on) {
         const size_t nv = (size_t)Cr * m->N;
         ch->sx_pending.ensure(Cr); ch->sx_count.ensure(Cr); ch->sx_flush_w.ensure(Cr); ch->sx_flush_n.ensure(Cr);
@@ -1182,7 +1445,7 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
         ICP_CUDA(cudaGetLastError());
     } else if (!resume) {
         ICP_CUDA(cudaMemcpyAsync(ch->theta_cur.p, theta0_dev, sizeof(double) * (size_t)C * Lt, cudaMemcpyDeviceToDevice, s));
-        k_chain_init<<<(C + 127) / 128, 128, 0, s>>>(C, r.st);
+        k_chain_init<<<(C + 127) / 128, 128, 0, s>>>(C, n_icp, r.st);
         ICP_CUDA(cudaGetLastError());
     }
     if (W > 1) {
@@ -1193,6 +1456,7 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
         size_t smem_p = sizeof(double) * ((size_t)7 * Kp + 40 + (size_t)Kp * (Kp + 1) / 2);
         ICP_REQUIRE(smem_p <= 227 * 1024, "rank too large for the propose kernel");
         ICP_CUDA(cudaFuncSetAttribute(k_chain_propose, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_p));
+        if (lazy) ICP_CUDA(cudaFuncSetAttribute(k_lazy_forward, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_p));
     }
     // state of theta0: log-values + posteriors of every ICP component (state 0)
     if (!resume) {
@@ -1282,6 +1546,14 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
             std::vector<const void *> tsp{ch->trec.p, ch->tidx.p, ch->etp_lane.p};
             for (const DevBuf<double> &b : ch->tp_lane) tsp.push_back(b.p);
             key.append((const char *)tsp.data(), sizeof(const void *) * tsp.size());
+            // the schedule (its state buffers are part of r.st) and the lazy schedule's observation stores
+            key.push_back(lazy ? 1 : 0);
+            std::vector<const void *> obs;
+            for (int i = 0; i < (lazy ? n_icp : 0); i++)
+                for (const void *q : {(const void *)ch->obs_vid[i].p, (const void *)ch->obs_F[i].p, (const void *)ch->obs_y[i].p,
+                                      (const void *)ch->obs_nrows[i].p, (const void *)ch->pwork[i].nobs.p})
+                    obs.push_back(q);
+            key.append((const char *)obs.data(), sizeof(const void *) * obs.size());
         }
         if (!(ch->exec && ch->exec_key == key)) {
             if (ch->exec) { cudaGraphExecDestroy(ch->exec); ch->exec = nullptr; }
@@ -1418,6 +1690,7 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
     ICP_CUDA(cudaEventRecord(ch->ev1, s));
     ch->resident_C = Cr;
     ch->resident_W = W;
+    ch->resident_lazy = lazy;
     ch->steps_total = step_base + n_steps;
     ch->last_launches = launches_total;
     ch->last_rounds = rounds_total;
@@ -1708,6 +1981,28 @@ extern "C" int32_t icp_debug_philox(icp_ctx ctx, uint64_t seed, uint64_t chain, 
         ICP_CUDA(cudaGetLastError());
         ICP_CUDA(cudaMemcpyAsync(out, d.p, 16, cudaMemcpyDeviceToHost, ctx->stream));
         ICP_CUDA(cudaStreamSynchronize(ctx->stream));
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
+    }
+}
+
+extern "C" int32_t icp_debug_chain_schedule(icp_chain c, int32_t schedule, int32_t *lazy, int64_t counters[3]) {
+    icp_ctx _ctx = c ? c->model->ctx : nullptr;
+    try {
+        ICP_REQUIRE(_ctx != nullptr, "null handle");
+        ICP_REQUIRE(schedule >= -1 && schedule <= 2, "schedule must be -1, 0, 1 or 2");
+        CtxLock lock(_ctx);
+        if (schedule >= 0) c->schedule = schedule;
+        if (lazy) *lazy = c->resident_lazy ? 1 : 0;
+        if (counters) {
+            long long h[3] = {0, 0, 0};
+            if (c->resident_lazy) {
+                ICP_CUDA(cudaMemcpyAsync(h, c->lz_tally.p, sizeof h, cudaMemcpyDeviceToHost, _ctx->stream));
+                ICP_CUDA(cudaStreamSynchronize(_ctx->stream));
+            }
+            for (int i = 0; i < 3; i++) counters[i] = h[i];
+        }
         return ICP_OK;
     } catch (...) {
         return translate_exception(_ctx);

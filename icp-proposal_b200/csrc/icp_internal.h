@@ -261,6 +261,13 @@ struct ObsDev {  // observation list of one ICP proposal for C chains, stride n 
     double *y;   // [C][n][3] F (y_i - mean_i)
     int *nobs;   // [C] observations kept
     int *nrows = nullptr;  // [C] leading slots in use (<= n; observations of one vertex may share a slot); null: n
+    // The chain runner keeps the observations of every posterior slot (lazy factorisation, chain.cu) and factors a list of them:
+    //   row (nullable: identity)   chain c's observations are row row[c] of vid / F / y / nrows (nobs stays per chain)
+    //   list (nullable: identity)  rank-update entry e is chain list[e]; M / b of the entry are written at e
+    //   count (nullable: C)        entries of the launch; the grid is sized for C, entries >= *count exit at once
+    //   nonfinite (nullable)       [rows] set to 1 when a written F or y is not finite (the caller clears it)
+    const int *row = nullptr, *list = nullptr, *count = nullptr;
+    uint8_t *nonfinite = nullptr;
 };
 struct ObsArgs {
     ModelDev m;
@@ -323,8 +330,13 @@ bool launch_rank_update_i8(const ModelDev &m, int C, const ObsDev &o, const Gram
 void launch_unit_basis(int rows, int Kp, const double *d_Q, const double *d_colnorm, double *d_Qhat, cudaStream_t s);
 void launch_pack_obs_rows(int n, int Kp, const int *d_ids, const double *d_Qhat, double *d_Qsub /* [n][3 Kp + 2] */, cudaStream_t s);
 // k_cholesky_packed on a block-packed M (the second half of launch_posterior_fused's default path)
+// d_list / d_count (nullable): factor entry e < *d_count as chain d_list[e] (M / b of entry e; L, mean, status and qa of the
+// chain), like ObsDev::list / count
 void launch_cholesky_packed(int C, int Kp, const double *d_Mp, const double *d_b, double *d_M_or_null, double *d_L, double *d_mu,
-                            const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s);
+                            const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s,
+                            const int *d_list = nullptr, const int *d_count = nullptr);
+// true when launch_posterior_fused takes its two-launch path (rank update -> block-packed M -> k_cholesky_packed) at rank Kp
+bool posterior_packed_path(int Kp);
 // the same quadratic form from L / mu (ymean: y) in global memory (paths whose factorisation kernel does not form it)
 void launch_quad_form(int C, int Kp, const double *d_L, const double *d_mu, const int *d_slot, const QuadArgs &qa, bool ymean,
                       cudaStream_t s);
@@ -662,6 +674,16 @@ struct TargetSet {
 void posterior_pipeline(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, double *d_L,
                         double *d_mu, const int *d_out_slot, cudaStream_t s, const SharedCp *shared = nullptr,
                         double *d_W = nullptr, const QuadArgs *qa = nullptr, bool ymean = false, const TargetSet *ts = nullptr);
+// posterior_pipeline in its two halves, for the chain runner's lazy factorisation (chain.cu):
+// posterior_observe: closest points + observations of C chains, into store (its vid / F / y / nrows / row / nonfinite; null: the
+// work buffers); returns the observation list to factor.
+ObsDev posterior_observe(icp_proposal p, int C, const double *d_theta, const double *d_X, PosteriorWork &w, cudaStream_t s,
+                         const SharedCp *shared, const TargetSet *ts, const ObsDev *store);
+// posterior_factor: rank update + Cholesky of od (od.list / count: the listed entries only); d_status nullable
+void posterior_factor(icp_proposal p, int C, const ObsDev &od, PosteriorWork &w, double *d_L, double *d_mu, const int *d_out_slot,
+                      int *d_status, cudaStream_t s, double *d_W, const QuadArgs *qa, bool ymean, bool has_boundary);
+// posterior_factor can factor a list of this proposal's posteriors: Cholesky factor, ungrouped observations, posterior_packed_path
+bool posterior_listable(icp_proposal p);
 // distance evaluator pipeline: values [C][3] = {product, prior, distance}; ts: see TargetSet
 void evaluator_pipeline(icp_evaluator e, EvalWork &w, int C, const double *d_theta, const double *d_X, double *d_values,
                         int *d_status, cudaStream_t s, const TargetSet *ts = nullptr);

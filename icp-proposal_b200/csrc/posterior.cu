@@ -176,14 +176,15 @@ __global__ void __launch_bounds__(256) k_observations(ObsArgs a, ObsDev o) {
         c = blockIdx.x;
         stage_mesh(a, c, sX);
         Xc = sX;
-        if (threadIdx.x == 0 && o.nrows) o.nrows[c] = o.n;
+        if (threadIdx.x == 0 && o.nrows) o.nrows[o.row ? o.row[c] : c] = o.n;
     } else {
         long long gt = (long long)blockIdx.x * blockDim.x + threadIdx.x;
         if (gt >= (long long)a.C * o.n) return;
         c = (int)(gt / o.n);
-        if (gt % o.n == 0 && o.nrows) o.nrows[c] = o.n;
+        if (gt % o.n == 0 && o.nrows) o.nrows[o.row ? o.row[c] : c] = o.n;
         Xc = a.X + (size_t)c * m.N * 3;
     }
+    const int r = o.row ? o.row[c] : c;   // where chain c's observations go
     const double *th = a.theta + (size_t)c * (m.K + kTheta0);
     for (int i0 = STAGED ? threadIdx.x : 0; i0 < (STAGED ? o.n : 1); i0 += blockDim.x) {
         if (STAGED) { i = i0; g = (long long)c * o.n + i; }
@@ -203,15 +204,16 @@ __global__ void __launch_bounds__(256) k_observations(ObsArgs a, ObsDev o) {
             tx = cpp[0]; ty = cpp[1]; tz = cpp[2];                          // :97 closest point on the target
             if (a.prm.boundary_aware && a.cp_on_boundary && a.cp_on_boundary[g]) drop = true;  // :99,104
         }
-        double *F = o.F + 9 * g, *y = o.y + 3 * g;
+        const long long go = (long long)r * o.n + i;
+        double *F = o.F + 9 * go, *y = o.y + 3 * go;
         if (drop) {
-            o.vid[g] = -1;
+            o.vid[go] = -1;
             for (int k = 0; k < 9; k++) F[k] = 0.0;
             y[0] = y[1] = y[2] = 0.0;
             continue;
         }
         atomicAdd(&o.nobs[c], 1);
-        o.vid[g] = id;
+        o.vid[go] = id;
         double f[9];
         whitening_frame(a, Xc, id, f);
         double R[9];
@@ -225,6 +227,11 @@ __global__ void __launch_bounds__(256) k_observations(ObsArgs a, ObsDev o) {
         y[0] = f[0] * y0 + f[1] * y1 + f[2] * y2;
         y[1] = f[3] * y0 + f[4] * y1 + f[5] * y2;
         y[2] = f[6] * y0 + f[7] * y1 + f[8] * y2;
+        if (o.nonfinite) {
+            bool fin = isfinite(y[0]) && isfinite(y[1]) && isfinite(y[2]);
+            for (int k = 0; k < 9; k++) fin = fin && isfinite(f[k]);
+            if (!fin) o.nonfinite[r] = 1;
+        }
     }
 }
 
@@ -235,7 +242,8 @@ void launch_observations(const ObsArgs &a, const ObsDev &o, cudaStream_t s) {
         ICP_CUDA(cudaMemsetAsync(o.nobs, 0, sizeof(int) * 2 * a.C, s));
     } else {
         ICP_CUDA(cudaMemsetAsync(o.nobs, 0, sizeof(int) * a.C, s));
-        if (o.nrows) ICP_CUDA(cudaMemsetAsync(o.nrows, 0, sizeof(int) * a.C, s));
+        // (rows addressed through o.row: k_observations writes the row count of every chain it observes)
+        if (o.nrows && !o.row) ICP_CUDA(cudaMemsetAsync(o.nrows, 0, sizeof(int) * a.C, s));
     }
     if (total <= 0) return;
     static const bool no_group = getenv("ICPCUDA_NO_GROUPING") && getenv("ICPCUDA_NO_GROUPING")[0] == '1';
@@ -983,7 +991,8 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
                                                                     const double *__restrict__ bvec, double *__restrict__ M_out,
                                                                     double *__restrict__ L, double *__restrict__ mu,
                                                                     const int *__restrict__ out_slot, int *__restrict__ status,
-                                                                    QuadArgs qa) {
+                                                                    QuadArgs qa, const int *__restrict__ list,
+                                                                    const int *__restrict__ count) {
     extern __shared__ __align__(16) double sp[];
     const int NB = Kp >> 3, ntri = NB * (NB + 1) / 2;
     double *A = sp;                  // [ntri][64]
@@ -992,11 +1001,15 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
     double *xs = dinv + Kp;          // [Kp] running right-hand side of the back substitution (YMEAN: w of the backward form)
     double *xo = xs + Kp;            // [Kp] solution (mu form only)
     __shared__ int bad;
-    const int c = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    // entry ent: M / b of the launch's ent-th matrix; chain c: where its factor, status and form go (list form: entries past the
+    // count have nothing to do)
+    const int ent = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (count && ent >= *count) return;
+    const int c = list ? list[ent] : ent;
     const int fr = lane >> 2, fc = lane & 3, sw = pk_swz(fr);
     {
         ICP_FT(const long long ftl = clock64();)
-        const double2 *src = reinterpret_cast<const double2 *>(Mp + (size_t)c * ntri * 64);
+        const double2 *src = reinterpret_cast<const double2 *>(Mp + (size_t)ent * ntri * 64);
         // 16-byte chunk e: block e / 32, row (e / 4) % 8, columns 2 (e % 4), + 1; 8 independent loads in flight per thread
         for (int e0 = tid; e0 < ntri * 32; e0 += 8 * NT) {
             double2 v[8];
@@ -1008,7 +1021,7 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
                 if (e < ntri * 32) *reinterpret_cast<double2 *>(A + (e >> 5) * 64 + r * 8 + ((2 * (e & 3)) ^ pk_swz(r))) = v[u];
             }
         }
-        for (int k = tid; k < Kp; k += NT) yv[k] = __ldcs(bvec + (size_t)c * Kp + k);
+        for (int k = tid; k < Kp; k += NT) yv[k] = __ldcs(bvec + (size_t)ent * Kp + k);
         if (tid == 0) bad = 0;
         ICP_FT(if (tid == 0 && c < 8192) g_ft[kFtStride * c + 8] = clock64() - ftl;)
     }
@@ -1016,9 +1029,9 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
     ICP_FT(const long long ftf = clock64();)
     if (M_out) {   // only the primitive API (icp_posterior) asks for M
         double *Mc = M_out + (size_t)c * Kp * Kp;
-        for (int e = tid; e < Kp * Kp; e += NT) {
-            const int i = e / Kp, j = e - i * Kp;
-            Mc[e] = j <= i ? A[pk_at(i, j)] : A[pk_at(j, i)];
+        for (int x = tid; x < Kp * Kp; x += NT) {
+            const int i = x / Kp, j = x - i * Kp;
+            Mc[x] = j <= i ? A[pk_at(i, j)] : A[pk_at(j, i)];
         }
         __syncthreads();
     }
@@ -1234,22 +1247,24 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 4 : 2) k_cholesky_packed(int K
 
 template <int NT, bool YMEAN>
 static void launch_cholesky_packed_nt(int C, int Kp, size_t smem_c, const double *d_Mp, const double *d_b, double *d_M, double *d_L,
-                                      double *d_mu, const int *d_out_slot, int *d_status, const QuadArgs &q, cudaStream_t s) {
+                                      double *d_mu, const int *d_out_slot, int *d_status, const QuadArgs &q, const int *d_list,
+                                      const int *d_count, cudaStream_t s) {
     ICP_CUDA(cudaFuncSetAttribute(k_cholesky_packed<NT, YMEAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
-    k_cholesky_packed<NT, YMEAN><<<C, NT, smem_c, s>>>(Kp, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q);
+    k_cholesky_packed<NT, YMEAN><<<C, NT, smem_c, s>>>(Kp, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, d_list, d_count);
 }
 
 static void run_cholesky_packed(int C, int Kp, size_t smem_c, const double *d_Mp, const double *d_b, double *d_M, double *d_L, double *d_mu,
-                                const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s) {
+                                const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, const int *d_list,
+                                const int *d_count, cudaStream_t s) {
     const QuadArgs q = qa ? *qa : QuadArgs{};
     // the two ICP posteriors of a step factorise concurrently: up to 148 chains all their matrices are resident at two per SM
     // (measured: 148 chains 605 k -> 646 k samples/s, one chain's round 0.179 -> 0.175 ms; at 296 chains 128 threads win)
     if (C <= 148 && Kp <= 128) {
-        if (ymean) launch_cholesky_packed_nt<256, true>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
-        else launch_cholesky_packed_nt<256, false>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
+        if (ymean) launch_cholesky_packed_nt<256, true>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, d_list, d_count, s);
+        else launch_cholesky_packed_nt<256, false>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, d_list, d_count, s);
     } else {
-        if (ymean) launch_cholesky_packed_nt<kCh3Threads, true>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
-        else launch_cholesky_packed_nt<kCh3Threads, false>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, s);
+        if (ymean) launch_cholesky_packed_nt<kCh3Threads, true>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, d_list, d_count, s);
+        else launch_cholesky_packed_nt<kCh3Threads, false>(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, q, d_list, d_count, s);
     }
 }
 
@@ -1294,12 +1309,16 @@ __global__ void __launch_bounds__((NWC + kProdWarps) * 32, 2) k_posterior_fused(
     double *sA = sm;                    // [2][24][ld]; later reused as the matrix of the factorisation
     __shared__ int bad;
     if (threadIdx.x == 0) bad = 0;
-    const int c = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    // entry ent of the launch is chain c (ObsDev::list), whose observations are row orow (ObsDev::row); CHOL = false writes M
+    // and b at ent
+    const int ent = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (o.count && ent >= *o.count) return;
+    const int c = o.list ? o.list[ent] : ent, orow = o.row ? o.row[c] : c;
     constexpr int nthreads = (NWC + kProdWarps) * 32, nwc = NWC;
     constexpr int kObsChunk = kMmaRows / RPO;   // observations per staged chunk (8 or 24)
-    const int nrows = o.nrows ? o.nrows[c] : o.n;   // slots in use (uniform over the CTA)
+    const int nrows = o.nrows ? o.nrows[orow] : o.n;   // slots in use (uniform over the CTA)
     const int nchunks = (nrows + kObsChunk - 1) / kObsChunk;
-    double *Mdst = CHOL ? sA : M_out + (size_t)c * nblk_total * 64;   // where the accumulator blocks go
+    double *Mdst = CHOL ? sA : M_out + (size_t)ent * nblk_total * 64;   // where the accumulator blocks go
     const int ldst = CHOL ? ld : 0;
     ICP_FT(long long ft0 = clock64(); long long ftw = 0; long long ftw2 = 0;)
     if (warp < nwc) {
@@ -1441,9 +1460,9 @@ __global__ void __launch_bounds__((NWC + kProdWarps) * 32, 2) k_posterior_fused(
         // ------------------------------- producers: gather + whiten ----------------------------------------
         const int pt = tid - nwc * 32;          // 0 .. 63
         const int ob = pt >> 3, cg = pt & 7;     // observation slot within the chunk, column group
-        const int *vid = o.vid + (size_t)c * o.n;
-        const double *F = o.F + (size_t)c * o.n * 9;
-        const double *y = o.y + (size_t)c * o.n * 3;
+        const int *vid = o.vid + (size_t)orow * o.n;
+        const double *F = o.F + (size_t)orow * o.n * 9;
+        const double *y = o.y + (size_t)orow * o.n * 3;
         constexpr int kNJ = (NBMAX + 1) / 2;     // column pairs per producer thread on the 16-byte path
         double bacc[2 * kNJ];
 #pragma unroll
@@ -1628,7 +1647,7 @@ __global__ void __launch_bounds__((NWC + kProdWarps) * 32, 2) k_posterior_fused(
 #pragma unroll
             for (int u = 0; u < (8 * NBMAX + kProdWarps * 32 - 1) / (kProdWarps * 32); u++) {
                 int j = pt + u * kProdWarps * 32;
-                if (j < Kp) mu[(size_t)c * Kp + j] = bval[u];
+                if (j < Kp) mu[(size_t)ent * Kp + j] = bval[u];
             }
             ICP_FT(if (pt == 0 && c < 8192) {
                 unsigned smid;
@@ -1696,7 +1715,7 @@ static void launch_fused(const ModelDev &m, int C, const ObsDev &o, double *d_M,
         }
         ProfScope _ps(ST_CHOLESKY, s);
         size_t smem_c = sizeof(double) * ((size_t)total * 64 + 4 * Kp);
-        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, qa, ymean, s);
+        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M, d_L, d_mu, d_out_slot, d_status, qa, ymean, o.list, o.count, s);
         if (quad_done) *quad_done = qa != nullptr;
         return;
     }
@@ -1712,11 +1731,12 @@ static void launch_fused(const ModelDev &m, int C, const ObsDev &o, double *d_M,
 }
 
 void launch_cholesky_packed(int C, int Kp, const double *d_Mp, const double *d_b, double *d_M_or_null, double *d_L, double *d_mu,
-                            const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s) {
+                            const int *d_out_slot, int *d_status, const QuadArgs *qa, bool ymean, cudaStream_t s,
+                            const int *d_list, const int *d_count) {
     ProfScope _ps(ST_CHOLESKY, s);
     const int NB = Kp / 8, total = NB * (NB + 1) / 2;
     size_t smem_c = sizeof(double) * ((size_t)total * 64 + 4 * Kp);
-    run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M_or_null, d_L, d_mu, d_out_slot, d_status, qa, ymean, s);
+    run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, d_M_or_null, d_L, d_mu, d_out_slot, d_status, qa, ymean, d_list, d_count, s);
     ICP_CUDA(cudaGetLastError());
 }
 
@@ -1724,16 +1744,25 @@ void launch_cholesky_packed(int C, int Kp, const double *d_Mp, const double *d_b
 // runs launch_posterior_build + launch_cholesky_solve). Default: two launches - the rank update writes M block-packed
 // (d_Mp, C x NB (NB + 1) / 2 x 64 doubles) and b (d_b), k_cholesky_packed factorises at four chains per SM.
 // ICPCUDA_FUSE=1 (or d_Mp == nullptr): the single-launch variant, whose factorisation runs at two chains per SM.
+static bool fused_off() {
+    static const bool off = (getenv("ICPCUDA_NO_DMMA") && getenv("ICPCUDA_NO_DMMA")[0] == '1') ||
+                            (getenv("ICPCUDA_NO_FUSE") && getenv("ICPCUDA_NO_FUSE")[0] == '1');
+    return off;
+}
+static bool fused_one_launch() {
+    static const bool one_launch = getenv("ICPCUDA_FUSE") && getenv("ICPCUDA_FUSE")[0] == '1';
+    return one_launch;
+}
+
+bool posterior_packed_path(int Kp) { return !fused_off() && !fused_one_launch() && Kp / 8 <= 13; }
+
 bool launch_posterior_fused(const ModelDev &m, int C, const ObsDev &o, const GramFast *gf, double *d_M_or_null, double *d_L,
                             double *d_mu, const int *d_out_slot, int *d_status, double *d_Mp, double *d_b, cudaStream_t s,
                             const QuadArgs *qa, bool *quad_done, bool ymean) {
     if (quad_done) *quad_done = false;
-    static const bool off = (getenv("ICPCUDA_NO_DMMA") && getenv("ICPCUDA_NO_DMMA")[0] == '1') ||
-                            (getenv("ICPCUDA_NO_FUSE") && getenv("ICPCUDA_NO_FUSE")[0] == '1');
-    static const bool one_launch = getenv("ICPCUDA_FUSE") && getenv("ICPCUDA_FUSE")[0] == '1';
     const int NB = m.Kp / 8, total = NB * (NB + 1) / 2;
-    if (off || NB > 13 || C <= 0) return false;   // NB <= 13: the 192-thread variants; the fused matrix must fit 2 CTAs / SM
-    if (one_launch) d_Mp = nullptr;
+    if (fused_off() || NB > 13 || C <= 0) return false;   // NB <= 13: the 192-thread variants; the fused matrix must fit 2 CTAs / SM
+    if (fused_one_launch()) d_Mp = nullptr;
     if (NB <= 4) launch_fused<4, 4, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done, ymean);
     else if (NB <= 7) launch_fused<8, 7, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done, ymean);
     else launch_fused<24, 13, 4>(m, C, o, d_M_or_null, total, gf, d_L, d_mu, d_out_slot, d_status, d_Mp, d_b, s, qa, quad_done, ymean);
@@ -1783,7 +1812,7 @@ void launch_cholesky_solve(int C, int K, int Kp, const double *d_M, const double
         ICP_REQUIRE(d_Mp != nullptr && smem_c <= 227 * 1024 - 64, "rank too large for the shared-memory Cholesky (K <= 224)");
         k_pack_lower<<<C, 128, 0, s>>>(Kp, d_M, d_Mp);
         ICP_CUDA(cudaGetLastError());
-        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, nullptr, d_L, d_mu, d_out_slot, d_status, qa, ymean, s);
+        run_cholesky_packed(C, Kp, smem_c, d_Mp, d_b, nullptr, d_L, d_mu, d_out_slot, d_status, qa, ymean, nullptr, nullptr, s);
         ICP_CUDA(cudaGetLastError());
         if (quad_done) *quad_done = qa != nullptr;
         return;

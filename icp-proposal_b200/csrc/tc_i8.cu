@@ -260,6 +260,12 @@ constexpr int kRuGroupBytes = (4 * kRuChunksPerImage + 1) * 128;   // 3712
 constexpr int kRuKBlockBytes = 4 * kRuGroupBytes;                  // 14848
 constexpr int kRuAccStride = 112;                    // TMEM columns between the accumulators of consecutive weights
 
+// observation row of rank-update entry e (ObsDev::list, ObsDev::row)
+__device__ __forceinline__ int obs_row(const ObsDev &o, int e) {
+    const int c = o.list ? __ldg(o.list + e) : e;
+    return o.row ? __ldg(o.row + c) : c;
+}
+
 template <int RPO>
 __global__ void __launch_bounds__(kRuThreads, 1) k_rank_update_i8(ModelDev m, ObsDev o, int C, I8Args a, const double *__restrict__ Gs,
                                                                   double gs_scale, double *__restrict__ Mp,
@@ -304,33 +310,44 @@ __global__ void __launch_bounds__(kRuThreads, 1) k_rank_update_i8(ModelDev m, Ob
     tc_fence_after();
     const uint32_t tmem = s_tmem;
     const int nmax = o.n;
+    if (o.count) C = min(C, *o.count);   // list form: the entries of this launch (M / b of entry e are written at e)
     I8T_DECL
 
     if (warp == kRuGatherWarp) {
         // ---------------- gather warp: raw stage R of the CTA's flattened (chain, stage) sequence ----------------
         unsigned R = 0, slot = 0, gphase = 0;                  // stage counter, its ring slot and the parity of R / NRAW
-        int c = blockIdx.x;
-        int nrows = c < C ? (o.nrows ? min(o.nrows[c], nmax) : nmax) : 0;
+        int c = blockIdx.x, rc = c < C ? obs_row(o, c) : 0;    // entry c, its observation row rc
+        int nrows = c < C ? (o.nrows ? min(o.nrows[rc], nmax) : nmax) : 0;
         int nst = 2 * ((nrows + 31) >> 5), rs = 0;
-        while (c < C && nst == 0) { c += gridDim.x; nrows = c < C ? (o.nrows ? min(o.nrows[c], nmax) : nmax) : 0; nst = 2 * ((nrows + 31) >> 5); }
+        while (c < C && nst == 0) {
+            c += gridDim.x;
+            rc = c < C ? obs_row(o, c) : 0;
+            nrows = c < C ? (o.nrows ? min(o.nrows[rc], nmax) : nmax) : 0;
+            nst = 2 * ((nrows + 31) >> 5);
+        }
         int v = -1;                                             // vertex of (c, rs) of lane's observation, loaded one stage ahead
-        if (c < C && lane < kRuRawObs && lane < nrows) v = __ldg(o.vid + (size_t)c * nmax + lane);
+        if (c < C && lane < kRuRawObs && lane < nrows) v = __ldg(o.vid + (size_t)rc * nmax + lane);
         while (c < C) {
             // successor (c2, rs2)
-            int c2 = c, rs2 = rs + 1, nrows2 = nrows, nst2 = nst;
+            int c2 = c, rc2 = rc, rs2 = rs + 1, nrows2 = nrows, nst2 = nst;
             if (rs2 >= nst) {
                 rs2 = 0;
-                do { c2 += gridDim.x; nrows2 = c2 < C ? (o.nrows ? min(o.nrows[c2], nmax) : nmax) : 0; nst2 = 2 * ((nrows2 + 31) >> 5); } while (c2 < C && nst2 == 0);
+                do {
+                    c2 += gridDim.x;
+                    rc2 = c2 < C ? obs_row(o, c2) : 0;
+                    nrows2 = c2 < C ? (o.nrows ? min(o.nrows[rc2], nmax) : nmax) : 0;
+                    nst2 = 2 * ((nrows2 + 31) >> 5);
+                } while (c2 < C && nst2 == 0);
             }
             int vnext = -1;
-            if (c2 < C && lane < kRuRawObs && rs2 * kRuRawObs + lane < nrows2) vnext = __ldg(o.vid + (size_t)c2 * nmax + rs2 * kRuRawObs + lane);
+            if (c2 < C && lane < kRuRawObs && rs2 * kRuRawObs + lane < nrows2) vnext = __ldg(o.vid + (size_t)rc2 * nmax + rs2 * kRuRawObs + lane);
             I8T_MARK();
             if (R >= (unsigned)NRAW) mbar_wait(&empty_raw[slot], gphase ^ 1u);      // parity of use (R / NRAW) - 1
             I8T_ADD(7);
             const int g0 = rs * kRuRawObs, nob = max(0, min(kRuRawObs, nrows - g0));       // observation slots of this stage
             double *fr0 = frames + (size_t)slot * kRuRawObs * kRuFrameDoubles;
             {   // frames and right-hand sides: 9 nob + 3 nob contiguous doubles, dealt over the 32 lanes
-                const double *F = o.F + ((size_t)c * nmax + g0) * 9, *y = o.y + ((size_t)c * nmax + g0) * 3;
+                const double *F = o.F + ((size_t)rc * nmax + g0) * 9, *y = o.y + ((size_t)rc * nmax + g0) * 3;
 #pragma unroll
                 for (int j = 0; j < 5; j++) {
                     const int e = lane + 32 * j;
@@ -368,7 +385,7 @@ __global__ void __launch_bounds__(kRuThreads, 1) k_rank_update_i8(ModelDev m, Ob
             R++;
             if (++slot == (unsigned)NRAW) { slot = 0; gphase ^= 1u; }                   // (no integer division in the loops: R % NRAW and
                                                                                         //  R / NRAW cost ~700 clocks per stage under contention)
-            c = c2; rs = rs2; nrows = nrows2; nst = nst2; v = vnext;
+            c = c2; rc = rc2; rs = rs2; nrows = nrows2; nst = nst2; v = vnext;
         }
         I8T_FLUSH(lane == 0, 7, 8);
     } else {
@@ -479,7 +496,7 @@ __global__ void __launch_bounds__(kRuThreads, 1) k_rank_update_i8(ModelDev m, Ob
             I8T_ADD(13);
         };
         for (int c = blockIdx.x; c < C; c += gridDim.x, it++) {
-            const int nrows = o.nrows ? min(o.nrows[c], nmax) : nmax;
+            const int nrows = o.nrows ? min(o.nrows[obs_row(o, c)], nmax) : nmax;
             const int nsteps = (nrows + 31) >> 5;
             double *sb = s_b + (it & 1) * 2 * Kp;
             if (warp == kRuMmaWarp) {
@@ -541,7 +558,7 @@ __global__ void __launch_bounds__(kRuThreads, 1) k_rank_update_i8(ModelDev m, Ob
                         published = true;
                         const int c2 = c + gridDim.x;
                         if (c2 >= C) break;
-                        const int nrows2 = o.nrows ? min(o.nrows[c2], nmax) : nmax, nsteps2 = (nrows2 + 31) >> 5;
+                        const int nrows2 = o.nrows ? min(o.nrows[obs_row(o, c2)], nmax) : nmax, nsteps2 = (nrows2 + 31) >> 5;
                         const unsigned S2 = S + nsteps;
                         const int first2 = (h - (int)S2) & 1;
                         if (first2 >= nsteps2) break;

@@ -55,6 +55,16 @@ int32_t icp_debug_factor(icp_ctx ctx, int32_t C, int32_t K, const double *M, con
 int32_t icp_debug_svd_factor(icp_ctx ctx, int32_t C, int32_t K, const double *L, const double *variance, double tol, double *W,
                              int32_t *sweeps);
 
+/* Posterior schedule of the step-by-step chain runner (DESIGN.md section 5). The runner factors an ICP posterior of a state only
+ * when a proposal from that state picks the component, or when a step's ICP transition terms are not certified negligible;
+ * the chain log is bit-identical to the eager schedule's, which factors both posteriors of every proposal.
+ * schedule for later runs from theta0: 0 the runner chooses (default), 1 eager, 2 lazy wherever it applies, also below the
+ * chain count from which the runner chooses it; -1 unchanged.
+ * lazy (nullable): whether the resident run uses the lazy schedule. counters (nullable) of the resident run, summed over the
+ * steps of the last call: [0] posteriors factored when picked, [1] chain-steps that fell back to the eager factorisations,
+ * [2] chain-steps certified (all zero under the eager schedule). */
+int32_t icp_debug_chain_schedule(icp_chain c, int32_t schedule, int32_t *lazy, int64_t counters[3]);
+
 #ifdef __cplusplus
 }
 #endif
