@@ -126,6 +126,8 @@ _SIGS = {
     "icp_eval_prior": [_h, C.c_int32, _dp, _dp],
     "icp_registration_metrics": [_h, _h, C.c_int32, _dp, _dp],
     "icp_dice_coefficient": [_h, _h, C.c_int32, _dp, C.c_int32, _dp, C.c_uint64, _dp],
+    "icp_registration_metrics_targets": [_h, C.c_int32, C.POINTER(_h), C.c_int32, _dp, _ip, _dp],
+    "icp_dice_coefficient_targets": [_h, C.c_int32, C.POINTER(_h), C.c_int32, _dp, _ip, C.c_int32, _dp, C.c_uint64, _dp],
     "icp_posterior_variability": [_h, C.c_int32, _dp, C.c_int32, _dp, _dp, _dp, _dp, _dp],
     "icp_gpmm_kernel_matrix": [_h, C.c_int32, _dp, C.c_int32, _dp, C.POINTER(KernelTerm), C.c_int32, _dp],
     "icp_gpmm_eigen_psd": [_h, C.c_int32, _dp, C.c_int32, _dp, _dp],

@@ -880,3 +880,19 @@ class RegistrationComparison:
         _, _, avg, mx = core.registration_metrics(model, target, theta.allParameters)[0]
         print(f"ID: {id_} average2surface: {avg} max: {mx}")
         return avg, mx
+
+    @staticmethod
+    def evaluateReconstructions2GroundTruth(model, thetas, targets, target_index=None, dice=False, n_samples=10000, seed=0,
+                                            unit_samples=None):
+        """The scoring stage of StdIcpVsChainICPrandomInitComparisonAll.scala:43-47 for many results at once: row c of thetas
+        (ModelFittingParameters, or a (C, K + 10) array) against targets[target_index[c]], as one device call per measure
+        (core.registration_metrics / core.dice_coefficient over the target set). Returns the (C, 4) metrics {average2surface,
+        hausdorff, boundary-aware average, boundary-aware max}, and with dice=True also the (C,) Dice coefficients
+        (n_samples / seed / unit_samples as core.dice_coefficient). Prints nothing."""
+        th = thetas if isinstance(thetas, np.ndarray) else np.stack(
+            [t.allParameters if isinstance(t, ModelFittingParameters) else np.asarray(t, float) for t in thetas])
+        metrics = core.registration_metrics(model, targets, th, target_index=target_index)
+        if not dice:
+            return metrics
+        return metrics, core.dice_coefficient(model, targets, th, unit_samples=unit_samples, n_samples=n_samples, seed=seed,
+                                              target_index=target_index)

@@ -381,23 +381,49 @@ class Evaluator:
             self.h = None
 
 
-def registration_metrics(model: Model, target: Target, theta):
+def _target_set(targets, target_index, c):
+    """(n_targets, handle array, index array or None) of a sequence of targets (icp_*_targets)."""
+    targets = list(targets)
+    hs = (_lib._h * len(targets))(*[t.h for t in targets])
+    ti = None
+    if target_index is not None:
+        ti = i32(np.asarray(target_index).reshape(-1))
+        if len(ti) != c:
+            raise ValueError(f"target_index has {len(ti)} entries for {c} parameter vectors")
+    return len(targets), hs, ti
+
+
+def registration_metrics(model: Model, target, theta, target_index=None):
+    """icp_registration_metrics: RegistrationComparison's {avg, hausdorff, avg_boundary_aware, max_boundary_aware} per
+    parameter vector. target: a Target, or a list / tuple of targets with target_index[c] naming the one of row c
+    (icp_registration_metrics_targets; target_index may be None for a one-entry list)."""
     th, c = model._theta(theta)
     out = np.empty((c, 4))
-    check(model.lib.icp_registration_metrics(model.h, target.h, c, dptr(th), dptr(out)), model.ctx.h)
+    if not isinstance(target, (list, tuple)):
+        check(model.lib.icp_registration_metrics(model.h, target.h, c, dptr(th), dptr(out)), model.ctx.h)
+        return out
+    g, hs, ti = _target_set(target, target_index, c)
+    check(model.lib.icp_registration_metrics_targets(model.h, g, hs, c, dptr(th), None if ti is None else iptr(ti), dptr(out)),
+          model.ctx.h)
     return out
 
 
-def dice_coefficient(model: Model, target: Target, theta, unit_samples=None, n_samples=10000, seed=0):
-    """icp_dice_coefficient: MeshMetrics.diceCoefficient(transformedMesh(theta), target) per parameter vector."""
+def dice_coefficient(model: Model, target, theta, unit_samples=None, n_samples=10000, seed=0, target_index=None):
+    """icp_dice_coefficient: MeshMetrics.diceCoefficient(transformedMesh(theta), target) per parameter vector. target: a
+    Target, or a sequence of targets with target_index as in registration_metrics (icp_dice_coefficient_targets)."""
     th, c = model._theta(theta)
     out = np.empty(c)
     us = None
     if unit_samples is not None:
         us = f64(unit_samples).reshape(-1, 3)
         n_samples = len(us)
-    check(model.lib.icp_dice_coefficient(model.h, target.h, c, dptr(th), int(n_samples), dptr(us) if us is not None else None,
-                                         int(seed), dptr(out)), model.ctx.h)
+    if not isinstance(target, (list, tuple)):
+        check(model.lib.icp_dice_coefficient(model.h, target.h, c, dptr(th), int(n_samples), dptr(us) if us is not None else None,
+                                             int(seed), dptr(out)), model.ctx.h)
+        return out
+    g, hs, ti = _target_set(target, target_index, c)
+    check(model.lib.icp_dice_coefficient_targets(model.h, g, hs, c, dptr(th), None if ti is None else iptr(ti), int(n_samples),
+                                                 dptr(us) if us is not None else None, int(seed), dptr(out)), model.ctx.h)
     return out
 
 

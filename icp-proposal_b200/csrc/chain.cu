@@ -1363,8 +1363,8 @@ void chain_run_device(icp_chain ch, int C, int n_steps, const double *theta0_dev
     ch->qf.ensure((size_t)std::max(n_icp, 1) * C); ch->qb.ensure((size_t)std::max(n_icp, 1) * C);
     ICP_REQUIRE(io->metrics_interval >= 0, "metrics_interval must be >= 0");
     ICP_REQUIRE(io->metrics_interval == 0 || ch->n_targets == 1,
-                "metrics_interval > 0 is not supported on a chain handle with several targets: measure each target's theta_best rows "
-                "with icp_registration_metrics after the run");
+                "metrics_interval > 0 is not supported on a chain handle with several targets: measure theta_best with "
+                "icp_registration_metrics_targets after the run");
     ICP_REQUIRE(io->metrics_interval == 0 || io->log_metrics != nullptr, "metrics_interval > 0 needs log_metrics");
     ch->L.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp * Kp); ch->ymean.ensure((size_t)std::max(n_icp, 1) * 2 * C * Kp);
     ch->X.ensure((size_t)C * m->N * 3);

@@ -643,11 +643,37 @@ struct MetricsWork {
     DevBuf<double> X, d2a, cpa, d2b;
     DevBuf<int> prim;
     DevBuf<uint8_t> skip;
+    DevBuf<double> tq;   // target set: every row's own target vertices [C][max_nt][3]
+};
+// One target of a set as the registration measures and the Dice coefficient read it: vertices, vertex normals, vertex
+// count and bounding box. Kept beside TargetRec rather than in it, so the closest-point kernels keep their record layout.
+struct TargetGeom {
+    const double *verts, *vnormals;   // [Nt][3]
+    int Nt;
+    double lo[3], hi[3];
+};
+// Several targets in one measurement (icp_registration_metrics_targets, icp_dice_coefficient_targets): row c is measured
+// against target tidx[c], whose closest-point structures are rec[tidx[c]] and whose geometry is geom[tidx[c]].
+struct MetricsTargets {
+    const TargetRec *rec;     // [G]
+    const TargetGeom *geom;   // [G]
+    const int *tidx;          // [C]
+    bool has_boundary;        // any target of the set has one: every row takes the boundary filter (a closed target's flags are 0)
+    int max_nt;               // largest Nt of the set: target -> model rows are padded to it with their last vertex
 };
 // RegistrationComparison measures of C parameter vectors on the device: d_out [C][4] = {avg, hausdorff,
-// avg_boundary_aware, max_boundary_aware}
+// avg_boundary_aware, max_boundary_aware}. ts (nullable): a target set, t then only gives the structures' primitive kinds.
 void registration_metrics_device(icp_model m, icp_target t, int C, const double *d_theta, double *d_out, MetricsWork &w,
-                                 cudaStream_t s);
+                                 cudaStream_t s, const MetricsTargets *ts = nullptr);
+// workspace of dice_device
+struct DiceWork {
+    DevBuf<double> X, pts;
+    DevBuf<int> va, vb;
+};
+// MeshMetrics.diceCoefficient of C parameter vectors on the device: d_out [C]. d_unit: [n][3] unit-cube samples, or
+// nullptr for the Philox samples of seed. ts (nullable): as registration_metrics_device.
+void dice_device(icp_model m, icp_target t, int C, const double *d_theta, int n, const double *d_unit, uint64_t seed,
+                 double *d_out, DiceWork &w, cudaStream_t s, const MetricsTargets *ts = nullptr);
 void nearest_model_vertex(icp_model m, int C, const double *d_X, int64_t nq, const double *d_q, int q_per_chain, int *d_seed,
                           int *d_prim, cudaStream_t s);
 // correspondence + posterior pipeline: L / mu (at out_slot[c] or c) for C parameter vectors on the device.

@@ -8,6 +8,8 @@
 // All of them are the closest-point / nearest-vertex queries of the hot path over every vertex (or over sample points).
 #include <algorithm>
 #include <cmath>
+#include <string>
+#include <vector>
 
 #include "icp_device.cuh"
 #include "icp_internal.h"
@@ -53,31 +55,60 @@ __global__ void __launch_bounds__(128) k_metrics(int N, int Nt, const double *__
     if (threadIdx.x == 0) { out[4 * c] = avg; out[4 * c + 1] = hd; out[4 * c + 2] = avgb; out[4 * c + 3] = empty ? NAN : red[0][0]; }
 }
 
+// row c of dst [C][nt][3]: the vertices of target tidx[c], its last vertex repeated up to nt entries. Only the maximum of the
+// target -> model distances is read (k_metrics), and a repeat does not change it.
+__global__ void k_gather_target_verts(long long total, int nt, const TargetGeom *__restrict__ geom, const int *__restrict__ tidx,
+                                      double *__restrict__ dst) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const TargetGeom &g = geom[tidx[i / nt]];
+    const int v = min((int)(i % nt), g.Nt - 1);
+#pragma unroll
+    for (int d = 0; d < 3; d++) dst[3 * i + d] = g.verts[3 * v + d];
+}
+
 void registration_metrics_device(icp_model m, icp_target t, int C, const double *d_theta, double *d_out, MetricsWork &w,
-                                 cudaStream_t s) {
+                                 cudaStream_t s, const MetricsTargets *ts) {
     if (C <= 0) return;
-    const int N = m->N, Nt = t->Nt;
-    w.X.ensure((size_t)C * N * 3); w.d2a.ensure((size_t)C * N); w.cpa.ensure((size_t)C * N * 3); w.d2b.ensure((size_t)C * Nt);
+    const int N = m->N, Nt = ts ? ts->max_nt : t->Nt;
+    const bool has_boundary = ts ? ts->has_boundary : t->has_boundary;
+    // a target set writes closest points only for the boundary filter
+    const bool want_cp = !ts || has_boundary;
+    w.X.ensure((size_t)C * N * 3); w.d2a.ensure((size_t)C * N); w.d2b.ensure((size_t)C * Nt);
+    if (want_cp) w.cpa.ensure((size_t)C * N * 3);
     launch_reconstruct(m->dev(), C, d_theta, w.X.p, s);
     // every model vertex against the target surface
     NearestArgs a;
     a.bvh = &t->tri_bvh; a.prim_data = t->tri_data.p; a.wide = t->wide(); a.sm_count = t->ctx->sm_count; a.C = C; a.nq = N; a.q = w.X.p; a.q_per_chain = 1;
-    a.out_d2 = w.d2a.p; a.out_cp = w.cpa.p;
+    a.out_d2 = w.d2a.p; a.out_cp = want_cp ? w.cpa.p : nullptr;
+    if (ts) { a.mt_rec = ts->rec; a.mt_idx = ts->tidx; }   // row c walks the BVH of its own target
     launch_nearest(a, s);
     const uint8_t *skip_p = nullptr;
-    if (t->has_boundary) {
+    if (has_boundary) {
         // :35-37 nearest target vertex of the closest point, dropped when it lies on the target's boundary
         w.prim.ensure((size_t)C * N); w.skip.ensure((size_t)C * N);
         NearestArgs v;
         v.bvh = &t->vert_bvh; v.prim_data = t->vert_data.p; v.C = C; v.nq = N; v.q = w.cpa.p; v.q_per_chain = 1; v.out_prim = w.prim.p;
+        if (ts) { v.mt_rec = ts->rec; v.mt_idx = ts->tidx; }
         launch_nearest(v, s);
-        launch_lookup_flags((int64_t)C * N, w.prim.p, t->boundary.p, Nt, w.skip.p, s);
+        // a closed target of a set has an all-zero table: its rows sum as with no filter, in the same order
+        if (ts) launch_lookup_flags((int64_t)C * N, w.prim.p, t->boundary.p, Nt, w.skip.p, s, ts->rec, ts->tidx, N);
+        else launch_lookup_flags((int64_t)C * N, w.prim.p, t->boundary.p, Nt, w.skip.p, s);
         skip_p = w.skip.p;
     }
     // every target vertex against the model surfaces (second half of hausdorffDistance)
+    const double *tq = t->verts.p;
+    if (ts) {
+        w.tq.ensure((size_t)C * Nt * 3);
+        const long long total = (long long)C * Nt;
+        k_gather_target_verts<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(total, Nt, ts->geom, ts->tidx, w.tq.p);
+        ICP_CUDA(cudaGetLastError());
+        tq = w.tq.p;
+    }
     bvh_refit(m->tri_bvh, C, w.X.p, N, m->tris.p, s);
     NearestArgs b;
-    b.bvh = &m->tri_bvh; b.X = w.X.p; b.tris = m->tris.p; b.N = N; b.C = C; b.nq = Nt; b.q = t->verts.p; b.out_d2 = w.d2b.p;
+    b.bvh = &m->tri_bvh; b.X = w.X.p; b.tris = m->tris.p; b.N = N; b.C = C; b.nq = Nt; b.q = tq; b.q_per_chain = ts ? 1 : 0;
+    b.out_d2 = w.d2b.p;
     launch_nearest(b, s);
     k_metrics<<<C, 128, 0, s>>>(N, Nt, w.d2a.p, skip_p, w.d2b.p, d_out);
     ICP_CUDA(cudaGetLastError());
@@ -88,12 +119,19 @@ void registration_metrics_device(icp_model m, icp_target t, int C, const double 
 // inside a mesh when  vertexNormal(v) . (v - p) > 0  for the mesh vertex v nearest to p (toBinaryImage);
 // dice = 2 |A and B| / (|A| + |B|). The reference draws the samples from an unseeded global RNG (10 000 of them), so the
 // caller supplies unit-cube samples (or a Philox seed) and they are scaled into each chain's evaluation region here.
+// MT: row c's target box is geom[tidx[c]]'s instead of (tlx .. thz).
+template <bool MT>
 __global__ void __launch_bounds__(256) k_dice_points(int N, const double *__restrict__ X, double tlx, double tly, double tlz,
                                                      double thx, double thy, double thz, int n,
                                                      const double *__restrict__ unit, unsigned long long seed,
-                                                     double *__restrict__ pts) {
+                                                     double *__restrict__ pts, const TargetGeom *__restrict__ geom,
+                                                     const int *__restrict__ tidx) {
     __shared__ double red[6][256];
     const int c = blockIdx.x, tid = threadIdx.x;
+    if (MT) {
+        const TargetGeom &g = geom[tidx[c]];
+        tlx = g.lo[0]; tly = g.lo[1]; tlz = g.lo[2]; thx = g.hi[0]; thy = g.hi[1]; thz = g.hi[2];
+    }
     const double *Xc = X + (size_t)c * N * 3;
     double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
     for (int v = tid; v < N; v += blockDim.x)
@@ -126,12 +164,19 @@ __global__ void __launch_bounds__(256) k_dice_points(int N, const double *__rest
     }
 }
 
+// MT: row c reads the vertices and vertex normals of target geom[tidx[c]] instead of (tverts, tnormals)
+template <bool MT>
 __global__ void __launch_bounds__(128) k_dice_count(ModelDev m, const double *__restrict__ X, int n,
                                                     const double *__restrict__ pts, const int *__restrict__ vid_model,
                                                     const int *__restrict__ vid_target, const double *__restrict__ tverts,
-                                                    const double *__restrict__ tnormals, double *__restrict__ out) {
+                                                    const double *__restrict__ tnormals, double *__restrict__ out,
+                                                    const TargetGeom *__restrict__ geom, const int *__restrict__ tidx) {
     __shared__ double red[40];
     const int c = blockIdx.x;
+    if (MT) {
+        const TargetGeom &g = geom[tidx[c]];
+        tverts = g.verts; tnormals = g.vnormals;
+    }
     const double *Xc = X + (size_t)c * m.N * 3;
     double na = 0.0, nb = 0.0, nab = 0.0;
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -150,6 +195,85 @@ __global__ void __launch_bounds__(128) k_dice_count(ModelDev m, const double *__
     __syncthreads();
     nab = block_sum(nab, red);
     if (threadIdx.x == 0) out[c] = 2.0 * nab / (na + nb);
+}
+
+void dice_device(icp_model m, icp_target t, int C, const double *d_theta, int n, const double *d_unit, uint64_t seed,
+                 double *d_out, DiceWork &w, cudaStream_t s, const MetricsTargets *ts) {
+    if (C <= 0) return;
+    const int N = m->N;
+    w.X.ensure((size_t)C * N * 3); w.pts.ensure((size_t)C * n * 3);
+    w.va.ensure((size_t)C * n); w.vb.ensure((size_t)C * n);
+    launch_reconstruct(m->dev(), C, d_theta, w.X.p, s);
+    const TargetGeom *geom = ts ? ts->geom : nullptr;
+    const int *tidx = ts ? ts->tidx : nullptr;
+    if (ts) k_dice_points<true><<<C, 256, 0, s>>>(N, w.X.p, 0, 0, 0, 0, 0, 0, n, d_unit, seed, w.pts.p, geom, tidx);
+    else k_dice_points<false><<<C, 256, 0, s>>>(N, w.X.p, t->lo[0], t->lo[1], t->lo[2], t->hi[0], t->hi[1], t->hi[2], n, d_unit, seed,
+                                                w.pts.p, nullptr, nullptr);
+    ICP_CUDA(cudaGetLastError());
+    nearest_model_vertex(m, C, w.X.p, n, w.pts.p, 1, nullptr, w.va.p, s);
+    NearestArgs v;
+    v.bvh = &t->vert_bvh; v.prim_data = t->vert_data.p; v.C = C; v.nq = n; v.q = w.pts.p; v.q_per_chain = 1; v.out_prim = w.vb.p;
+    if (ts) { v.mt_rec = ts->rec; v.mt_idx = ts->tidx; }
+    launch_nearest(v, s);
+    if (ts) k_dice_count<true><<<C, 128, 0, s>>>(m->dev(), w.X.p, n, w.pts.p, w.va.p, w.vb.p, nullptr, nullptr, d_out, geom, tidx);
+    else k_dice_count<false><<<C, 128, 0, s>>>(m->dev(), w.X.p, n, w.pts.p, w.va.p, w.vb.p, t->verts.p, t->vnormals.p, d_out,
+                                                nullptr, nullptr);
+    ICP_CUDA(cudaGetLastError());
+}
+
+// ---- target sets -----------------------------------------------------------------------------------------------------
+// The target-set calls process their rows in chunks, so that their scratch stays within a fixed budget whatever C is. Every
+// row depends on its own data only, so the results do not depend on the chunking. Metrics: model vertices + padded target
+// vertices of a row (each model vertex also carries its share of the refitted model BVH, about 300 bytes in all);
+// Dice: sample points of a row (32 bytes each).
+constexpr int64_t kMetricsChunkPoints = int64_t(1) << 23;
+constexpr int64_t kDiceChunkPoints = int64_t(1) << 25;
+
+int chunk_rows(int64_t budget, int64_t points_per_row, int C) {
+    return (int)std::max<int64_t>(1, std::min<int64_t>(C, budget / std::max<int64_t>(points_per_row, 1)));
+}
+
+void upload_unit_samples(const double *h, int n, DevBuf<double> &d, cudaStream_t s) {
+    for (size_t i = 0; i < (size_t)3 * n; i++) ICP_REQUIRE(h[i] >= 0.0 && h[i] <= 1.0, "unit_samples must lie in [0, 1]");
+    d.upload(h, (size_t)3 * n, s);
+}
+
+// every entry non-null and of the model's context
+void check_target_list(icp_model m, int G, const icp_target *targets) {
+    ICP_REQUIRE(G >= 1 && targets != nullptr, "n_targets must be >= 1 and targets non-null");
+    for (int g = 0; g < G; g++) {
+        ICP_REQUIRE(targets[g] != nullptr, "targets[" + std::to_string(g) + "] is null");
+        ICP_REQUIRE(targets[g]->ctx == m->ctx, "targets[" + std::to_string(g) + "] belongs to another context than the model");
+    }
+}
+
+// A target set of one call on the device (nothing outlives the call)
+struct TargetSetUpload {
+    DevBuf<TargetRec> rec;
+    DevBuf<TargetGeom> geom;
+    DevBuf<int> tidx;
+    MetricsTargets ts{};
+};
+
+void upload_metrics_targets(int G, const icp_target *targets, int C, const int32_t *target_index, TargetSetUpload &u,
+                            cudaStream_t s) {
+    for (int c = 0; c < C; c++)
+        ICP_REQUIRE(target_index[c] >= 0 && target_index[c] < G, "target_index[" + std::to_string(c) + "] = " +
+                    std::to_string(target_index[c]) + " is outside [0, n_targets)");
+    std::vector<icp_target> list(targets, targets + G);
+    std::vector<TargetGeom> geom(G);
+    bool has_boundary = false;
+    int max_nt = 0;
+    for (int g = 0; g < G; g++) {
+        const icp_target t = targets[g];
+        geom[g] = TargetGeom{t->verts.p, t->vnormals.p, t->Nt, {t->lo[0], t->lo[1], t->lo[2]}, {t->hi[0], t->hi[1], t->hi[2]}};
+        has_boundary = has_boundary || t->has_boundary;
+        max_nt = std::max(max_nt, t->Nt);
+    }
+    upload_target_table(list, u.rec, s);
+    u.geom.upload(geom.data(), geom.size(), s);
+    u.tidx.upload(target_index, C, s);
+    u.ts = MetricsTargets{u.rec.p, u.geom.p, u.tidx.p, has_boundary, max_nt};
 }
 
 }  // namespace icp
@@ -186,27 +310,82 @@ extern "C" int32_t icp_dice_coefficient(icp_model m, icp_target t, int32_t C, co
         if (C == 0) return ICP_OK;
         ICP_REQUIRE(C > 0 && theta != nullptr && out != nullptr && n_samples >= 1, "bad arguments");
         cudaStream_t s = _ctx->stream;
-        const int N = m->N, n = n_samples;
         m->s_theta.upload(theta, (size_t)C * (m->K + kTheta0), s);
-        DevBuf<double> X, unit, pts, dout;
-        DevBuf<int> va, vb;
-        X.alloc((size_t)C * N * 3); pts.alloc((size_t)C * n * 3); dout.alloc(C);
-        va.alloc((size_t)C * n); vb.alloc((size_t)C * n);
-        if (unit_samples) {
-            for (size_t i = 0; i < (size_t)3 * n; i++)
-                ICP_REQUIRE(unit_samples[i] >= 0.0 && unit_samples[i] <= 1.0, "unit_samples must lie in [0, 1]");
-            unit.upload(unit_samples, (size_t)3 * n, s);
+        DevBuf<double> unit, dout;
+        DiceWork w;
+        dout.alloc(C);
+        if (unit_samples) upload_unit_samples(unit_samples, n_samples, unit, s);
+        dice_device(m, t, C, m->s_theta.p, n_samples, unit_samples ? unit.p : nullptr, seed, dout.p, w, s);
+        ICP_CUDA(cudaMemcpyAsync(out, dout.p, sizeof(double) * C, cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaStreamSynchronize(s));
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
+    }
+}
+
+extern "C" int32_t icp_registration_metrics_targets(icp_model m, int32_t n_targets, const icp_target *targets, int32_t C,
+                                                    const double *theta, const int32_t *target_index, double *out) {
+    icp_ctx _ctx = m ? m->ctx : nullptr;
+    try {
+        ICP_REQUIRE(_ctx != nullptr, "null handle");
+        check_target_list(m, n_targets, targets);
+        if (n_targets == 1 && target_index == nullptr) return icp_registration_metrics(m, targets[0], C, theta, out);
+        ICP_REQUIRE(target_index != nullptr || C == 0, "target_index is required when n_targets > 1");
+        CtxLock lock(_ctx);
+        if (C == 0) return ICP_OK;
+        ICP_REQUIRE(C > 0 && theta != nullptr && out != nullptr, "bad arguments");
+        cudaStream_t s = _ctx->stream;
+        TargetSetUpload u;
+        upload_metrics_targets(n_targets, targets, C, target_index, u, s);
+        const size_t Lt = (size_t)m->K + kTheta0;
+        DevBuf<double> dth, dout;
+        dth.upload(theta, (size_t)C * Lt, s);
+        dout.alloc((size_t)4 * C);
+        MetricsWork w;
+        const int rows = chunk_rows(kMetricsChunkPoints, (int64_t)m->N + u.ts.max_nt, C);
+        for (int c0 = 0; c0 < C; c0 += rows) {
+            MetricsTargets ts = u.ts;
+            ts.tidx += c0;
+            registration_metrics_device(m, targets[0], std::min(rows, C - c0), dth.p + c0 * Lt, dout.p + (size_t)4 * c0, w, s, &ts);
         }
-        launch_reconstruct(m->dev(), C, m->s_theta.p, X.p, s);
-        k_dice_points<<<C, 256, 0, s>>>(N, X.p, t->lo[0], t->lo[1], t->lo[2], t->hi[0], t->hi[1], t->hi[2], n,
-                                        unit_samples ? unit.p : nullptr, seed, pts.p);
-        ICP_CUDA(cudaGetLastError());
-        nearest_model_vertex(m, C, X.p, n, pts.p, 1, nullptr, va.p, s);
-        NearestArgs v;
-        v.bvh = &t->vert_bvh; v.prim_data = t->vert_data.p; v.C = C; v.nq = n; v.q = pts.p; v.q_per_chain = 1; v.out_prim = vb.p;
-        launch_nearest(v, s);
-        k_dice_count<<<C, 128, 0, s>>>(m->dev(), X.p, n, pts.p, va.p, vb.p, t->verts.p, t->vnormals.p, dout.p);
-        ICP_CUDA(cudaGetLastError());
+        ICP_CUDA(cudaMemcpyAsync(out, dout.p, sizeof(double) * 4 * C, cudaMemcpyDeviceToHost, s));
+        ICP_CUDA(cudaStreamSynchronize(s));
+        return ICP_OK;
+    } catch (...) {
+        return translate_exception(_ctx);
+    }
+}
+
+extern "C" int32_t icp_dice_coefficient_targets(icp_model m, int32_t n_targets, const icp_target *targets, int32_t C,
+                                                const double *theta, const int32_t *target_index, int32_t n_samples,
+                                                const double *unit_samples, uint64_t seed, double *out) {
+    icp_ctx _ctx = m ? m->ctx : nullptr;
+    try {
+        ICP_REQUIRE(_ctx != nullptr, "null handle");
+        check_target_list(m, n_targets, targets);
+        if (n_targets == 1 && target_index == nullptr)
+            return icp_dice_coefficient(m, targets[0], C, theta, n_samples, unit_samples, seed, out);
+        ICP_REQUIRE(target_index != nullptr || C == 0, "target_index is required when n_targets > 1");
+        CtxLock lock(_ctx);
+        if (C == 0) return ICP_OK;
+        ICP_REQUIRE(C > 0 && theta != nullptr && out != nullptr && n_samples >= 1, "bad arguments");
+        cudaStream_t s = _ctx->stream;
+        TargetSetUpload u;
+        upload_metrics_targets(n_targets, targets, C, target_index, u, s);
+        const size_t Lt = (size_t)m->K + kTheta0;
+        DevBuf<double> dth, unit, dout;
+        if (unit_samples) upload_unit_samples(unit_samples, n_samples, unit, s);
+        dth.upload(theta, (size_t)C * Lt, s);
+        dout.alloc(C);
+        DiceWork w;
+        const int rows = chunk_rows(kDiceChunkPoints, n_samples, C);
+        for (int c0 = 0; c0 < C; c0 += rows) {
+            MetricsTargets ts = u.ts;
+            ts.tidx += c0;
+            dice_device(m, targets[0], std::min(rows, C - c0), dth.p + c0 * Lt, n_samples, unit_samples ? unit.p : nullptr, seed,
+                        dout.p + c0, w, s, &ts);
+        }
         ICP_CUDA(cudaMemcpyAsync(out, dout.p, sizeof(double) * C, cudaMemcpyDeviceToHost, s));
         ICP_CUDA(cudaStreamSynchronize(s));
         return ICP_OK;

@@ -283,6 +283,19 @@ int32_t icp_registration_metrics(icp_model m, icp_target t, int32_t C, const dou
  * device-generated Philox samples keyed by `seed` (the same set for every chain). out: C. */
 int32_t icp_dice_coefficient(icp_model m, icp_target t, int32_t C, const double *theta, int32_t n_samples,
                              const double *unit_samples, uint64_t seed, double *out);
+/* icp_registration_metrics / icp_dice_coefficient over a target set: row c is measured against targets[target_index[c]]
+ * (target_index: C entries in [0, n_targets), host). out as the single-target calls ([C][4] / [C]). Row c equals, bit for
+ * bit, the single-target call on targets[target_index[c]] with theta[c], NaN rows included; the seeded Dice samples are
+ * keyed by the sample index only, so every row sees the same set, as in icp_dice_coefficient. A target may appear more
+ * than once in the list. The rows are processed in chunks of bounded scratch; results do not depend on the chunking.
+ * n_targets == 1 with target_index == NULL is the single-target call. Refused with ICP_ERR_INVALID_ARGUMENT and a message
+ * naming the entry or index: a null targets[g], a target of another context than the model, target_index[c] outside
+ * [0, n_targets), target_index == NULL when n_targets > 1. Host buffers, synchronous; nothing is retained after the call. */
+int32_t icp_registration_metrics_targets(icp_model m, int32_t n_targets, const icp_target *targets, int32_t C,
+                                         const double *theta, const int32_t *target_index, double *out);
+int32_t icp_dice_coefficient_targets(icp_model m, int32_t n_targets, const icp_target *targets, int32_t C,
+                                     const double *theta, const int32_t *target_index, int32_t n_samples,
+                                     const double *unit_samples, uint64_t seed, double *out);
 /* PosteriorVariability.computeDistanceMapFromMeshesTotal / ...Normal (apps/util/PosteriorVariability.scala:30-73)
  * over the shapes LogHelper.logSamples2shapes reconstructs from S logged parameter vectors
  * (apps/util/LogHelper.scala:39-41): per model vertex the sample mean (mean: N x 3), the sample covariance with
@@ -326,8 +339,9 @@ int32_t icp_chain_destroy(icp_chain c);
  * every target, proposal and evaluator.
  * Boundary policy: the boundary path (no closest-point sharing with the evaluator, no constant-Gram posterior) is taken
  * for every chain when any target has a boundary, so a chain on a closed target of such a set agrees with its
- * single-target run to rounding, not bit for bit. Runs with metrics_interval > 0 are refused when n_targets > 1
- * (icp_registration_metrics on each target's rows of theta_best afterwards gives the same measures). */
+ * single-target run to rounding, not bit for bit. Runs with metrics_interval > 0 are refused when n_targets > 1:
+ * icp_registration_metrics_targets on theta_best with the handle's target index afterwards gives the same measures of
+ * every chain in one call. */
 typedef struct {
     icp_target target;
     const icp_component *components;  /* n_components entries */
